@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SDXL 1024x1024 UNet training-step throughput on N B200s (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--mode v_prediction]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--mode v_prediction] [--dump-outputs DIR]
 
 Own arm: ``SDXLTrainStep.step`` (aozora_sdxl_training_b200/trainer.py) on synthetic SDXL-shaped batches and random-init
 weights of the exact SDXL UNet layout: noising -> UNet fwd -> weighted MSE -> reverse sweep -> clip -> Raven update,
@@ -12,6 +12,9 @@ HOST buffers (H2D of latents / text embeddings inside the timed region) with the
 (oracle/train_step_ref.py; the UNet arithmetic is diffusers', restated -- kind "port") at BASELINE config 1 (512x512, batch 1,
 epsilon, fp32), split into fwd+bwd / clip / Raven, best of >= 3 steps, no rescaling.  ``--workload 3 | 4`` select BASELINE
 configs 3 (rectified flow, logit-normal tickets, batch 8/GPU) and 4 (layer exclusion over three aspect-ratio buckets).
+``--dump-outputs DIR`` writes what the own arm's last timed step computed as DIR/<name>.npy (see ``dump_outputs``); inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.  Compare with a tolerance: the
+attention backward adds dQ partial tiles into fp32 in arrival order, so two runs of one build agree to rounding, not bit for bit.
 """
 from __future__ import annotations
 
@@ -297,6 +300,41 @@ def cpu_config1_step(steps, warmup):
                 moments="fp32" if mdt == torch.float32 else "bf16 (host has < 64 GB free)")
 
 
+DUMP_PER_TENSOR = 2048              # sampled elements per trainable tensor: SDXL's 1680 tensors -> 31 MB in the three float32 arrays
+
+
+def dump_outputs(out_dir, res, unet, opt, dp, rank):
+    """What a caller of ``SDXLTrainStep.step`` holds after the last timed step, as float32 / float64 .npy files: the returned
+    ``loss``, ``grad_norm`` (norm, clip coefficient, sum of squares) and ``timesteps``, and the state the step updated in place --
+    ``params``, ``exp_avg`` and ``exp_avg_sq`` (Raven moments) -- as a fixed, seeded sample of ``DUMP_PER_TENSOR`` elements of
+    every trainable tensor in ``named_parameters`` order (the full state is 15 GB).  Data parallel: every rank takes part in
+    gathering the parameters and moments; rank 0 writes."""
+    import numpy as np
+    import torch
+    params = [p for p in unet.parameters() if p.requires_grad]
+    if dp is None:
+        moments = [(opt.state[p]["exp_avg"].reshape(-1), opt.state[p]["exp_avg_sq"].reshape(-1)) for p in params]
+    else:
+        dp.gather_params()
+        full_m, full_v = dp.gather_shards(opt.m_shard), dp.gather_shards(opt.v_shard)
+        moments = [(full_m[o:o + p.numel()], full_v[o:o + p.numel()]) for o, p in zip(dp.layout.offsets, params)]
+    if rank != 0:
+        return
+    g = torch.Generator().manual_seed(0)
+    picks = [torch.arange(p.numel()) if p.numel() <= DUMP_PER_TENSOR else torch.randint(p.numel(), (DUMP_PER_TENSOR,), generator=g)
+             for p in params]
+
+    def sample(flats):
+        return torch.cat([f[i.to(f.device)].float() for f, i in zip(flats, picks)]).cpu().numpy()
+
+    arrays = dict(loss=res.loss.float().cpu().numpy(), grad_norm=res.grad_norm.float().cpu().numpy(),
+                  timesteps=res.timesteps.cpu().numpy().astype(np.float64), params=sample([p.detach().reshape(-1) for p in params]),
+                  exp_avg=sample([m for m, _ in moments]), exp_avg_sq=sample([v for _, v in moments]))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 CONFIG1 = ("BASELINE config 1: SDXL UNet random-init single train step, epsilon, 512x512 (64x64x4 latents), batch 1, cached 77x2048 "
            "text embeds + 1280 pooled, Raven step, fp32 weights and moments, torch-CPU")
 
@@ -332,7 +370,13 @@ def main():
     ap.add_argument("--bucket-mb", type=int, default=512, help="data parallel: gradient reduce-scatter bucket size")
     ap.add_argument("--no-defer-all-gather", action="store_true",
                     help="data parallel: all-gather the updated parameters at the end of the step instead of behind the next forward pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, < 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU step; the reference arm has none")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -451,8 +495,10 @@ def main():
     launches = sum(per_shape_launches[i % nb] for i in range(args.steps))      # replayed from the captured graphs
     clk = clocks.stop()
 
+    last = {}
+
     def e2e_step(i):
-        res = step.step(host_batches[i % nb])
+        res = last["res"] = step.step(host_batches[i % nb])
         return res.loss_value()                                 # device -> host read of the step's loss
 
     def timed_wall(fn, n):
@@ -470,6 +516,8 @@ def main():
 
     e2e_step(0)
     ms_e2e = timed_wall(e2e_step, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last["res"], unet, opt, dp, rank)
 
     imgs = args.batch * world * args.steps
     value = imgs / (ms_dev * 1e-3)
