@@ -3,17 +3,23 @@
 // Replaces F.scaled_dot_product_attention as called by diffusers' AttnProcessor2_0 for Attention.attn1
 // (self, Tk = Tq) and Attention.attn2 (cross, Tk = 77*n) inside the UNet (reference: train.py:213-229 selects the
 // processor, train.py:2760 runs it; no mask, no dropout, scale 1/sqrt(64)).  The reference's backward is autograd
-// through SDPA; here it is two kernels (dK/dV and dQ) that recompute P from the saved log-sum-exp.
+// through SDPA; here the backward recomputes P from the saved log-sum-exp, after attn_bwd_prep_kernel has formed
+// D = rowsum(dO * O), in one of two forms:
+//   attn_bwd_fused_kernel (default)          ONE kernel: dK, dV and each KV tile's share of dQ, the shares summed in fp32
+//                                            (not bit-reproducible); attn_dq_tiles_convert_kernel scales and rounds them
+//   attn_bwd_dkv_kernel + attn_bwd_dq_kernel bit-reproducible: the reference the fused kernel is tested against, and the
+//                                            path taken when Tq % 4 != 0 (aoz_attn_set_bwd_mode(0) selects it everywhere)
 //
-// Common structure (per CTA, 192 threads):
-//   warps 0..3  one thread per tile row: softmax / dS math on the TMEM accumulators (tcgen05.ld), results written
-//               as bf16 MMA operands into 128B-swizzled shared memory
-//   warp 4      TMA producer (4-D tensor maps over [B, T, H, 64]; rows past T are zero-filled by the TMA unit)
-//   warp 5      MMA issuer (one thread, tcgen05.mma, completion through tcgen05.commit -> mbarrier)
-// S / dP / O / dK / dV / dQ accumulators live in TMEM.  Tiles: 128 query rows x 128 key rows.
+// Common structure (per CTA): compute warps, one thread per tile row, do the softmax / dS math on the TMEM accumulators
+// (tcgen05.ld); one warp is the TMA producer (4-D tensor maps over [B, T, H, 64]; rows past T are zero-filled by the TMA
+// unit), one the MMA issuer (tcgen05.mma, completion through tcgen05.commit -> mbarrier).  S / dP / O / dK / dV / dQ
+// accumulators live in TMEM.  Tiles: 128 query rows x 128 key rows (forward: 64 key rows).
 //
-// forward : S = Q K^T -> online softmax (log2 domain, lazy rescale of O) -> O += P V ; stores O (bf16), LSE (fp32)
-// dK/dV   : per KV tile, loop over Q tiles:  S^T = K Q^T, dP^T = V dO^T, P^T = exp(S^T - LSE), dS^T = P^T (dP^T - D),
+// forward : per Q tile, loop over KV tiles:  S = Q K^T -> online softmax (log2 domain, lazy rescale of O) -> O += P V ;
+//           stores O (bf16), LSE (fp32)
+// fused   : per KV tile, loop over Q tiles:  S^T = K Q^T, dP^T = V dO^T, P^T = exp(S^T - LSE), dS^T = P^T (dP^T - D),
+//           dV += P^T dO, dK += dS^T Q, dQ share += dS K
+// dK/dV   : per KV tile, loop over Q tiles:  S = Q K^T, dP = dO V^T, P = exp(S - LSE), dS = P (dP - D),
 //           dV += P^T dO, dK += dS^T Q
 // dQ      : per Q tile, loop over KV tiles:  S = Q K^T, dP = dO V^T, dS = P (dP - D), dQ += dS K
 // A [rows, 64] tile loaded once by TMA serves both as a K-major operand (contraction over d) and as an
@@ -23,7 +29,6 @@
 
 namespace aoz {
 
-constexpr int ATT_THREADS = 192;          // forward: 4 softmax warps + producer + issuer
 constexpr int BWD_CW = 16;                 // backward: 16 compute warps = four per TMEM lane quarter, 32 of a tile's 128 columns each
 constexpr int BWD_CT = BWD_CW * 32;        // (the math is latency-bound: 8 warps left the issue slots 73 % idle, ncu r01)
 constexpr int ATT_BWD_THREADS = BWD_CT + 64;   // + TMA producer warp + MMA issuer warp
@@ -43,19 +48,11 @@ struct AttnParams {
     __nv_bfloat16* dQ; long long lddq;
     __nv_bfloat16* dK; long long lddk;
     __nv_bfloat16* dV; long long lddv;
-    int fuse_dq;                // dK/dV kernel also computes dQ = dS K of every Q tile: 1 = one KV tile (cross-attention), stored as
-                                // bf16; 2 = many KV tiles, partial tiles summed into dQacc with red.global.add (fp32)
-    float* dQacc;               // [B, H, Tq, 64] fp32, zeroed by the host (fuse_dq == 2); one-kernel backward: swizzled fp32 tiles
-    int fwd_full, fwd_split;    // forward: CTAs that take a whole (b, h, Q tile) unit; CTAs per unit of the cut tail wave
-    float* fwd_ws;              // forward: [tail units][fwd_split][128][64 + 4] fp32 shares (O, reference, row sum, pad)
+    float* dQacc;               // one-kernel backward: the KV tiles' dQ shares, summed into swizzled fp32 tiles
     int q_split;                // one-kernel backward: the Q tiles of a KV tile are cut over q_split CTAs (cross-attention: one KV tile,
     float* dKacc;               //   B * H CTAs would leave most SMs idle); with q_split > 1 the CTAs' dK / dV shares are summed into
     float* dVacc;               //   these fp32 tile buffers by bulk reduce-add, like dQ
 };
-
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" :: "l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
 
 __device__ __forceinline__ float fast_exp2(float x) {
     float y;
@@ -84,15 +81,6 @@ __device__ __forceinline__ uint64_t desc_rows_as_k(uint32_t tile_addr, int k16) 
 __device__ __forceinline__ uint64_t desc_ptile(uint32_t p_addr, int k16) {                 // [128, 128] as two [128,64] blocks
     return make_sdesc_sw128(p_addr + (k16 >> 2) * TILE_BYTES + (k16 & 3) * 32, 16, 1024);
 }
-// write 32 consecutive bf16 values (packed in 16 words) of row `r`, columns [c0, c0+32) of a [128,128] P tile
-__device__ __forceinline__ void store_p_chunk(uint32_t p_addr, int r, int c0, const uint32_t* w) {
-    const uint32_t blk = p_addr + (c0 >> 6) * TILE_BYTES;
-    const int chunk0 = (c0 & 63) >> 3;                      // first 16-byte chunk inside the 128-byte row
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-        st_shared_v4(blk + sw128_offset(r, chunk0 + q), w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
-}
-
 // write 16 consecutive bf16 values (8 words) of row `r`, columns [c0, c0+16) of a [128,128] P tile
 __device__ __forceinline__ void store_p_16(uint32_t p_addr, int r, int c0, const uint32_t* w) {
     const uint32_t blk = p_addr + (c0 >> 6) * TILE_BYTES;
@@ -102,500 +90,13 @@ __device__ __forceinline__ void store_p_16(uint32_t p_addr, int r, int c0, const
 }
 
 // ================================================================================================
-// forward
-// ================================================================================================
-struct FwdSmem {
-    static constexpr int Q = 0;
-    static constexpr int K = Q + TILE_BYTES;            // 2 stages
-    static constexpr int V = K + 2 * TILE_BYTES;        // 2 stages
-    static constexpr int P = V + 2 * TILE_BYTES;        // 32 KB
-    static constexpr int BAR = P + 2 * TILE_BYTES;      // 256 B of mbarriers
-    static constexpr int XCH = BAR + 256;               // 512 B: row-max / row-sum exchange between the two column halves
-    static constexpr int TOTAL = XCH + 512;             // 2 CTAs/SM: 2 * (TOTAL + 1 KB reserved) <= 228 KB  (512 B of slack: measured,
-                                                        // 1.5 KB more drops the kernel to one CTA per SM and 321 -> 470 us)
-};
-static_assert(2 * (FwdSmem::TOTAL + 1024) <= 228 * 1024, "attention forward must keep two CTAs per SM");
-
-constexpr int ATT_FWD_THREADS = 320;                    // 8 softmax warps + producer + issuer
-
-// round a finite float UP to a bf16-representable value (exchanged row maxima only need to be consistent and >= true max)
-__device__ __forceinline__ float bf16_ceil(float x) {
-    const uint32_t t = __float_as_uint(x) & 0xffff0000u;        // truncate the magnitude
-    const float r = __uint_as_float(t);
-    return (r < x) ? __uint_as_float(t + 0x10000u) : r;         // only positive x can end up below: bump one bf16 ulp
-}
-
-__global__ void __launch_bounds__(ATT_FWD_THREADS, 2)
-attn_fwd_kernel(const __grid_constant__ AttnParams P) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = (uint64_t*)(smem + FwdSmem::BAR);
-    uint64_t* q_full = bars;            // 1
-    uint64_t* kv_full = bars + 1;       // 2
-    uint64_t* kv_empty = bars + 3;      // 2
-    uint64_t* s_ready = bars + 5;
-    uint64_t* p_ready = bars + 6;
-    uint64_t* o_ready = bars + 7;
-    uint64_t* p_free = bars + 8;        // P V of the previous tile has retired: the P tile in smem (and O in TMEM) may be touched again
-    uint32_t* tmem_slot = (uint32_t*)(bars + 9);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q_tiles = (P.Tq + TILE - 1) / TILE;
-    const int qt = blockIdx.x % q_tiles;
-    const int bh = blockIdx.x / q_tiles;
-    const int h = bh % P.H, b = bh / P.H;
-    const int q0 = qt * TILE;
-    const int nkv = (P.Tk + TILE - 1) / TILE;
-
-    if (threadIdx.x == 0) {
-        mbar_init(q_full, 1);
-        for (int i = 0; i < 2; ++i) { mbar_init(&kv_full[i], 1); mbar_init(&kv_empty[i], 1); }
-        mbar_init(s_ready, 1); mbar_init(p_ready, 256); mbar_init(o_ready, 1); mbar_init(p_free, 1);
-        fence_mbar_init();
-    }
-    if (warp == 9) tmem_alloc(tmem_slot, 256);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-    const uint32_t tS = tmem, tO = tmem + 128;
-    pdl_enter();          // prologue done: wait for the previous kernel's results before the first global access
-
-    if (warp == 8) {
-        if (lane == 0) {
-            tma_prefetch_desc(&P.tmQ); tma_prefetch_desc(&P.tmK); tma_prefetch_desc(&P.tmV);
-            mbar_arrive_expect_tx(q_full, TILE_BYTES);
-            tma_load_4d(smem + FwdSmem::Q, &P.tmQ, q_full, 0, h, q0, b);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j & 1;
-                mbar_wait(&kv_empty[s], ((j >> 1) & 1) ^ 1);
-                mbar_arrive_expect_tx(&kv_full[s], 2 * TILE_BYTES);
-                tma_load_4d(smem + FwdSmem::K + s * TILE_BYTES, &P.tmK, &kv_full[s], 0, h, j * TILE, b);
-                tma_load_4d(smem + FwdSmem::V + s * TILE_BYTES, &P.tmV, &kv_full[s], 0, h, j * TILE, b);
-            }
-        }
-    } else if (warp == 9) {
-        if (lane == 0) {
-            const uint32_t idesc_qk = make_idesc_bf16(128, 128, 0, 0);
-            const uint32_t idesc_pv = make_idesc_bf16(128, 64, 0, 1);
-            const uint32_t sQ = smem_u32(smem + FwdSmem::Q), sK = smem_u32(smem + FwdSmem::K);
-            const uint32_t sV = smem_u32(smem + FwdSmem::V), sP = smem_u32(smem + FwdSmem::P);
-            mbar_wait(q_full, 0);
-            mbar_wait(&kv_full[0], 0);
-            tc_fence_after();
-#pragma unroll
-            for (int k = 0; k < 4; ++k) umma_bf16(tS, desc_kmajor(sQ, k), desc_kmajor(sK, k), idesc_qk, k > 0);
-            umma_commit(s_ready);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j & 1;
-                mbar_wait(p_ready, j & 1);
-                tc_fence_after();
-                // S of the next tile first (the softmax warps are idle until it lands), then this tile's P V
-                if (j + 1 < nkv) {
-                    const int s2 = (j + 1) & 1;
-                    mbar_wait(&kv_full[s2], ((j + 1) >> 1) & 1);
-                    tc_fence_after();
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        umma_bf16(tS, desc_kmajor(sQ, k), desc_kmajor(sK + s2 * TILE_BYTES, k), idesc_qk, k > 0);
-                    umma_commit(s_ready);
-                }
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    umma_bf16(tO, desc_ptile(sP, k), desc_rows_as_k(sV + s * TILE_BYTES, k), idesc_pv, (j > 0 || k > 0) ? 1u : 0u);
-                umma_commit(&kv_empty[s]);
-                umma_commit(p_free);
-                if (j + 1 == nkv) umma_commit(o_ready);
-            }
-        }
-        __syncwarp();
-    } else {
-        // ---- softmax warps 0..7: two threads per query row, each owns 64 of the 128 key columns of a tile ----
-        const int qtr = warp & 3, hf = warp >> 2;
-        const int r = qtr * 32 + lane;
-        const uint32_t lane_off = (uint32_t)(qtr * 32) << 16;
-        const uint32_t sP = smem_u32(smem + FwdSmem::P);
-        __nv_bfloat16* xmax = (__nv_bfloat16*)(smem + FwdSmem::XCH);      // [2][128] bf16 (256 B used per half)
-        float* xsum = (float*)(smem + FwdSmem::XCH);                     // [128] fp32, used once at the end
-        const float sl2 = P.scale * LOG2E;
-        float m_ref = -INFINITY, l = 0.f;
-        // exp2(s * sl2 - m_ref) of this thread's 64 columns -> bf16 P tile in shared memory; returns the partial row sum and
-        // (through mx) the raw maximum.  ONE pass over TMEM: reading S is the scarce resource (64 B/clk/SM), not the math.
-        auto softmax_pass = [&](int kvalid, bool full, float& mx, int wait_parity) -> float {
-            // four 16-column chunks, software-pipelined: the tcgen05.ld of chunk c+1 is in flight during chunk c's exp math
-            float lsum = 0.f;
-            uint32_t v[2][16];
-            const int col0 = hf * 64;
-            tmem_ld16(tS + lane_off + col0, v[0]);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                tc_wait_ld();
-                if (c + 1 < 4) tmem_ld16(tS + lane_off + col0 + (c + 1) * 16, v[(c + 1) & 1]);
-                const uint32_t* cv = v[c & 1];
-                uint32_t w[8];
-                if (full) {
-#pragma unroll
-                    for (int e = 0; e < 16; e += 2) {
-                        const float s0 = __uint_as_float(cv[e]), s1 = __uint_as_float(cv[e + 1]);
-                        mx = fmaxf(mx, fmaxf(s0, s1));
-                        const float p0 = fast_exp2(fmaf(s0, sl2, -m_ref));
-                        const float p1 = fast_exp2(fmaf(s1, sl2, -m_ref));
-                        lsum += p0 + p1;
-                        w[e >> 1] = pack_bf16(p0, p1);
-                    }
-                } else {
-#pragma unroll
-                    for (int e = 0; e < 16; e += 2) {
-                        const int ka = col0 + c * 16 + e;
-                        const bool ok0 = ka < kvalid, ok1 = ka + 1 < kvalid;
-                        const float s0 = __uint_as_float(cv[e]), s1 = __uint_as_float(cv[e + 1]);
-                        if (ok0) mx = fmaxf(mx, s0);
-                        if (ok1) mx = fmaxf(mx, s1);
-                        const float p0 = ok0 ? fast_exp2(fmaf(s0, sl2, -m_ref)) : 0.f;
-                        const float p1 = ok1 ? fast_exp2(fmaf(s1, sl2, -m_ref)) : 0.f;
-                        lsum += p0 + p1;
-                        w[e >> 1] = pack_bf16(p0, p1);
-                    }
-                }
-                // the previous tile's P V reads the P tile until p_free (its MMAs are issued AFTER this tile's Q K^T)
-                if (c == 0 && wait_parity >= 0) { mbar_wait(p_free, (uint32_t)wait_parity); tc_fence_after(); }
-                store_p_16(sP, r, col0 + c * 16, w);
-            }
-            return lsum;
-        };
-        for (int j = 0; j < nkv; ++j) {
-            mbar_wait(s_ready, j & 1);
-            tc_fence_after();
-            const int kvalid = P.Tk - j * TILE;              // keys >= kvalid are padding
-            const bool full = kvalid >= TILE;                // warp-uniform: full tiles skip every per-element predicate
-            if (j == 0) {
-                // first tile: a max-only pass seeds the reference (rounded up to bf16: both threads of a row must use the SAME one)
-                float mx = -3.0e38f;
-#pragma unroll 1
-                for (int c = hf * 2; c < hf * 2 + 2; ++c) {
-                    uint32_t v[32];
-                    tmem_ld32(tS + lane_off + c * 32, v);
-                    tc_wait_ld();
-#pragma unroll
-                    for (int e = 0; e < 32; ++e)
-                        if (full || c * 32 + e < kvalid) mx = fmaxf(mx, __uint_as_float(v[e]));
-                }
-                mx = bf16_ceil(mx * sl2);
-                xmax[hf * 128 + r] = __float2bfloat16_rn(mx);    // exact: mx is bf16-representable
-                named_bar_sync(1, 256);
-                m_ref = fmaxf(mx, __bfloat162float(xmax[(hf ^ 1) * 128 + r]));
-                named_bar_sync(1, 256);                          // xmax is reused by the next tile
-                float dummy = -3.0e38f;
-                l = softmax_pass(kvalid, full, dummy, -1);
-            } else {
-                // optimistic single pass against the running reference; redo only if the row maximum jumped by > 2^8
-                float mx = -3.0e38f;
-                float lsum = softmax_pass(kvalid, full, mx, (j - 1) & 1);       // also orders the O rescale below after P V (j-1)
-                mx = bf16_ceil(mx * sl2);
-                xmax[hf * 128 + r] = __float2bfloat16_rn(mx);
-                named_bar_sync(1, 256);
-                mx = fmaxf(mx, __bfloat162float(xmax[(hf ^ 1) * 128 + r]));
-                const float m_new = fmaxf(m_ref, mx);
-                const bool need = (m_new - m_ref) > 8.0f;
-                if (__any_sync(0xffffffffu, need)) {         // identical decision in both warps that share these rows
-                    const float alpha = fast_exp2(m_ref - m_new);
-                    uint32_t v[32];
-                    tmem_ld32(tO + lane_off + hf * 32, v);   // each half rescales its 32 of the 64 output columns
-                    tc_wait_ld();
-#pragma unroll
-                    for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * alpha);
-                    tmem_st32(tO + lane_off + hf * 32, v);
-                    tc_wait_st();
-                    l *= alpha;
-                    m_ref = m_new;
-                    float dummy = -3.0e38f;
-                    lsum = softmax_pass(kvalid, full, dummy, -1);    // P of this tile again, against the new reference
-                }
-                l += lsum;
-                named_bar_sync(1, 256);                          // xmax is reused by the next tile
-            }
-            fence_proxy_async_smem();
-            tc_fence_before();
-            mbar_arrive(p_ready);
-        }
-        mbar_wait(o_ready, 0);
-        tc_fence_after();
-        // total row sum = sum of the two halves
-        if (hf == 1) xsum[r] = l;
-        named_bar_sync(1, 256);
-        if (hf == 0) { l += xsum[r]; }
-        named_bar_sync(1, 256);
-        if (hf == 0) xsum[r] = l;
-        named_bar_sync(1, 256);
-        l = xsum[r];
-        const float inv_l = 1.0f / l;
-        const int q = q0 + r;
-        {
-            const int c = hf;
-            uint32_t v[32];
-            tmem_ld32(tO + lane_off + c * 32, v);
-            tc_wait_ld();
-            if (q < P.Tq) {
-                __nv_bfloat16* dst = P.O + ((long long)b * P.Tq + q) * P.ldo + h * HD + c * 32;
-#pragma unroll
-                for (int e = 0; e < 32; e += 8) {
-                    uint4 o;
-                    o.x = pack_bf16(__uint_as_float(v[e]) * inv_l, __uint_as_float(v[e + 1]) * inv_l);
-                    o.y = pack_bf16(__uint_as_float(v[e + 2]) * inv_l, __uint_as_float(v[e + 3]) * inv_l);
-                    o.z = pack_bf16(__uint_as_float(v[e + 4]) * inv_l, __uint_as_float(v[e + 5]) * inv_l);
-                    o.w = pack_bf16(__uint_as_float(v[e + 6]) * inv_l, __uint_as_float(v[e + 7]) * inv_l);
-                    *reinterpret_cast<uint4*>(dst + e) = o;
-                }
-            }
-        }
-        if (hf == 0 && q < P.Tq) P.lse[((long long)b * P.H + h) * P.Tq + q] = (m_ref + log2f(l)) * LN2;
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 9) { tc_fence_after(); tmem_dealloc(tmem, 256); }
-}
-
-// Forward, split-statistics form (default).  The two threads that share a query row (key columns 0..63 / 64..127 of every tile) keep
-// SEPARATE running maxima and row sums and accumulate into SEPARATE O tiles in TMEM (P V is issued as two K = 64 MMA groups), so the
-// per-tile maximum exchange through shared memory and its two 256-thread named barriers disappear from the loop; the halves are
-// merged once after the last tile.  TMEM: S 128 + O_a 64 + O_b 64 = the same 256 columns as the single-O kernel.
-__global__ void __launch_bounds__(ATT_FWD_THREADS, 2)
-attn_fwd_split_kernel(const __grid_constant__ AttnParams P) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = (uint64_t*)(smem + FwdSmem::BAR);
-    uint64_t* q_full = bars;            // 1
-    uint64_t* kv_full = bars + 1;       // 2
-    uint64_t* kv_empty = bars + 3;      // 2
-    uint64_t* s_ready = bars + 5;
-    uint64_t* p_ready = bars + 6;
-    uint64_t* o_ready = bars + 7;
-    uint64_t* p_free = bars + 8;        // P V of the previous tile has retired: the P tile in smem (and O in TMEM) may be touched again
-    uint32_t* tmem_slot = (uint32_t*)(bars + 9);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q_tiles = (P.Tq + TILE - 1) / TILE;
-    const int qt = blockIdx.x % q_tiles;
-    const int bh = blockIdx.x / q_tiles;
-    const int h = bh % P.H, b = bh / P.H;
-    const int q0 = qt * TILE;
-    const int nkv = (P.Tk + TILE - 1) / TILE;
-
-    if (threadIdx.x == 0) {
-        mbar_init(q_full, 1);
-        for (int i = 0; i < 2; ++i) { mbar_init(&kv_full[i], 1); mbar_init(&kv_empty[i], 1); }
-        mbar_init(s_ready, 1); mbar_init(p_ready, 256); mbar_init(o_ready, 1); mbar_init(p_free, 1);
-        fence_mbar_init();
-    }
-    if (warp == 9) tmem_alloc(tmem_slot, 256);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-    const uint32_t tS = tmem, tOa = tmem + 128, tOb = tmem + 192;      // O accumulators of the two key halves
-    pdl_enter();          // prologue done: wait for the previous kernel's results before the first global access
-
-    if (warp == 8) {
-        if (lane == 0) {
-            tma_prefetch_desc(&P.tmQ); tma_prefetch_desc(&P.tmK); tma_prefetch_desc(&P.tmV);
-            mbar_arrive_expect_tx(q_full, TILE_BYTES);
-            tma_load_4d(smem + FwdSmem::Q, &P.tmQ, q_full, 0, h, q0, b);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j & 1;
-                mbar_wait(&kv_empty[s], ((j >> 1) & 1) ^ 1);
-                mbar_arrive_expect_tx(&kv_full[s], 2 * TILE_BYTES);
-                tma_load_4d(smem + FwdSmem::K + s * TILE_BYTES, &P.tmK, &kv_full[s], 0, h, j * TILE, b);
-                tma_load_4d(smem + FwdSmem::V + s * TILE_BYTES, &P.tmV, &kv_full[s], 0, h, j * TILE, b);
-            }
-        }
-    } else if (warp == 9) {
-        if (lane == 0) {
-            const uint32_t idesc_qk = make_idesc_bf16(128, 128, 0, 0);
-            const uint32_t idesc_pv = make_idesc_bf16(128, 64, 0, 1);
-            const uint32_t sQ = smem_u32(smem + FwdSmem::Q), sK = smem_u32(smem + FwdSmem::K);
-            const uint32_t sV = smem_u32(smem + FwdSmem::V), sP = smem_u32(smem + FwdSmem::P);
-            mbar_wait(q_full, 0);
-            mbar_wait(&kv_full[0], 0);
-            tc_fence_after();
-#pragma unroll
-            for (int k = 0; k < 4; ++k) umma_bf16(tS, desc_kmajor(sQ, k), desc_kmajor(sK, k), idesc_qk, k > 0);
-            umma_commit(s_ready);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j & 1;
-                mbar_wait(p_ready, j & 1);
-                tc_fence_after();
-                // S of the next tile first (the softmax warps are idle until it lands), then this tile's P V
-                if (j + 1 < nkv) {
-                    const int s2 = (j + 1) & 1;
-                    mbar_wait(&kv_full[s2], ((j + 1) >> 1) & 1);
-                    tc_fence_after();
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        umma_bf16(tS, desc_kmajor(sQ, k), desc_kmajor(sK + s2 * TILE_BYTES, k), idesc_qk, k > 0);
-                    umma_commit(s_ready);
-                }
-#pragma unroll
-                for (int k = 0; k < 4; ++k)          // keys 0..63 of the tile -> O_a, keys 64..127 -> O_b (each half has its own running max)
-                    umma_bf16(tOa, desc_ptile(sP, k), desc_rows_as_k(sV + s * TILE_BYTES, k), idesc_pv, (j > 0 || k > 0) ? 1u : 0u);
-#pragma unroll
-                for (int k = 4; k < 8; ++k)
-                    umma_bf16(tOb, desc_ptile(sP, k), desc_rows_as_k(sV + s * TILE_BYTES, k), idesc_pv, (j > 0 || k > 4) ? 1u : 0u);
-                umma_commit(&kv_empty[s]);
-                umma_commit(p_free);
-                if (j + 1 == nkv) umma_commit(o_ready);
-            }
-        }
-        __syncwarp();
-    } else {
-        // ---- softmax warps 0..7: two threads per query row, each owns 64 of the 128 key columns of a tile ----
-        const int qtr = warp & 3, hf = warp >> 2;
-        const int r = qtr * 32 + lane;
-        const uint32_t lane_off = (uint32_t)(qtr * 32) << 16;
-        const uint32_t sP = smem_u32(smem + FwdSmem::P);
-        float* xm = (float*)(smem + FwdSmem::P);                         // [2][128] running max of each half, exchanged once at the end
-        float* xl = xm + 256;                                            // [2][128] row sums  (the P tile is idle by then)
-        const float sl2 = P.scale * LOG2E;
-        float m_ref = -INFINITY, l = 0.f;
-        // exp2(s * sl2 - m_ref) of this thread's 64 columns -> bf16 P tile in shared memory; returns the partial row sum and
-        // (through mx) the raw maximum.  ONE pass over TMEM: reading S is the scarce resource (64 B/clk/SM), not the math.
-        auto softmax_pass = [&](int kvalid, bool full, float& mx, int wait_parity) -> float {
-            // four 16-column chunks, software-pipelined: the tcgen05.ld of chunk c+1 is in flight during chunk c's exp math
-            float lsum = 0.f;
-            uint32_t v[2][16];
-            const int col0 = hf * 64;
-            tmem_ld16(tS + lane_off + col0, v[0]);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                tc_wait_ld();
-                if (c + 1 < 4) tmem_ld16(tS + lane_off + col0 + (c + 1) * 16, v[(c + 1) & 1]);
-                const uint32_t* cv = v[c & 1];
-                uint32_t w[8];
-                if (full) {
-#pragma unroll
-                    for (int e = 0; e < 16; e += 2) {
-                        const float s0 = __uint_as_float(cv[e]), s1 = __uint_as_float(cv[e + 1]);
-                        mx = fmaxf(mx, fmaxf(s0, s1));
-                        const float p0 = fast_exp2(fmaf(s0, sl2, -m_ref));
-                        const float p1 = fast_exp2(fmaf(s1, sl2, -m_ref));
-                        lsum += p0 + p1;
-                        w[e >> 1] = pack_bf16(p0, p1);
-                    }
-                } else {
-#pragma unroll
-                    for (int e = 0; e < 16; e += 2) {
-                        const int ka = col0 + c * 16 + e;
-                        const bool ok0 = ka < kvalid, ok1 = ka + 1 < kvalid;
-                        const float s0 = __uint_as_float(cv[e]), s1 = __uint_as_float(cv[e + 1]);
-                        if (ok0) mx = fmaxf(mx, s0);
-                        if (ok1) mx = fmaxf(mx, s1);
-                        const float p0 = ok0 ? fast_exp2(fmaf(s0, sl2, -m_ref)) : 0.f;
-                        const float p1 = ok1 ? fast_exp2(fmaf(s1, sl2, -m_ref)) : 0.f;
-                        lsum += p0 + p1;
-                        w[e >> 1] = pack_bf16(p0, p1);
-                    }
-                }
-                // the previous tile's P V reads the P tile until p_free (its MMAs are issued AFTER this tile's Q K^T)
-                if (c == 0 && wait_parity >= 0) { mbar_wait(p_free, (uint32_t)wait_parity); tc_fence_after(); }
-                store_p_16(sP, r, col0 + c * 16, w);
-            }
-            return lsum;
-        };
-        for (int j = 0; j < nkv; ++j) {
-            mbar_wait(s_ready, j & 1);
-            tc_fence_after();
-            const int kvalid = P.Tk - j * TILE;              // keys >= kvalid are padding
-            const bool full = kvalid >= TILE;                // warp-uniform: full tiles skip every per-element predicate
-            if (j == 0) {
-                // first tile: a max-only pass over this thread's 64 columns seeds ITS reference (no exchange with the other half)
-                float mx = -3.0e38f;
-#pragma unroll 1
-                for (int c = hf * 2; c < hf * 2 + 2; ++c) {
-                    uint32_t v[32];
-                    tmem_ld32(tS + lane_off + c * 32, v);
-                    tc_wait_ld();
-#pragma unroll
-                    for (int e = 0; e < 32; ++e)
-                        if (full || c * 32 + e < kvalid) mx = fmaxf(mx, __uint_as_float(v[e]));
-                }
-                m_ref = mx * sl2;
-                float dummy = -3.0e38f;
-                l = softmax_pass(kvalid, full, dummy, -1);
-            } else {
-                // optimistic single pass against the running reference; redo only if the row maximum jumped by > 2^8
-                float mx = -3.0e38f;
-                float lsum = softmax_pass(kvalid, full, mx, (j - 1) & 1);       // also orders the O rescale below after P V (j-1)
-                const float m_new = fmaxf(m_ref, mx * sl2);
-                const bool need = (m_new - m_ref) > 8.0f;
-                if (__any_sync(0xffffffffu, need)) {
-                    const float alpha = fast_exp2(m_ref - m_new);
-                    const uint32_t tOx = hf == 0 ? tOa : tOb;                  // this half's own accumulator: all 64 columns
-#pragma unroll 1
-                    for (int c = 0; c < 2; ++c) {
-                        uint32_t v[32];
-                        tmem_ld32(tOx + lane_off + c * 32, v);
-                        tc_wait_ld();
-#pragma unroll
-                        for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * alpha);
-                        tmem_st32(tOx + lane_off + c * 32, v);
-                        tc_wait_st();
-                    }
-                    l *= alpha;
-                    m_ref = m_new;
-                    float dummy = -3.0e38f;
-                    lsum = softmax_pass(kvalid, full, dummy, -1);    // P of this tile again, against the new reference
-                }
-                l += lsum;
-            }
-            fence_proxy_async_smem();
-            tc_fence_before();
-            mbar_arrive(p_ready);
-        }
-        mbar_wait(o_ready, 0);
-        tc_fence_after();
-        // combine the two halves: O = (O_a 2^(m_a - m) + O_b 2^(m_b - m)) / (l_a 2^(m_a - m) + l_b 2^(m_b - m))
-        xm[hf * 128 + r] = m_ref;
-        xl[hf * 128 + r] = l;
-        named_bar_sync(1, 256);
-        const float m_o = xm[(hf ^ 1) * 128 + r], l_o = xl[(hf ^ 1) * 128 + r];
-        const float m = fmaxf(m_ref, m_o);
-        const float w_me = fast_exp2(m_ref - m), w_o = fast_exp2(m_o - m);
-        const float wa = hf == 0 ? w_me : w_o, wb = hf == 0 ? w_o : w_me;
-        const float lt = l * w_me + l_o * w_o;
-        const float inv_l = 1.0f / lt;
-        const int q = q0 + r;
-        {
-            const int c = hf;                                    // this thread stores 32 of the 64 output columns
-            uint32_t va[32], vb[32];
-            tmem_ld32(tOa + lane_off + c * 32, va);
-            tmem_ld32(tOb + lane_off + c * 32, vb);
-            tc_wait_ld();
-            if (q < P.Tq) {
-                __nv_bfloat16* dst = P.O + ((long long)b * P.Tq + q) * P.ldo + h * HD + c * 32;
-                const float sa = wa * inv_l, sb = wb * inv_l;
-#pragma unroll
-                for (int e = 0; e < 32; e += 8) {
-                    float f[8];
-#pragma unroll
-                    for (int t = 0; t < 8; ++t) f[t] = fmaf(__uint_as_float(va[e + t]), sa, __uint_as_float(vb[e + t]) * sb);
-                    uint4 o;
-                    o.x = pack_bf16(f[0], f[1]); o.y = pack_bf16(f[2], f[3]); o.z = pack_bf16(f[4], f[5]); o.w = pack_bf16(f[6], f[7]);
-                    *reinterpret_cast<uint4*>(dst + e) = o;
-                }
-            }
-        }
-        if (hf == 0 && q < P.Tq) P.lse[((long long)b * P.H + h) * P.Tq + q] = (m + log2f(lt)) * LN2;
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 9) { tc_fence_after(); tmem_dealloc(tmem, 256); }
-}
-
-// ================================================================================================
-// forward, P-in-TMEM form (default)
+// forward: S = Q K^T -> online softmax -> O += P V, P kept in tensor memory
 // ================================================================================================
 // Measured on B200 (tools/tmem_probe.cu, profiles/r02_tmem_probe.txt): tcgen05.ld sustains ~930 B/clk/SM and ex2 exactly 16 /clk/SM,
 // so a 128 x 128 score tile costs 1024 MUFU cycles against 512 MMA cycles and ~70 cycles of TMEM reads: the exponentials are the
-// bound.  The split-statistics kernel above ran at 1966 cycles per tile (ncu r01) for two reasons that ncu's source view showed in
-// round 2: its single issuing THREAD was the critical path (see elect_one_sync), and with ~9 instructions per score element the
-// softmax warps were issue-bound.  This form is built to keep the MUFU pipe fed:
+// bound.  The round-1 forward (split statistics, P through shared memory) ran at 1966 cycles per tile (ncu r01) for two reasons
+// that ncu's source view showed in round 2: its single issuing THREAD was the critical path (see elect_one_sync), and with ~9
+// instructions per score element the softmax warps were issue-bound.  This kernel is built to keep the MUFU pipe fed:
 //   * one thread per query row and 64-key tiles; per score element 1 FFMA + 1 MUFU + 1 FADD + 0.5 F2FP + 0.17 integer max;
 //   * P never leaves tensor memory: a thread overwrites the front of ITS OWN score row with 32 packed bf16x2 words (tcgen05.st) and
 //     P V is a tcgen05.mma whose A operand is read from TMEM (layout verified by tools/tmem_probe.cu) -- no shared-memory P tile,
@@ -603,9 +104,7 @@ attn_fwd_split_kernel(const __grid_constant__ AttnParams P) {
 //     hardware interleaves their softmax / MMA phases (16 softmax warps per SM; measured 3 CTAs: 697, 4 CTAs: 724 TFLOP/s);
 //   * the running maximum is only a REFERENCE (any value that keeps 2^(s - ref) finite works: LSE = ref + log2 l exactly), so the
 //     common path does not track the maximum of S at all -- it takes an integer max over the packed bf16 P words and falls back
-//     to an exact max + rescale of O and l only when some P exceeded 2^8;
-//   * optionally part of the exponentials go to the FMA pipe (Cody-Waite reduction + degree-3 polynomial, relative error 9e-5 <<
-//     bf16's 2^-9), POLY_MASK selecting which elements of every 16.
+//     to an exact max + rescale of O and l only when some P exceeded 2^8.
 constexpr int KT = 64;                         // keys per score tile
 constexpr int KT_BYTES = KT * HD * 2;          // 8 KB: one [64, 64] bf16 tile
 constexpr int TM_STAGES = 2;                   // K / V ring
@@ -621,19 +120,6 @@ struct TmSmem {
 };
 static_assert(TM_CTAS * (TmSmem::TOTAL + 1024) <= 228 * 1024, "attention forward must keep TM_CTAS CTAs per SM");
 
-// 2^x for x <= ~100 on the FMA pipe: n = round(x), r = x - n in [-0.5, 0.5], 2^r by a degree-3 minimax polynomial, exponent added
-// through the integer view.  Max relative error 8.8e-5 (the result is rounded to bf16, 3.9e-3).  x below -126 flushes to ~0.
-__device__ __forceinline__ float poly_exp2(float x) {
-    x = fmaxf(x, -126.0f);
-    const float t = x + 12582912.0f;                        // 1.5 * 2^23: low mantissa bits now hold round(x) (two's complement)
-    const float r = x - (t - 12582912.0f);
-    float p = fmaf(0.0555041086648216f, r, 0.2402264923172690f);
-    p = fmaf(p, r, 0.6931471805599453f);
-    p = fmaf(p, r, 1.0f);
-    return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
-// which elements of every 16 take the polynomial: 0x8888 = one in four, 0x8080 = one in eight, 0 = none, 0xAAAA = every other
-
 __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
@@ -647,7 +133,6 @@ __device__ __forceinline__ uint32_t max_u16x2(uint32_t a, uint32_t b) {
     return d;
 }
 
-template <uint32_t POLY_MASK>
 __global__ void __launch_bounds__(ATT_TM_THREADS, TM_CTAS)
 attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -662,23 +147,11 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int q_tiles = (P.Tq + TILE - 1) / TILE;
-    // Work units are (b, h, Q tile).  The first P.fwd_full CTAs take one whole unit each; the units of the last, partly filled wave
-    // are cut along the keys over P.fwd_split CTAs each (their unnormalised O, reference and row sum go to P.fwd_ws and
-    // attn_fwd_combine_kernel merges them): 1280 equal CTAs on 592 slots would otherwise cost three waves for 2.16 waves of work.
-    const int kv_all = (P.Tk + KT - 1) / KT;
-    int unit = blockIdx.x, j0 = 0, nkv = kv_all, part = -1;
-    if ((int)blockIdx.x >= P.fwd_full) {
-        const int idx = blockIdx.x - P.fwd_full;
-        unit = P.fwd_full + idx / P.fwd_split;
-        part = idx % P.fwd_split;
-        const int per = (kv_all + P.fwd_split - 1) / P.fwd_split;
-        j0 = part * per;
-        nkv = max(0, min(per, kv_all - j0));                 // key tiles j0 .. j0 + nkv - 1 (the loop index j below is LOCAL)
-    }
-    const int qt = unit % q_tiles;
-    const int bh = unit / q_tiles;
+    const int qt = blockIdx.x % q_tiles;
+    const int bh = blockIdx.x / q_tiles;
     const int h = bh % P.H, b = bh / P.H;
     const int q0 = qt * TILE;
+    const int nkv = (P.Tk + KT - 1) / KT;
 
     if (threadIdx.x == 0) {
         mbar_init(q_full, 1);
@@ -703,8 +176,8 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
                 const int s = j % TM_STAGES;
                 mbar_wait_relaxed(&kv_empty[s], ((j / TM_STAGES) & 1) ^ 1);
                 mbar_arrive_expect_tx(&kv_full[s], 2 * KT_BYTES);
-                tma_load_4d(smem + TmSmem::K + s * KT_BYTES, &P.tmK, &kv_full[s], 0, h, (j0 + j) * KT, b);
-                tma_load_4d(smem + TmSmem::V + s * KT_BYTES, &P.tmV, &kv_full[s], 0, h, (j0 + j) * KT, b);
+                tma_load_4d(smem + TmSmem::K + s * KT_BYTES, &P.tmK, &kv_full[s], 0, h, j * KT, b);
+                tma_load_4d(smem + TmSmem::V + s * KT_BYTES, &P.tmV, &kv_full[s], 0, h, j * KT, b);
             }
         }
     } else if (warp == 5) {
@@ -729,7 +202,7 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
             __syncwarp();
         };
         mbar_wait(q_full, 0);
-        if (nkv > 0) issue_s(0);
+        issue_s(0);
         for (int j = 0; j < nkv; ++j) {
             const int s = j % TM_STAGES;
             mbar_wait(p_ready, j & 1);
@@ -768,10 +241,7 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
                 for (int e = 0; e < 16; e += 4) {
                     float p[4];
 #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const float x = fmaf(__uint_as_float(cv[e + t]), sl2, -m_ref);
-                        p[t] = ((POLY_MASK >> (e + t)) & 1u) ? poly_exp2(x) : fast_exp2(x);
-                    }
+                    for (int t = 0; t < 4; ++t) p[t] = fast_exp2(fmaf(__uint_as_float(cv[e + t]), sl2, -m_ref));
                     a0 += p[0]; a1 += p[1]; a2 += p[2]; a3 += p[3];
                     const uint32_t w0 = pack_bf16(p[0], p[1]), w1 = pack_bf16(p[2], p[3]);
                     w[c * 8 + (e >> 1)] = w0; w[c * 8 + (e >> 1) + 1] = w1;
@@ -818,7 +288,7 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
         for (int j = 0; j < nkv; ++j) {
             mbar_wait(s_ready, j & 1);                       // also: P V(j-1) has retired, O may be rescaled
             tc_fence_after();
-            const int kvalid = P.Tk - (j0 + j) * KT;         // keys >= kvalid are padding
+            const int kvalid = P.Tk - j * KT;                // keys >= kvalid are padding
             uint32_t w[32];
             float lsum = 0.f;
             if (j == 0) {
@@ -859,22 +329,9 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
             __syncwarp();
             if (lane == 0) mbar_arrive(p_ready);             // one arrival per warp: 32 same-address arrivals serialise in the MIO pipe
         }
-        if (nkv > 0) { mbar_wait(o_ready, 0); tc_fence_after(); }
+        mbar_wait(o_ready, 0);
+        tc_fence_after();
         const int q = q0 + r;
-        if (part >= 0) {
-            // a share of the keys: unnormalised accumulator, reference and row sum (an empty share: l = 0, reference -inf)
-            const long long slot = (long long)(unit - P.fwd_full) * P.fwd_split + part;
-            float* wo = P.fwd_ws + (slot * TILE + r) * (HD + 4);
-#pragma unroll 1
-            for (int c = 0; c < 2; ++c) {
-                uint32_t v[32];
-                if (nkv > 0) { tmem_ld32(tO + lane_off + c * 32, v); tc_wait_ld(); }
-#pragma unroll
-                for (int e = 0; e < 32; e += 2)
-                    *reinterpret_cast<float2*>(wo + c * 32 + e) = nkv > 0 ? make_float2(__uint_as_float(v[e]), __uint_as_float(v[e + 1])) : make_float2(0.f, 0.f);
-            }
-            *reinterpret_cast<float2*>(wo + HD) = make_float2(m_ref, l);
-        } else {
         const float inv_l = 1.0f / l;
 #pragma unroll 1
         for (int c = 0; c < 2; ++c) {
@@ -895,307 +352,10 @@ attn_fwd_tm_kernel(const __grid_constant__ AttnParams P) {
             }
         }
         if (q < P.Tq) P.lse[((long long)b * P.H + h) * P.Tq + q] = (m_ref + log2f(l)) * LN2;
-        }
     }
     tc_fence_before();
     __syncthreads();
     if (warp == 5) { tc_fence_after(); tmem_dealloc(tmem, 128); }
-}
-
-// ================================================================================================
-// forward, P-in-TMEM form with 128-key tiles and two threads per query row (measurement variant, aoz_attn_set_fwd_split(7))
-// ================================================================================================
-// Same ingredients as attn_fwd_tm_kernel, other balance: one S -> P -> P V round trip (~900 cycles through two mbarriers and the tensor
-// pipe) per 128 keys instead of per 64; two threads per row with SEPARATE references, row sums and O accumulators (S | O_a | O_b =
-// 256 TMEM columns, two CTAs of 8 softmax warps per SM), merged once at the end like the round-1 split-statistics kernel.
-constexpr int ATT_TM2_THREADS = 320;           // 8 softmax warps + producer + issuer
-constexpr int TM2_STAGES = 2;
-
-struct Tm2Smem {
-    static constexpr int Q = 0;
-    static constexpr int K = Q + TILE_BYTES;
-    static constexpr int V = K + TM2_STAGES * TILE_BYTES;
-    static constexpr int BAR = V + TM2_STAGES * TILE_BYTES;
-    static constexpr int XCH = BAR + 256;                   // [2][128] reference + [2][128] row sum, fp32: merge of the two key halves
-    static constexpr int TOTAL = XCH + 2048;
-};
-static_assert(2 * (Tm2Smem::TOTAL + 1024) <= 228 * 1024, "attention forward (128-key variant) must keep two CTAs per SM");
-
-__global__ void __launch_bounds__(ATT_TM2_THREADS, 2)
-attn_fwd_tm2_kernel(const __grid_constant__ AttnParams P) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = (uint64_t*)(smem + Tm2Smem::BAR);
-    uint64_t* q_full = bars;
-    uint64_t* kv_full = bars + 1;               // TM2_STAGES
-    uint64_t* kv_empty = bars + 1 + TM2_STAGES; // TM2_STAGES
-    uint64_t* s_ready = bars + 1 + 2 * TM2_STAGES;
-    uint64_t* p_ready = s_ready + 1;            // 256 arrivals
-    uint64_t* o_ready = p_ready + 1;
-    uint32_t* tmem_slot = (uint32_t*)(o_ready + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q_tiles = (P.Tq + TILE - 1) / TILE;
-    const int qt = blockIdx.x % q_tiles;
-    const int bh = blockIdx.x / q_tiles;
-    const int h = bh % P.H, b = bh / P.H;
-    const int q0 = qt * TILE;
-    const int nkv = (P.Tk + TILE - 1) / TILE;
-
-    if (threadIdx.x == 0) {
-        mbar_init(q_full, 1);
-        for (int i = 0; i < TM2_STAGES; ++i) { mbar_init(&kv_full[i], 1); mbar_init(&kv_empty[i], 1); }
-        mbar_init(s_ready, 1); mbar_init(p_ready, 256); mbar_init(o_ready, 1);
-        fence_mbar_init();
-    }
-    if (warp == 9) tmem_alloc(tmem_slot, 256);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-    const uint32_t tS = tmem, tOa = tmem + 128, tOb = tmem + 192;
-    pdl_enter();
-
-    if (warp == 8) {
-        if (lane == 0) {
-            tma_prefetch_desc(&P.tmQ); tma_prefetch_desc(&P.tmK); tma_prefetch_desc(&P.tmV);
-            mbar_arrive_expect_tx(q_full, TILE_BYTES);
-            tma_load_4d(smem + Tm2Smem::Q, &P.tmQ, q_full, 0, h, q0, b);
-            for (int j = 0; j < nkv; ++j) {
-                const int s = j % TM2_STAGES;
-                mbar_wait_relaxed(&kv_empty[s], ((j / TM2_STAGES) & 1) ^ 1);
-                mbar_arrive_expect_tx(&kv_full[s], 2 * TILE_BYTES);
-                tma_load_4d(smem + Tm2Smem::K + s * TILE_BYTES, &P.tmK, &kv_full[s], 0, h, j * TILE, b);
-                tma_load_4d(smem + Tm2Smem::V + s * TILE_BYTES, &P.tmV, &kv_full[s], 0, h, j * TILE, b);
-            }
-        }
-    } else if (warp == 9) {
-        const uint32_t idesc_qk = make_idesc_bf16(128, 128, 0, 0);
-        const uint32_t idesc_pv = make_idesc_bf16(128, 64, 0, 1);
-        const uint64_t dQ = desc_kmajor(smem_u32(smem + Tm2Smem::Q), 0);
-        const uint64_t dK = desc_kmajor(smem_u32(smem + Tm2Smem::K), 0);
-        const uint64_t dV = desc_rows_as_k(smem_u32(smem + Tm2Smem::V), 0);
-        auto issue_s = [&](int j) {
-            const int s = j % TM2_STAGES;
-            mbar_wait(&kv_full[s], (j / TM2_STAGES) & 1);
-            tc_fence_after();
-            if (elect_one_sync()) {
-                const uint64_t dk = dK + (uint64_t)(s * (TILE_BYTES >> 4));
-                umma_bf16(tS, dQ, dk, idesc_qk, 0u);
-#pragma unroll
-                for (int k = 1; k < 4; ++k) umma_bf16(tS, dQ + 2 * k, dk + 2 * k, idesc_qk, 1u);
-                umma_commit(s_ready);
-            }
-            __syncwarp();
-        };
-        mbar_wait(q_full, 0);
-        issue_s(0);
-        for (int j = 0; j < nkv; ++j) {
-            const int s = j % TM2_STAGES;
-            mbar_wait(p_ready, j & 1);
-            tc_fence_after();
-            if (elect_one_sync()) {
-                const uint64_t dv = dV + (uint64_t)(s * (TILE_BYTES >> 4));
-                const uint32_t acc = j > 0 ? 1u : 0u;
-                umma_bf16_ts(tOa, tS, dv, idesc_pv, acc);                           // keys 0..63: P words at columns [0, 32)
-#pragma unroll
-                for (int k = 1; k < 4; ++k) umma_bf16_ts(tOa, tS + 8 * k, dv + 128 * k, idesc_pv, 1u);
-                umma_bf16_ts(tOb, tS + 64, dv + 128 * 4, idesc_pv, acc);            // keys 64..127: P words at columns [64, 96)
-#pragma unroll
-                for (int k = 1; k < 4; ++k) umma_bf16_ts(tOb, tS + 64 + 8 * k, dv + 128 * (4 + k), idesc_pv, 1u);
-                umma_commit(&kv_empty[s]);
-                if (j + 1 == nkv) umma_commit(o_ready);
-            }
-            __syncwarp();
-            if (j + 1 < nkv) issue_s(j + 1);
-        }
-    } else {
-        const int qtr = warp & 3, hf = warp >> 2;
-        const int r = qtr * 32 + lane;
-        const uint32_t lane_off = (uint32_t)(qtr * 32) << 16;
-        const uint32_t tSh = tS + hf * 64;                     // this thread's 64 score columns; its P words go over their front
-        const uint32_t tOx = hf == 0 ? tOa : tOb;
-        float* xm = (float*)(smem + Tm2Smem::XCH);
-        float* xl = xm + 256;
-        const float sl2 = P.scale * LOG2E;
-        float m_ref = -INFINITY, l = 0.f;
-        auto exp_pass = [&](uint32_t* w, float& lsum) -> uint32_t {
-            uint32_t v[2][16];
-            uint32_t mw = 0;
-            float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-            tmem_ld16(tSh + lane_off, v[0]);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                tc_wait_ld();
-                if (c + 1 < 4) tmem_ld16(tSh + lane_off + (c + 1) * 16, v[(c + 1) & 1]);
-                const uint32_t* cv = v[c & 1];
-#pragma unroll
-                for (int e = 0; e < 16; e += 4) {
-                    float p[4];
-#pragma unroll
-                    for (int t = 0; t < 4; ++t) p[t] = fast_exp2(fmaf(__uint_as_float(cv[e + t]), sl2, -m_ref));
-                    a0 += p[0]; a1 += p[1]; a2 += p[2]; a3 += p[3];
-                    const uint32_t w0 = pack_bf16(p[0], p[1]), w1 = pack_bf16(p[2], p[3]);
-                    w[c * 8 + (e >> 1)] = w0; w[c * 8 + (e >> 1) + 1] = w1;
-                    mw = max_u16x2(mw, max_u16x2(w0, w1));
-                }
-            }
-            lsum = (a0 + a1) + (a2 + a3);
-            return mw;
-        };
-        auto max_pass = [&](int kvalid) -> float {             // kvalid: valid columns of THIS half
-            float mx = -3.0e38f;
-#pragma unroll 1
-            for (int c = 0; c < 2; ++c) {
-                uint32_t v[32];
-                tmem_ld32(tSh + lane_off + c * 32, v);
-                tc_wait_ld();
-#pragma unroll
-                for (int e = 0; e < 32; ++e)
-                    if (c * 32 + e < kvalid) mx = fmaxf(mx, __uint_as_float(v[e]));
-            }
-            return mx;
-        };
-        auto exp_pass_masked = [&](int kvalid, uint32_t* w, float& lsum) {
-            float acc = 0.f;
-#pragma unroll 1
-            for (int c = 0; c < 2; ++c) {
-                uint32_t v[32];
-                tmem_ld32(tSh + lane_off + c * 32, v);
-                tc_wait_ld();
-#pragma unroll
-                for (int e = 0; e < 32; e += 2) {
-                    const int ka = c * 32 + e;
-                    const float p0 = ka < kvalid ? fast_exp2(fmaf(__uint_as_float(v[e]), sl2, -m_ref)) : 0.f;
-                    const float p1 = ka + 1 < kvalid ? fast_exp2(fmaf(__uint_as_float(v[e + 1]), sl2, -m_ref)) : 0.f;
-                    acc += p0 + p1;
-                    const uint32_t pk = pack_bf16(p0, p1);
-                    if (c == 0) w[e >> 1] = pk; else w[16 + (e >> 1)] = pk;
-                }
-            }
-            lsum = acc;
-        };
-        for (int j = 0; j < nkv; ++j) {
-            mbar_wait(s_ready, j & 1);
-            tc_fence_after();
-            const int kvalid = P.Tk - j * TILE - hf * 64;        // valid keys among this thread's 64 columns (may be <= 0)
-            uint32_t w[32];
-            float lsum = 0.f;
-            if (j == 0) {
-                m_ref = max_pass(kvalid) * sl2;                  // (-3e38 * sl2 when this half has no valid key: every P is masked to 0)
-                if (kvalid >= 64) exp_pass(w, lsum); else exp_pass_masked(kvalid, w, lsum);
-            } else {
-                bool need;
-                if (kvalid >= 64) {
-                    const uint32_t mw = exp_pass(w, lsum);
-                    need = (mw & 0xffffu) > 0x4380u || (mw >> 16) > 0x4380u;
-                } else {
-                    need = max_pass(kvalid) * sl2 - m_ref > 8.0f;
-                    if (!__any_sync(0xffffffffu, need)) exp_pass_masked(kvalid, w, lsum);
-                }
-                if (__any_sync(0xffffffffu, need)) {
-                    const float m_new = fmaxf(m_ref, max_pass(kvalid) * sl2);
-                    const float alpha = fast_exp2(m_ref - m_new);
-#pragma unroll 1
-                    for (int c = 0; c < 2; ++c) {
-                        uint32_t v[32];
-                        tmem_ld32(tOx + lane_off + c * 32, v);
-                        tc_wait_ld();
-#pragma unroll
-                        for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * alpha);
-                        tmem_st32(tOx + lane_off + c * 32, v);
-                        tc_wait_st();
-                    }
-                    l *= alpha;
-                    m_ref = m_new;
-                    if (kvalid >= 64) exp_pass(w, lsum); else exp_pass_masked(kvalid, w, lsum);
-                }
-            }
-            l += lsum;
-            tmem_st32(tSh + lane_off, w);
-            tc_wait_st();
-            tc_fence_before();
-            mbar_arrive(p_ready);
-        }
-        mbar_wait(o_ready, 0);
-        tc_fence_after();
-        // combine the two halves: O = (O_a 2^(m_a - m) + O_b 2^(m_b - m)) / (l_a 2^(m_a - m) + l_b 2^(m_b - m))
-        xm[hf * 128 + r] = m_ref;
-        xl[hf * 128 + r] = l;
-        named_bar_sync(1, 256);
-        const float m_o = xm[(hf ^ 1) * 128 + r], l_o = xl[(hf ^ 1) * 128 + r];
-        const float m = fmaxf(m_ref, m_o);
-        const float w_me = fast_exp2(m_ref - m), w_o = fast_exp2(m_o - m);
-        const float wa = hf == 0 ? w_me : w_o, wb = hf == 0 ? w_o : w_me;
-        const float lt = l * w_me + l_o * w_o;
-        const float inv_l = 1.0f / lt;
-        const int q = q0 + r;
-        {
-            const int c = hf;
-            uint32_t va[32], vb[32];
-            tmem_ld32(tOa + lane_off + c * 32, va);
-            tmem_ld32(tOb + lane_off + c * 32, vb);
-            tc_wait_ld();
-            if (q < P.Tq) {
-                __nv_bfloat16* dst = P.O + ((long long)b * P.Tq + q) * P.ldo + h * HD + c * 32;
-                const float sa = wa * inv_l, sb = wb * inv_l;
-#pragma unroll
-                for (int e = 0; e < 32; e += 8) {
-                    float f[8];
-#pragma unroll
-                    for (int t = 0; t < 8; ++t) f[t] = fmaf(__uint_as_float(va[e + t]), sa, __uint_as_float(vb[e + t]) * sb);
-                    uint4 o;
-                    o.x = pack_bf16(f[0], f[1]); o.y = pack_bf16(f[2], f[3]); o.z = pack_bf16(f[4], f[5]); o.w = pack_bf16(f[6], f[7]);
-                    *reinterpret_cast<uint4*>(dst + e) = o;
-                }
-            }
-        }
-        if (hf == 0 && q < P.Tq) P.lse[((long long)b * P.H + h) * P.Tq + q] = (m + log2f(lt)) * LN2;
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 9) { tc_fence_after(); tmem_dealloc(tmem, 256); }
-}
-
-// Merge the key shares of the units that attn_fwd_tm_kernel cut (see there): one thread per (unit, row, 8 output columns).
-//   m = max_i m_i,  L = sum_i l_i 2^(m_i - m),  O = sum_i O_i 2^(m_i - m) / L,  LSE = (m + log2 L) ln 2
-__global__ void __launch_bounds__(256)
-attn_fwd_combine_kernel(const float* __restrict__ ws, int n_units, int unit0, int split, int B, int H, int Tq, __nv_bfloat16* __restrict__ O,
-                        long long ldo, float* __restrict__ lse) {
-    pdl_enter();
-    const int q_tiles = (Tq + TILE - 1) / TILE;
-    const long long total = (long long)n_units * TILE * 8;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const int c8 = (int)(i & 7);
-        const long long ur = i >> 3;
-        const int r = (int)(ur % TILE);
-        const int u = (int)(ur / TILE);
-        const int unit = unit0 + u;
-        const int qt = unit % q_tiles, bh = unit / q_tiles;
-        const int h = bh % H, b = bh / H;
-        const int q = qt * TILE + r;
-        if (q >= Tq) continue;
-        const float* base = ws + ((long long)u * split * TILE + r) * (HD + 4);
-        const long long pstride = (long long)TILE * (HD + 4);
-        float m = -INFINITY;
-        for (int p = 0; p < split; ++p) m = fmaxf(m, base[p * pstride + HD]);
-        float L = 0.f, acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        for (int p = 0; p < split; ++p) {
-            const float* wp = base + p * pstride;
-            const float lp = wp[HD + 1];
-            if (lp <= 0.f) continue;                                     // empty share
-            const float w = fast_exp2(wp[HD] - m);
-            L = fmaf(lp, w, L);
-            const float4 a = *reinterpret_cast<const float4*>(wp + c8 * 8), c = *reinterpret_cast<const float4*>(wp + c8 * 8 + 4);
-            acc[0] = fmaf(a.x, w, acc[0]); acc[1] = fmaf(a.y, w, acc[1]); acc[2] = fmaf(a.z, w, acc[2]); acc[3] = fmaf(a.w, w, acc[3]);
-            acc[4] = fmaf(c.x, w, acc[4]); acc[5] = fmaf(c.y, w, acc[5]); acc[6] = fmaf(c.z, w, acc[6]); acc[7] = fmaf(c.w, w, acc[7]);
-        }
-        const float inv = 1.0f / L;
-        uint4 o;
-        o.x = pack_bf16(acc[0] * inv, acc[1] * inv); o.y = pack_bf16(acc[2] * inv, acc[3] * inv);
-        o.z = pack_bf16(acc[4] * inv, acc[5] * inv); o.w = pack_bf16(acc[6] * inv, acc[7] * inv);
-        *reinterpret_cast<uint4*>(O + ((long long)b * Tq + q) * ldo + h * HD + c8 * 8) = o;
-        if (c8 == 0) lse[((long long)b * H + h) * Tq + q] = (m + log2f(L)) * LN2;
-    }
 }
 
 // ================================================================================================
@@ -1304,7 +464,7 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = *tmem_slot;
-    const uint32_t tS = tmem, tdP = tmem + 128, tdV = tmem + 256, tdK = tmem + 320, tdQ = tmem + 384;
+    const uint32_t tS = tmem, tdP = tmem + 128, tdV = tmem + 256, tdK = tmem + 320;
     pdl_enter();          // prologue done: wait for the previous kernel's results before the first global access
 
     if (warp == BWD_CW) {
@@ -1328,13 +488,10 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
         // stage-0 descriptors plus integer offsets on the address field (16-byte units).
         const uint32_t idesc_s = make_idesc_bf16(128, 128, 0, 0);
         const uint32_t idesc_acc = make_idesc_bf16(128, 64, 1, 1);           // A = P / dS read MN-major, B = dO / Q read MN-major
-        const uint32_t idesc_dq = make_idesc_bf16(128, 64, 0, 1);            // A = dS read K-major (over keys), B = K read MN-major
         const uint64_t dK_k = desc_kmajor(smem_u32(smem + KvSmem::K), 0), dV_k = desc_kmajor(smem_u32(smem + KvSmem::V), 0);
         const uint64_t dQ_k = desc_kmajor(smem_u32(smem + KvSmem::Q), 0), dDO_k = desc_kmajor(smem_u32(smem + KvSmem::DO), 0);
         const uint64_t dQ_r = desc_rows_as_k(smem_u32(smem + KvSmem::Q), 0), dDO_r = desc_rows_as_k(smem_u32(smem + KvSmem::DO), 0);
-        const uint64_t dK_r = desc_rows_as_k(smem_u32(smem + KvSmem::K), 0);
         const uint64_t dP_r = desc_ptile_rows_as_k(smem_u32(smem + KvSmem::PT), 0), dDS_r = desc_ptile_rows_as_k(smem_u32(smem + KvSmem::DST), 0);
-        const uint32_t sDS = smem_u32(smem + KvSmem::DST);
         constexpr uint64_t STG = TILE_BYTES >> 4;
         auto issue_scores = [&](int i) {
             const int s = i % BWD_STAGES;
@@ -1372,11 +529,6 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
                 umma_bf16(tdK, dDS_r, q, idesc_acc, acc);
 #pragma unroll
                 for (int k = 1; k < 8; ++k) umma_bf16(tdK, dDS_r + 128 * k, q + 128 * k, idesc_acc, 1u);
-                if (P.fuse_dq) {
-                    // the only KV tile: dQ(i) = dS(i) K is complete after this tile (the compute warps drain it during tile i+1)
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) umma_bf16(tdQ, desc_ptile(sDS, k), dK_r + 128 * k, idesc_dq, k > 0 ? 1u : 0u);
-                }
                 umma_commit(&q_empty[s]);
                 umma_commit(pd_free);
                 if (i == nq - 1) umma_commit(acc_ready);
@@ -1398,32 +550,6 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
             const long long idx = ((long long)b * P.H + h) * P.Tq + q;
             nx_lse = q < P.Tq ? P.lse[idx] : INFINITY;       // +inf -> P = 0 for padded queries
             nx_d = q < P.Tq ? P.Dvec[idx] : 0.f;
-        };
-        // fused dQ (cross-attention): each of the four warps of a lane quarter stores 16 of the 64 columns of Q tile `i`
-        auto drain_dq = [&](int i) {
-            uint32_t v[16];
-            tmem_ld16(tdQ + lane_off + hf * 16, v);
-            tc_wait_ld();
-            const int q = i * TILE + r;
-            if (q < P.Tq && P.fuse_dq == 2) {
-                // this KV tile's share of dQ(i): summed in fp32 across the KV-tile CTAs (unscaled; the convert kernel applies `scale`)
-                float* dst = P.dQacc + (((long long)b * P.H + h) * P.Tq + q) * HD + hf * 16;
-#pragma unroll
-                for (int e = 0; e < 16; e += 4)
-                    red_add_v4(dst + e, __uint_as_float(v[e]), __uint_as_float(v[e + 1]), __uint_as_float(v[e + 2]), __uint_as_float(v[e + 3]));
-            } else if (q < P.Tq) {
-                __nv_bfloat16* dst = P.dQ + ((long long)b * P.Tq + q) * P.lddq + h * HD + hf * 16;
-                const float mul = P.scale;
-#pragma unroll
-                for (int e = 0; e < 16; e += 8) {
-                    uint4 o;
-                    o.x = pack_bf16(__uint_as_float(v[e]) * mul, __uint_as_float(v[e + 1]) * mul);
-                    o.y = pack_bf16(__uint_as_float(v[e + 2]) * mul, __uint_as_float(v[e + 3]) * mul);
-                    o.z = pack_bf16(__uint_as_float(v[e + 4]) * mul, __uint_as_float(v[e + 5]) * mul);
-                    o.w = pack_bf16(__uint_as_float(v[e + 6]) * mul, __uint_as_float(v[e + 7]) * mul);
-                    *reinterpret_cast<uint4*>(dst + e) = o;
-                }
-            }
         };
         fetch_vec(0);
         for (int i = 0; i < nq; ++i) {
@@ -1470,11 +596,7 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
                 // chunk 0 waits in registers: the previous tile's dV / dK MMAs (issued when that tile's P / dS were complete)
                 // still read these smem tiles for the first few hundred cycles of this tile
                 if (c == 1) {
-                    if (i > 0) {
-                        mbar_wait(pd_free, (i - 1) & 1);
-                        // dQ(i-1) retired with those MMAs; dQ(i) is issued only after every compute thread arrived at pds_ready(i)
-                        if (P.fuse_dq) { tc_fence_after(); drain_dq(i - 1); }
-                    }
+                    if (i > 0) mbar_wait(pd_free, (i - 1) & 1);
                     store_p_16(sP, r, hf * 32, hp[0]);
                     store_p_16(sDS, r, hf * 32, hd[0]);
                     store_p_16(sP, r, hf * 32 + 16, hp[1]);
@@ -1487,7 +609,6 @@ attn_bwd_dkv_kernel(const __grid_constant__ AttnParams P) {
         }
         mbar_wait(acc_ready, 0);
         tc_fence_after();
-        if (P.fuse_dq) drain_dq(nq - 1);
         const int key = k0 + r;                              // accumulator rows are keys
         {
             const int which = hf >> 1, c = hf & 1;               // warps hf 0,1 store dV chunks 0,1; hf 2,3 store dK chunks 0,1
@@ -2114,26 +1235,6 @@ attn_dq_tiles_convert_kernel(const float* __restrict__ acc, __nv_bfloat16* __res
     }
 }
 
-// dQ = scale * dQacc: fp32 [B, H, Tq, 64] (head-major accumulation buffer) -> bf16 [B, Tq, H, 64] with a row stride
-__global__ void __launch_bounds__(256)
-attn_dq_convert_kernel(const float* __restrict__ acc, __nv_bfloat16* __restrict__ dq, long long lddq, int B, int H, int Tq, float scale) {
-    pdl_enter();
-    const long long total = (long long)B * H * Tq * 8;                    // one work item = 8 elements
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const int part = (int)(i & 7);
-        const long long row = i >> 3;                                     // (b, h, q)
-        const int q = (int)(row % Tq);
-        const long long bh = row / Tq;
-        const int h = (int)(bh % H), b = (int)(bh / H);
-        const float4 a0 = *reinterpret_cast<const float4*>(acc + row * HD + part * 8);
-        const float4 a1 = *reinterpret_cast<const float4*>(acc + row * HD + part * 8 + 4);
-        uint4 o;
-        o.x = pack_bf16(a0.x * scale, a0.y * scale); o.y = pack_bf16(a0.z * scale, a0.w * scale);
-        o.z = pack_bf16(a1.x * scale, a1.y * scale); o.w = pack_bf16(a1.z * scale, a1.w * scale);
-        *reinterpret_cast<uint4*>(dq + ((long long)b * Tq + q) * lddq + h * HD + part * 8) = o;
-    }
-}
-
 static int make_qkv_map(CUtensorMap* m, const void* base, long long ld, int B, int H, int T, int rows = TILE) {
     uint64_t dims[4] = {(uint64_t)HD, (uint64_t)H, (uint64_t)T, (uint64_t)B};
     uint64_t strides[3] = {(uint64_t)HD * 2, (uint64_t)ld * 2, (uint64_t)T * (uint64_t)ld * 2};
@@ -2147,44 +1248,8 @@ using namespace aoz;
 
 extern "C" {
 
-static int g_fwd_split = 2;       // 2 = P-in-TMEM kernel (default), 1 = split-statistics kernel (P through smem), 0 = shared-maximum kernel
-
-// Tail-wave plan of the P-in-TMEM forward: how many CTAs take whole units, and into how many key shares each remaining unit is cut.
-static void fwd_tail_plan(int units, int kv_tiles, int* full, int* split) {
-    const int slots = TM_CTAS * sm_count();
-    const int rem = units % slots;
-    *full = units; *split = 1;
-    if (units < slots || rem == 0 || 4 * rem > 3 * slots || kv_tiles < 4) return;     // one wave, or a tail that is nearly full anyway
-    int s = slots / rem;                                                               // shares that fit beside each other
-    if (s > kv_tiles / 2) s = kv_tiles / 2;                                            // at least two key tiles per share
-    if (s < 2) return;
-    *full = units - rem; *split = s;
-}
-// Measured (profiles/r02_attn_bench_tail_split.json): 4096 tokens x 10 heads 729 against 718 TFLOP/s, 1024 tokens x 20 heads 410 against
-// 467 -- co-resident CTAs share the MUFU pipe, so a thinly filled last "wave" simply runs faster per CTA; the cut only adds
-// prologues and a merge launch.  Off by default.
-static int g_fwd_tail_split = 0;
-// experiment switch: 1 = cut the units of the last, partly filled wave along the keys, 0 = every CTA takes a whole unit (default)
-int aoz_attn_set_fwd_tail_split(int on) { g_fwd_tail_split = on ? 1 : 0; return AOZ_OK; }
-
-long long aoz_attn_fwd_workspace_floats(int B, int H, int Tq, int Tk) {
-    int full, split;
-    fwd_tail_plan(B * H * ((Tq + TILE - 1) / TILE), (Tk + KT - 1) / KT, &full, &split);
-    const int units = B * H * ((Tq + TILE - 1) / TILE);
-    return split > 1 ? (long long)(units - full) * split * TILE * (HD + 4) : 0;
-}
-
-int aoz_attn_fwd_ws(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, void* o, long long ldo,
-                    void* lse, int B, int H, int Tq, int Tk, float scale, void* workspace, void* stream);
-
 int aoz_attn_fwd(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, void* o, long long ldo,
                  void* lse, int B, int H, int Tq, int Tk, float scale, void* stream) {
-    return aoz_attn_fwd_ws(q, ldq, k, ldk, v, ldv, o, ldo, lse, B, H, Tq, Tk, scale, nullptr, stream);
-}
-
-// `workspace`: aoz_attn_fwd_workspace_floats(B, H, Tq, Tk) floats, or null (then every CTA takes a whole unit)
-int aoz_attn_fwd_ws(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, void* o, long long ldo,
-                    void* lse, int B, int H, int Tq, int Tk, float scale, void* workspace, void* stream) {
     AOZ_CHECK_ARG(q && k && v && o && lse, "aoz_attn_fwd: null pointer");
     AOZ_CHECK_ARG(B > 0 && H > 0 && Tq > 0 && Tk > 0, "aoz_attn_fwd: empty problem");
     AOZ_CHECK_ARG((ldq % 8) == 0 && (ldk % 8) == 0 && (ldv % 8) == 0 && (ldo % 8) == 0, "aoz_attn_fwd: strides must be multiples of 8");
@@ -2192,72 +1257,32 @@ int aoz_attn_fwd_ws(const void* q, long long ldq, const void* k, long long ldk, 
     memset(&P, 0, sizeof(P));
     int rc;
     if ((rc = make_qkv_map(&P.tmQ, q, ldq, B, H, Tq)) != AOZ_OK) return rc;
-    const int kv_rows = (g_fwd_split >= 2 && g_fwd_split != 7) ? KT : TILE;          // the P-in-TMEM kernel streams 64-key tiles
-    if ((rc = make_qkv_map(&P.tmK, k, ldk, B, H, Tk, kv_rows)) != AOZ_OK) return rc;
-    if ((rc = make_qkv_map(&P.tmV, v, ldv, B, H, Tk, kv_rows)) != AOZ_OK) return rc;
+    if ((rc = make_qkv_map(&P.tmK, k, ldk, B, H, Tk, KT)) != AOZ_OK) return rc;       // the forward streams 64-key tiles
+    if ((rc = make_qkv_map(&P.tmV, v, ldv, B, H, Tk, KT)) != AOZ_OK) return rc;
     P.B = B; P.H = H; P.Tq = Tq; P.Tk = Tk; P.scale = scale;
     P.O = (__nv_bfloat16*)o; P.ldo = ldo; P.lse = (float*)lse;
     static bool attr = false;
-    if (!attr) {
-        cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_tm_kernel<0x8888u>, cudaFuncAttributeMaxDynamicSharedMemorySize, TmSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_tm_kernel<0x8080u>, cudaFuncAttributeMaxDynamicSharedMemorySize, TmSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_tm_kernel<0u>, cudaFuncAttributeMaxDynamicSharedMemorySize, TmSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_tm_kernel<0xAAAAu>, cudaFuncAttributeMaxDynamicSharedMemorySize, TmSmem::TOTAL);
-        cudaFuncSetAttribute(attn_fwd_tm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Tm2Smem::TOTAL);
-        attr = true;
-    }
-    int grid = B * H * ((Tq + TILE - 1) / TILE);
-    P.fwd_full = grid; P.fwd_split = 1; P.fwd_ws = nullptr;
-    const int units = grid;
-    if (g_fwd_split >= 2 && g_fwd_split != 7 && workspace != nullptr && g_fwd_tail_split) {
-        fwd_tail_plan(units, (Tk + KT - 1) / KT, &P.fwd_full, &P.fwd_split);
-        if (P.fwd_split > 1) { P.fwd_ws = (float*)workspace; grid = P.fwd_full + (units - P.fwd_full) * P.fwd_split; }
-    }
-    if (g_fwd_split == 7) launch_k(attn_fwd_tm2_kernel, dim3(units), dim3(ATT_TM2_THREADS), (size_t)(Tm2Smem::TOTAL), (cudaStream_t)stream, P);
-    else if (g_fwd_split == 6) launch_k(attn_fwd_tm_kernel<0x8888u>, dim3(grid), dim3(ATT_TM_THREADS), (size_t)(TmSmem::TOTAL), (cudaStream_t)stream, P);
-    else if (g_fwd_split == 3) launch_k(attn_fwd_tm_kernel<0x8080u>, dim3(grid), dim3(ATT_TM_THREADS), (size_t)(TmSmem::TOTAL), (cudaStream_t)stream, P);
-    else if (g_fwd_split == 2) launch_k(attn_fwd_tm_kernel<0u>, dim3(grid), dim3(ATT_TM_THREADS), (size_t)(TmSmem::TOTAL), (cudaStream_t)stream, P);
-    else if (g_fwd_split == 4) launch_k(attn_fwd_tm_kernel<0xAAAAu>, dim3(grid), dim3(ATT_TM_THREADS), (size_t)(TmSmem::TOTAL), (cudaStream_t)stream, P);
-    else if (g_fwd_split) launch_k(attn_fwd_split_kernel, dim3(grid), dim3(ATT_FWD_THREADS), (size_t)(FwdSmem::TOTAL), (cudaStream_t)stream, P);
-    else launch_k(attn_fwd_kernel, dim3(grid), dim3(ATT_FWD_THREADS), (size_t)(FwdSmem::TOTAL), (cudaStream_t)stream, P);
-    AOZ_CHECK_LAUNCH("attn_fwd_kernel");
-    if (P.fwd_split > 1) {
-        const int n_tail = units - P.fwd_full;
-        long long blocks = ((long long)n_tail * TILE * 8 + 255) / 256;
-        launch_k(attn_fwd_combine_kernel, dim3((int)blocks), dim3(256), (size_t)(0), (cudaStream_t)stream, (const float*)P.fwd_ws, n_tail, P.fwd_full,
-                 P.fwd_split, B, H, Tq, (__nv_bfloat16*)o, ldo, (float*)lse);
-        AOZ_CHECK_LAUNCH("attn_fwd_combine_kernel");
-    }
+    if (!attr) { cudaFuncSetAttribute(attn_fwd_tm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TmSmem::TOTAL); attr = true; }
+    launch_k(attn_fwd_tm_kernel, dim3(B * H * ((Tq + TILE - 1) / TILE)), dim3(ATT_TM_THREADS), (size_t)(TmSmem::TOTAL), (cudaStream_t)stream, P);
+    AOZ_CHECK_LAUNCH("attn_fwd_tm_kernel");
     return AOZ_OK;
 }
 
-// experiment switch: 2 = P-in-TMEM forward (default), 1 = split-statistics forward (P through shared memory), 0 = shared-maximum forward
-// (2: every exponential on the MUFU pipe -- measured as fast as any split, and LSE keeps ex2.approx accuracy; 3 / 6 / 4: the same
-// kernel with 1/8, 1/4, 1/2 of them on the FMA pipe -- measurement variants: 724 / 697 / 584 TFLOP/s against 718 for none)
-int aoz_attn_set_fwd_split(int mode) { g_fwd_split = mode < 0 ? 0 : (mode > 7 ? 2 : mode); return AOZ_OK; }
-
-// D vector [B, H, Tq] + the fp32 dQ accumulation buffer [B, H, Tq, 64] of the one-kernel backward
-static long long bwd_vec_floats(int B, int H, int Tq) { return (((long long)B * H * Tq + 31) / 32) * 32; }      // 128-byte granules
+// one per-row vector [B, H, Tq] of the backward workspace (D, lse2), padded to 128-byte granules
+static long long bwd_vec_floats(int B, int H, int Tq) { return (((long long)B * H * Tq + 31) / 32) * 32; }
 long long aoz_attn_bwd_workspace_floats(int B, int H, int Tq) {
     // D and lse2 vectors, the dQ tile buffer, and (one KV tile, Q tiles cut over several CTAs) one dK and one dV tile per (b, h)
     return 2 * bwd_vec_floats(B, H, Tq) + (long long)B * H * ((Tq + TILE - 1) / TILE + 2) * TILE * HD;
 }
 
-// Measured (profiles/r01_cross_bwd_ab.txt): alone the fused kernel wins (1024 queries x 77 keys x 20 heads: 48.1 -> 30.6 us) and the
-// per-kernel times inside the step drop by 1.2 ms, but the event-timed training step is 1.5 ms SLOWER (139.3 vs 137.8 ms, two
-// runs each): one 80-CTA kernel per layer leaves 68 SMs idle for 25 us where the 640-CTA dQ kernel filled them.  Off by default.
-static int g_fuse_cross_dq = 0;
-// Self-attention (more than one KV tile): 1 = ONE kernel -- the dK/dV kernel also forms dQ(i) = dS(i) K for every Q tile and adds it
-// into an fp32 buffer with red.global.add (5 MMAs and one exponential pass per tile pair instead of 7 and two; the sum over KV tiles
-// is not bit-reproducible), 0 = dK/dV kernel + dQ kernel (bit-reproducible).
-// 2 = attn_bwd_fused_kernel (key-major scores, P^T / dS^T in tensor memory, bulk-reduced dQ; default), 1 = the dK/dV kernel with a
-// per-thread red.global drain (measured slower than two kernels; kept for the record), 0 = two kernels.
+// 2 = attn_bwd_fused_kernel (key-major scores, P^T / dS^T in tensor memory, bulk-reduced dQ; default), 0 = dK/dV kernel + dQ kernel
+// (bit-reproducible).  Any other value is refused rather than mapped onto one of the two.
 static int g_bwd_fused = 2;
-int aoz_attn_set_bwd_mode(int fused) { g_bwd_fused = fused < 0 ? 0 : (fused > 2 ? 2 : fused); return AOZ_OK; }
-// experiment switch: 1 = cross-attention (Tk <= 128) backward runs as ONE kernel, 0 = dK/dV + dQ kernels (default)
-int aoz_attn_set_fused_cross_bwd(int on) { g_fuse_cross_dq = on ? 1 : 0; return AOZ_OK; }
+int aoz_attn_set_bwd_mode(int fused) {
+    AOZ_CHECK_ARG(fused == 0 || fused == 2, "aoz_attn_set_bwd_mode: mode must be 2 (one kernel) or 0 (two kernels)");
+    g_bwd_fused = fused;
+    return AOZ_OK;
+}
 
 int aoz_attn_bwd(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, const void* o,
                  long long ldo, const void* d_o, long long lddo, const void* lse, void* dq, long long lddq, void* dk,
@@ -2337,25 +1362,8 @@ int aoz_attn_bwd(const void* q, long long ldq, const void* k, long long ldk, con
         cudaFuncSetAttribute(attn_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DqSmem::TOTAL);
         attr = true;
     }
-    // one KV tile (cross-attention, 77 text tokens): the dK/dV kernel's dS tile is all dQ needs, so it computes dQ as well and
-    // the dQ launch (one prologue-bound CTA per Q tile: 24..44 us for a few GFLOP) disappears
-    P.fuse_dq = (Tk <= TILE && g_fuse_cross_dq) ? 1 : ((Tk > TILE && g_bwd_fused == 1) ? 2 : 0);
-    if (P.fuse_dq == 2) {
-        P.dQacc = acc_ws;
-        cudaError_t e = cudaMemsetAsync(P.dQacc, 0, sizeof(float) * (size_t)B * H * Tq * HD, s);
-        if (e != cudaSuccess) { set_error("aoz_attn_bwd: memset: %s", cudaGetErrorString(e)); return AOZ_ERR_CUDA; }
-    }
     launch_k(attn_bwd_dkv_kernel, dim3(B * H * ((Tk + TILE - 1) / TILE)), dim3(ATT_BWD_THREADS), (size_t)(KvSmem::TOTAL), s, P);
     AOZ_CHECK_LAUNCH("attn_bwd_dkv_kernel");
-    if (P.fuse_dq == 1) return AOZ_OK;
-    if (P.fuse_dq == 2) {
-        const long long items = (long long)B * H * Tq * 8;
-        long long blocks = (items + 255) / 256;
-        if (blocks > sm_count() * 16) blocks = sm_count() * 16;
-        launch_k(attn_dq_convert_kernel, dim3((int)blocks), dim3(256), (size_t)(0), s, (const float*)P.dQacc, (__nv_bfloat16*)dq, lddq, B, H, Tq, scale);
-        AOZ_CHECK_LAUNCH("attn_dq_convert_kernel");
-        return AOZ_OK;
-    }
     launch_k(attn_bwd_dq_kernel, dim3(B * H * ((Tq + TILE - 1) / TILE)), dim3(ATT_BWD_THREADS), (size_t)(DqSmem::TOTAL), s, P);
     AOZ_CHECK_LAUNCH("attn_bwd_dq_kernel");
     return AOZ_OK;

@@ -209,9 +209,6 @@ def conv_wgrad(dy, x, ks, *, stride=1, pad=1, grad_w=None, accumulate=False, cin
 # ------------------------------------------------------------------------------------------------------------
 # attention
 # ------------------------------------------------------------------------------------------------------------
-_ATTN_FWD_TAIL_SPLIT = False          # aoz_attn_set_fwd_tail_split(1) + this flag: the tail-wave key split (measured no faster)
-
-
 def attn_fwd(q, k, v, scale):
     """q: [B,Tq,H,64], k/v: [B,Tk,H,64] (views with row stride allowed: last two dims dense). -> (o, lse)."""
     B, Tq, H, D = q.shape
@@ -219,11 +216,9 @@ def attn_fwd(q, k, v, scale):
     assert D == 64
     o = torch.empty((B, Tq, H, D), dtype=BF16, device=q.device)
     lse = torch.empty((B, H, Tq), dtype=torch.float32, device=q.device)
-    nws = _lib.query("aoz_attn_fwd_workspace_floats", B, H, Tq, Tk) if _ATTN_FWD_TAIL_SPLIT else 0      # key shares of the tail wave
-    ws = workspace(nws, q.device).data_ptr() if nws > 0 else 0
-    _lib.call("aoz_attn_fwd_ws", q.data_ptr(), q.stride(1), k.data_ptr(), k.stride(1), v.data_ptr(), v.stride(1),
-              o.data_ptr(), o.stride(1), lse.data_ptr(), B, H, Tq, Tk, float(scale), ws, _stream())
-    _count(2 if nws > 0 else 1)
+    _lib.call("aoz_attn_fwd", q.data_ptr(), q.stride(1), k.data_ptr(), k.stride(1), v.data_ptr(), v.stride(1),
+              o.data_ptr(), o.stride(1), lse.data_ptr(), B, H, Tq, Tk, float(scale), _stream())
+    _count(1)
     return o, lse
 
 

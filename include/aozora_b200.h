@@ -102,21 +102,9 @@ int aoz_pack_conv_weight(const void* w, int Cout, int Cin, int ks, int CinPad, i
  * lse: [B, H, Tq] fp32 (log-sum-exp of the scaled scores, natural log). */
 int aoz_attn_fwd(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, void* o, long long ldo,
                  void* lse, int B, int H, int Tq, int Tk, float scale, void* stream);
-/* The same with a caller-owned workspace of aoz_attn_fwd_workspace_floats(B, H, Tq, Tk) floats: the P-in-TMEM forward cuts the (b, h,
- * Q tile) units of its last, partly filled wave of CTAs along the keys and merges the shares (a null workspace: whole units only). */
-int aoz_attn_fwd_ws(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, void* o, long long ldo,
-                    void* lse, int B, int H, int Tq, int Tk, float scale, void* workspace, void* stream);
-long long aoz_attn_fwd_workspace_floats(int B, int H, int Tq, int Tk);
-/* experiment switch: 1 = cut the tail wave's units along the keys, 0 = whole units only (default: the cut measured no faster) */
-int aoz_attn_set_fwd_tail_split(int on);
-/* experiment switch: 2 = P-in-TMEM forward kernel (64-key tiles, double-buffered scores, P V with A read from tensor memory;
- * default), 1 = split-statistics forward kernel (P through shared memory), 0 = shared-maximum forward kernel */
-int aoz_attn_set_fwd_split(int mode);
-/* experiment switch: 1 = with a single KV tile (cross-attention, Tk <= 128) the dK/dV kernel also produces dQ and the dQ
- * launch is skipped, 0 = always two kernels (default: the fused form measured slower inside the training step) */
-int aoz_attn_set_fused_cross_bwd(int on);
-/* experiment switch, self-attention backward (Tk > 128): 1 = one kernel, dQ summed over the KV tiles in fp32 with red.global.add
- * (default; not bit-reproducible), 0 = dK/dV kernel + dQ kernel (bit-reproducible) */
+/* backward form: 2 = one kernel, dQ (and with a single KV tile dK / dV) summed over CTAs in fp32 by bulk reduce-add (default;
+ * not bit-reproducible), 0 = dK/dV kernel + dQ kernel (bit-reproducible; also taken under 2 when Tq % 4 != 0).  Any other
+ * value returns AOZ_ERR_ARG and leaves the form unchanged. */
 int aoz_attn_set_bwd_mode(int fused);
 long long aoz_attn_bwd_workspace_floats(int B, int H, int Tq);
 int aoz_attn_bwd(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv, const void* o,

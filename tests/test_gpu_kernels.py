@@ -378,14 +378,18 @@ def test_conv_fused_time_embedding_and_residual():
     check(ops.conv_fwd(x, wf, C, 3, bias=b, residual=res), conv.to(BF16).float() + res.float())
 
 
-@pytest.mark.parametrize("B,H,Tq,Tk", [(1, 2, 128, 128), (2, 5, 1024, 1024), (1, 3, 1008, 1008), (2, 10, 1024, 77),
+@pytest.mark.parametrize("xs", [1.0, 1.5])
+@pytest.mark.parametrize("B,H,Tq,Tk", [(1, 2, 128, 128), (2, 5, 1024, 1024), (2, 10, 1024, 1024), (1, 3, 1008, 1008), (2, 10, 1024, 77),
                                         (1, 5, 988, 154), (1, 2, 64, 64), (1, 1, 16, 77), (1, 10, 4096, 77), (2, 3, 200, 77),
-                                        (1, 2, 300, 128)])
-def test_attention_fwd_bwd(B, H, Tq, Tk):
+                                        (1, 2, 300, 128), (1, 2, 300, 40)])
+def test_attention_fwd_bwd(B, H, Tq, Tk, xs):
+    """Forward and backward against fp32 SDPA.  With Q and K scaled by xs = 1.5 the scores are wide enough that in a few rows of the
+    larger shapes a later key tile's P exceeds 2^8 against the running reference (never at 1.0), so the forward's exact-maximum
+    rescale of O and the row sum runs as well."""
     ops = _ops()
     g = gen(6)
-    q = torch.randn(B, Tq, H, 64, device="cuda", generator=g).to(BF16)
-    k = torch.randn(B, Tk, H, 64, device="cuda", generator=g).to(BF16)
+    q = (torch.randn(B, Tq, H, 64, device="cuda", generator=g) * xs).to(BF16)
+    k = (torch.randn(B, Tk, H, 64, device="cuda", generator=g) * xs).to(BF16)
     v = torch.randn(B, Tk, H, 64, device="cuda", generator=g).to(BF16)
     do = torch.randn(B, Tq, H, 64, device="cuda", generator=g).to(BF16)
     o, lse = ops.attn_fwd(q, k, v, 0.125)
@@ -399,79 +403,6 @@ def test_attention_fwd_bwd(B, H, Tq, Tk):
     check(dq, qr.grad.permute(0, 2, 1, 3), rel=8e-3)
     check(dk, kr.grad.permute(0, 2, 1, 3), rel=8e-3)
     check(dv, vr.grad.permute(0, 2, 1, 3), rel=8e-3)
-
-
-@pytest.mark.parametrize("B,H,Tq,Tk", [(2, 10, 1024, 1024), (1, 3, 1008, 1008), (2, 10, 1024, 77), (1, 2, 64, 64), (1, 2, 300, 40)])
-def test_attention_forward_variants_agree(B, H, Tq, Tk):
-    """The three forward kernels -- P-in-TMEM (64-key tiles, part of the exponentials on the FMA pipe; default), split-statistics
-    and shared-maximum -- compute the same softmax with different rescale points: equal within bf16 rounding; LSE equal to 2e-5."""
-    from aozora_sdxl_training_b200 import _lib
-    ops = _ops()
-    g = gen(26)
-    q = (torch.randn(B, Tq, H, 64, device="cuda", generator=g) * 1.5).to(BF16)
-    k = (torch.randn(B, Tk, H, 64, device="cuda", generator=g) * 1.5).to(BF16)
-    v = torch.randn(B, Tk, H, 64, device="cuda", generator=g).to(BF16)
-    res = {}
-    try:
-        for split in (2, 1, 0):
-            _lib.call("aoz_attn_set_fwd_split", split)
-            o, lse = ops.attn_fwd(q, k, v, 0.125)
-            res[split] = (o.clone(), lse.clone())
-    finally:
-        _lib.call("aoz_attn_set_fwd_split", 2)
-    check(res[1][0], res[0][0], rel=4e-3)
-    check(res[2][0], res[0][0], rel=4e-3)
-    assert (res[1][1] - res[0][1]).abs().max().item() < 2e-5
-    assert (res[2][1] - res[0][1]).abs().max().item() < 1e-4          # 1/4 of the exponentials by polynomial (rel. error 9e-5)
-    qr, kr, vr = [t.float().permute(0, 2, 1, 3) for t in (q, k, v)]
-    ref = torch.nn.functional.scaled_dot_product_attention(qr, kr, vr, scale=0.125).permute(0, 2, 1, 3)
-    check(res[1][0], ref, rel=6e-3)
-    check(res[2][0], ref, rel=6e-3)
-
-
-def test_attention_forward_tail_wave_key_split():
-    """Switchable path (off by default): the units of the last, partly filled wave of forward CTAs are cut along the keys and merged
-    by attn_fwd_combine_kernel -- same softmax, one more merge: equal within bf16 rounding, LSE to 2e-5."""
-    from aozora_sdxl_training_b200 import _lib
-    ops = _ops()
-    g = gen(46)
-    B, H, Tq, Tk = 4, 10, 4096, 1024                    # 1280 units on 592 slots: 96 tail units, cut six ways
-    q = torch.randn(B, Tq, H, 64, device="cuda", generator=g).to(BF16)
-    k, v = [torch.randn(B, Tk, H, 64, device="cuda", generator=g).to(BF16) for _ in range(2)]
-    o0, lse0 = ops.attn_fwd(q, k, v, 0.125)
-    try:
-        _lib.call("aoz_attn_set_fwd_tail_split", 1)
-        ops._ATTN_FWD_TAIL_SPLIT = True
-        assert _lib.query("aoz_attn_fwd_workspace_floats", B, H, Tq, Tk) > 0
-        o1, lse1 = ops.attn_fwd(q, k, v, 0.125)
-    finally:
-        _lib.call("aoz_attn_set_fwd_tail_split", 0)
-        ops._ATTN_FWD_TAIL_SPLIT = False
-    check(o1, o0, rel=4e-3)
-    assert (lse1 - lse0).abs().max().item() < 2e-5
-
-
-def test_cross_attention_backward_one_kernel_equals_two_kernels():
-    """The bit-reproducible two-kernel backward (aoz_attn_set_bwd_mode(0)): with one KV tile (77 text tokens) its dK/dV kernel can
-    also produce dQ; same dS tile, same MMA chain as the dQ kernel -> identical bits."""
-    from aozora_sdxl_training_b200 import _lib
-    ops = _ops()
-    g = gen(16)
-    B, H, Tq, Tk = 2, 20, 1024, 77
-    q, do = [torch.randn(B, Tq, H, 64, device="cuda", generator=g).to(BF16) for _ in range(2)]
-    k, v = [torch.randn(B, Tk, H, 64, device="cuda", generator=g).to(BF16) for _ in range(2)]
-    o, lse = ops.attn_fwd(q, k, v, 0.125)
-    res = {}
-    try:
-        _lib.call("aoz_attn_set_bwd_mode", 0)
-        for fused in (1, 0):
-            _lib.call("aoz_attn_set_fused_cross_bwd", fused)
-            res[fused] = [t.clone() for t in ops.attn_bwd(q, k, v, o, do, lse, 0.125)]
-    finally:
-        _lib.call("aoz_attn_set_fused_cross_bwd", 0)
-        _lib.call("aoz_attn_set_bwd_mode", 2)
-    for a, b in zip(res[1], res[0]):
-        assert torch.equal(a, b)
 
 
 @pytest.mark.parametrize("B,H,Tq,Tk", [(2, 10, 1024, 1024), (1, 3, 1008, 1008), (2, 10, 1024, 77), (1, 10, 4096, 77), (1, 2, 64, 64),

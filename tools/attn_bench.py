@@ -1,5 +1,6 @@
-"""Attention forward / backward: correctness against fp32 SDPA and CUDA-event timing of every kernel variant at the SDXL shapes.
-    python tools/attn_bench.py [--modes 2,1] [--out gpurun_out/attn_bench.json]"""
+"""Attention forward / backward: correctness against fp32 SDPA and CUDA-event timing at the SDXL shapes; --bwd-modes times the
+backward forms of aoz_attn_set_bwd_mode (2 = one kernel, 0 = dK/dV + dQ kernels).
+    python tools/attn_bench.py [--bwd-modes 2,0] [--out PATH]"""
 import argparse
 import json
 import os
@@ -31,11 +32,9 @@ def timeit(fn, n=20):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--modes", default="2,1")
     ap.add_argument("--bwd-modes", default="")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "attn_bench.json"))
     args = ap.parse_args()
-    modes = [int(m) for m in args.modes.split(",") if m != ""]
     bwd_modes = [int(m) for m in args.bwd_modes.split(",") if m != ""]
     res = {}
     g = torch.Generator(device="cuda").manual_seed(7)
@@ -47,20 +46,13 @@ def main():
         ref.backward(do.float().permute(0, 2, 1, 3))
         ref = ref.detach().permute(0, 2, 1, 3)
         f = 4.0 * B * H * T * Tk * 64
-        for m in modes:
-            _lib.call("aoz_attn_set_fwd_split", m)
-            try:
-                o, lse = ops.attn_fwd(q, k, v, 0.125)
-                torch.cuda.synchronize()
-                err = (o.float() - ref).abs().max().item() / ref.abs().max().item()
-                cos = torch.nn.functional.cosine_similarity(o.float().flatten(), ref.flatten(), dim=0).item()
-                ms = timeit(lambda: ops.attn_fwd(q, k, v, 0.125))
-                res[f"{name}_fwd_mode{m}"] = dict(us=round(ms * 1e3, 1), tflops=round(f / ms / 1e9, 1), rel_err=round(err, 5), cos=round(cos, 6))
-            except Exception as e:
-                res[f"{name}_fwd_mode{m}"] = dict(error=str(e)[:200])
-            print(name, "fwd mode", m, res[f"{name}_fwd_mode{m}"], flush=True)
-        _lib.call("aoz_attn_set_fwd_split", modes[0] if modes else 2)
         o, lse = ops.attn_fwd(q, k, v, 0.125)
+        torch.cuda.synchronize()
+        err = (o.float() - ref).abs().max().item() / ref.abs().max().item()
+        cos = torch.nn.functional.cosine_similarity(o.float().flatten(), ref.flatten(), dim=0).item()
+        ms = timeit(lambda: ops.attn_fwd(q, k, v, 0.125))
+        res[f"{name}_fwd"] = dict(us=round(ms * 1e3, 1), tflops=round(f / ms / 1e9, 1), rel_err=round(err, 5), cos=round(cos, 6))
+        print(name, "fwd", res[f"{name}_fwd"], flush=True)
         for m in (bwd_modes or [None]):
             if m is not None:
                 _lib.call("aoz_attn_set_bwd_mode", m)

@@ -1,7 +1,8 @@
 """How far do two VALID variants of the product drift apart over the 50-step loss curve of tests/test_gpu_fullsize.py?  The same
 training run (tiny config, lr 1e-4, bf16 weights, fp32 moments) is executed with the default kernels and with the round-1 attention
-kernels (two-kernel backward, split-statistics forward): the two differ only in rounding order, and both pass every parity test.
-Their mutual deviation is the noise floor of any free-running comparison at this learning rate.
+backward (two-kernel form, aoz_attn_set_bwd_mode(0)): the two differ only in rounding order, and both pass every parity test.
+Their mutual deviation is the noise floor of any free-running comparison at this learning rate.  profiles/r02_loss_curve_variants.txt
+was recorded when the round-1 variant also ran the split-statistics attention forward, since removed.
     python tools/loss_curve_variants.py [epsilon|v_prediction|rectified_flow]"""
 import os
 import sys
@@ -19,8 +20,7 @@ from oracle import host_ref  # noqa: E402
 BF16 = torch.bfloat16
 
 
-def run(mode, fwd_mode, bwd_mode, steps=50):
-    _lib.call("aoz_attn_set_fwd_split", fwd_mode)
+def run(mode, bwd_mode, steps=50):
     _lib.call("aoz_attn_set_bwd_mode", bwd_mode)
     prod = init_weights_(UNet2DConditionModel(tiny_config()), seed=42, std=0.05).to(BF16).cuda()
 
@@ -54,17 +54,16 @@ def run(mode, fwd_mode, bwd_mode, steps=50):
 
 def main():
     mode = sys.argv[1] if len(sys.argv) > 1 else "epsilon"
-    a = run(mode, 2, 2)
-    b = run(mode, 1, 0)
-    a2 = run(mode, 2, 2)
+    a = run(mode, 2)
+    b = run(mode, 0)
+    a2 = run(mode, 2)
     rel = (a - b).abs() / b
     win = (a.view(5, 10).mean(1) / b.view(5, 10).mean(1) - 1).abs()
     rel2 = (a - a2).abs() / a
-    print(f"[{mode}] default kernels vs round-1 attention kernels: step max {rel.max():.3f}, mean {rel.mean():.4f}, window max {win.max():.4f}; "
+    print(f"[{mode}] default kernels vs round-1 attention backward: step max {rel.max():.3f}, mean {rel.mean():.4f}, window max {win.max():.4f}; "
           f"default vs default again (fp32 reduce-add order only): step max {rel2.max():.3f}, mean {rel2.mean():.4f}")
     print("default :", [round(x, 3) for x in a.tolist()])
     print("round-1 :", [round(x, 3) for x in b.tolist()])
-    _lib.call("aoz_attn_set_fwd_split", 2)
     _lib.call("aoz_attn_set_bwd_mode", 2)
 
 
