@@ -63,16 +63,12 @@ def load():
         fn.restype = _CTYPES[ret]
         fn.argtypes = [_CTYPES[a] for a in args]
     _lib = lib
-    # experiment switches (tools / A-B runs): AOZ_PDL=1 enables programmatic dependent launch, AOZ_AUTOTUNE=1 times tile plans,
+    # experiment switches (tools / A-B runs): AOZ_PDL=1 enables programmatic dependent launch, AOZ_GEMM_WIDE the 320-wide plan mode,
     # AOZ_GN_SLAB=0 selects the two-kernel GroupNorm path, AOZ_ATTN_BWD_MODE=0 the bit-reproducible two-kernel attention backward
     if os.environ.get("AOZ_PDL") is not None:
         lib.aoz_set_pdl(int(os.environ["AOZ_PDL"]))
-    if os.environ.get("AOZ_AUTOTUNE") is not None:
-        lib.aoz_gemm_set_autotune(int(os.environ["AOZ_AUTOTUNE"]))
-    if os.environ.get("AOZ_TAIL_INKERNEL") is not None:
-        lib.aoz_gemm_set_tail_inkernel(int(os.environ["AOZ_TAIL_INKERNEL"]))
     if os.environ.get("AOZ_GEMM_WIDE") is not None:
-        lib.aoz_gemm_set_wide_mode(int(os.environ["AOZ_GEMM_WIDE"]), int(os.environ.get("AOZ_GEMM_WIDE_N2", "0")))
+        lib.aoz_gemm_set_wide_mode(int(os.environ["AOZ_GEMM_WIDE"]))
     if os.environ.get("AOZ_ATTN_BWD_MODE") is not None:
         call("aoz_attn_set_bwd_mode", int(os.environ["AOZ_ATTN_BWD_MODE"]))     # refuses anything but 2 and 0
     if os.environ.get("AOZ_GN_SLAB") is not None:

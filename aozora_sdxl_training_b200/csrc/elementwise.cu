@@ -284,8 +284,8 @@ __global__ void copy_channels_kernel(const __nv_bfloat16* __restrict__ src, long
 // sums the chunk partials in fixed order (deterministic) and writes the bf16 result.  No second launch.
 __device__ unsigned int g_colsum_tickets[4096];     // zero at module load; atomicInc wraps back to zero after every use
 
-// body shared by the single-tensor / per-image launch (colsum_kernel) and the batched launch (colsum_batch_kernel):
-// x, partial [gridDim.y][N] and out [N] already point at this block's problem; `ticket` = its (problem, column block) slot
+// body of colsum_kernel for one group (grid.z): x, partial [gridDim.y][N] and out [N] already point at this block's group;
+// `ticket` = its (group, column block) slot
 __device__ __forceinline__ void colsum_body(const __nv_bfloat16* __restrict__ x, long long M, int N, long long ld,
                                             float* __restrict__ partial, __nv_bfloat16* __restrict__ out, int accumulate, int ticket) {
     __shared__ float sm[8][256];
@@ -350,112 +350,12 @@ __device__ __forceinline__ void colsum_body(const __nv_bfloat16* __restrict__ x,
     }
 }
 
-// GEGLU backward WITH the bias gradient of the projection: daux = [dh | dg] is written as in geglu_bwd_kernel and its column sums
-// (db of ff.net.0.proj, 2 * half = 10240 columns at C = 1280) are formed from the rounded values on the way out -- the separate
-// column-sum launch re-read the 84 MB it had just written.  Same grid / partial / ticket scheme as colsum_body: a thread owns 8
-// columns of the value half AND the same 8 of the gate half, 8 row lanes per block, four rows in flight.
-__global__ void __launch_bounds__(256)
-geglu_bwd_colsum_kernel(const __nv_bfloat16* __restrict__ dy, const __nv_bfloat16* __restrict__ aux, long long M, int half,
-                        __nv_bfloat16* __restrict__ daux, float* __restrict__ partial, __nv_bfloat16* __restrict__ db, int accumulate) {
-    pdl_enter();
-    __shared__ float smh[8][256], smg[8][256];
-    __shared__ unsigned int s_last;
-    const int vcol = blockIdx.x * 32 + (threadIdx.x & 31);
-    const int rl = threadIdx.x >> 5;
-    const int chunks = gridDim.y;
-    const int N = 2 * half;
-    const long long rows_per_chunk = (M + chunks - 1) / chunks;
-    const long long r0 = blockIdx.y * rows_per_chunk, r1 = min(M, r0 + rows_per_chunk);
-    float acch[8] = {0, 0, 0, 0, 0, 0, 0, 0}, accg[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    if (vcol * 8 < half) {
-        auto one_row = [&](long long r, const uint4& qd, const uint4& qh, const uint4& qg) {
-            float d[8], h[8], g[8], dh[8], dg[8];
-            unpack8e(qd, d); unpack8e(qh, h); unpack8e(qg, g);
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-                float ex;
-                const float cdf = gelu_cdf(g[e], ex);
-                const float pdf = 0.39894228040143267794f * ex;
-                const float gelu = round_bf16(g[e] * cdf);
-                dh[e] = round_bf16(d[e] * gelu);
-                dg[e] = round_bf16(round_bf16(d[e] * h[e]) * (cdf + g[e] * pdf));
-                acch[e] += dh[e]; accg[e] += dg[e];
-            }
-            st_stream(daux + r * N + vcol * 8, pack8e(dh));
-            st_stream(daux + r * N + half + vcol * 8, pack8e(dg));
-        };
-        long long r = r0 + rl;
-        for (; r + 24 < r1; r += 32) {
-            uint4 qd[4], qh[4], qg[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                qd[u] = ld_stream(dy + (r + 8 * u) * half + vcol * 8);
-                qh[u] = ld_stream(aux + (r + 8 * u) * N + vcol * 8);
-                qg[u] = ld_stream(aux + (r + 8 * u) * N + half + vcol * 8);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) one_row(r + 8 * u, qd[u], qh[u], qg[u]);
-        }
-        for (; r < r1; r += 8)
-            one_row(r, ld_stream(dy + r * half + vcol * 8), ld_stream(aux + r * N + vcol * 8), ld_stream(aux + r * N + half + vcol * 8));
-    }
-#pragma unroll
-    for (int e = 0; e < 8; ++e) { smh[rl][(threadIdx.x & 31) * 8 + e] = acch[e]; smg[rl][(threadIdx.x & 31) * 8 + e] = accg[e]; }
-    __syncthreads();
-    const int c = threadIdx.x;
-    float sh = 0.f, sg = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { sh += smh[k][c]; sg += smg[k][c]; }
-    const int col = blockIdx.x * 256 + c;
-    if (col < half) {
-        partial[(long long)blockIdx.y * N + col] = sh;
-        partial[(long long)blockIdx.y * N + half + col] = sg;
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const unsigned int t = atomicInc(&g_colsum_tickets[blockIdx.x & 4095], (unsigned int)chunks - 1);
-        s_last = (t == (unsigned int)chunks - 1);
-    }
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    if (col < half) {
-#pragma unroll 1
-        for (int part = 0; part < 2; ++part) {
-            const int oc = part * half + col;
-            float v[64];
-#pragma unroll
-            for (int k = 0; k < 64; ++k) v[k] = k < chunks ? __ldcg(partial + (long long)k * N + oc) : 0.f;
-            float t = 0.f;
-#pragma unroll
-            for (int k = 0; k < 64; ++k) t += v[k];
-            if (accumulate) t = round_bf16(t) + __bfloat162float(db[oc]);
-            db[oc] = __float2bfloat16_rn(t);
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256)
 colsum_kernel(const __nv_bfloat16* __restrict__ x0, long long M, int N, long long ld, long long group_stride,
               float* __restrict__ partial0, __nv_bfloat16* __restrict__ out0, int accumulate) {
     pdl_enter();
     colsum_body(x0 + (long long)blockIdx.z * group_stride, M, N, ld, partial0 + (long long)blockIdx.z * gridDim.y * N,
                 out0 + (long long)blockIdx.z * N, accumulate, blockIdx.z * gridDim.x + blockIdx.x);
-}
-
-// Batched column sums: up to 8 independent [M_i, N_i] tensors in ONE launch (grid.z = tensor).  A transformer block's bias
-// gradients (attn1.to_out, attn2.to_out, ff.net.0.proj, ff.net.2) are four latency-bound 6..18 us launches otherwise.
-constexpr int COLSUM_BATCH = 8;
-struct ColsumProb { const __nv_bfloat16* x; long long M; long long ld; float* partial; __nv_bfloat16* out; int N; int colblocks; };
-struct ColsumBatch { ColsumProb p[COLSUM_BATCH]; int accumulate; int col_block_base[COLSUM_BATCH]; };
-
-__global__ void __launch_bounds__(256)
-colsum_batch_kernel(const __grid_constant__ ColsumBatch B) {
-    pdl_enter();
-    const ColsumProb& p = B.p[blockIdx.z];
-    if ((int)blockIdx.x >= p.colblocks) return;           // block-uniform: this tensor has fewer column blocks than the widest
-    colsum_body(p.x, p.M, p.N, p.ld, p.partial, p.out, B.accumulate, B.col_block_base[blockIdx.z] + blockIdx.x);
 }
 
 // ---- conv weight packing: OIHW -> [Cout][taps][CinPad] (forward) and [Cin][taps][CoutPad] (dgrad) -------------
@@ -605,37 +505,14 @@ int aoz_mse_loss(const void* pred, long long p_sn, long long p_sc, long long p_s
     return AOZ_OK;
 }
 
-// (a variant that also produced the projection-bias gradient in the same pass measured 73 us against 37 + 22 us for this
-// kernel followed by aoz_colsum on B200, so the two stay separate)
+// (a variant that also produced the projection-bias gradient in the same pass measured 61-66 us against 50.8 us for this
+// kernel followed by aoz_colsum at 4096 x 10240 on B200, so the two stay separate)
 int aoz_geglu_bwd(const void* dy, const void* aux, long long M, int half, void* daux, void* stream) {
     AOZ_CHECK_ARG(dy && aux && daux && half % 8 == 0, "aoz_geglu_bwd: bad arguments");
     if (M <= 0) return AOZ_OK;
     launch_k(geglu_bwd_kernel, dim3(grid_for(M * (half / 8), 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const __nv_bfloat16*)dy, (const __nv_bfloat16*)aux, M, half,
                                                                                       (__nv_bfloat16*)daux);
     AOZ_CHECK_LAUNCH("geglu_bwd_kernel");
-    return AOZ_OK;
-}
-
-static int g_geglu_chunk_mul = 4;         // row chunks ~ this many blocks per SM (experiment knob: aoz_geglu_colsum_set_blocks_per_sm)
-int aoz_geglu_colsum_set_blocks_per_sm(int n) { g_geglu_chunk_mul = n < 1 ? 1 : n; return AOZ_OK; }
-static int geglu_colsum_chunks(long long M, int half) {
-    const int colblocks = (half + 255) / 256;
-    int chunks = (sm_count() * g_geglu_chunk_mul + colblocks - 1) / colblocks;
-    if (chunks > 64) chunks = 64;
-    if ((long long)chunks * 8 > M) chunks = (int)((M + 7) / 8);
-    return chunks < 1 ? 1 : chunks;
-}
-long long aoz_geglu_bwd_colsum_workspace_floats(long long M, int half) { return (long long)geglu_colsum_chunks(M, half) * 2 * half; }
-// geglu_bwd + db = column sums of daux (the bias gradient of ff.net.0.proj) in one pass; workspace: the function above
-int aoz_geglu_bwd_colsum(const void* dy, const void* aux, long long M, int half, void* daux, void* db, int accumulate, void* workspace,
-                         void* stream) {
-    AOZ_CHECK_ARG(dy && aux && daux && db && workspace && half % 8 == 0, "aoz_geglu_bwd_colsum: bad arguments");
-    if (M <= 0) return AOZ_OK;
-    const int colblocks = (half + 255) / 256;
-    AOZ_CHECK_ARG(colblocks <= 4096, "aoz_geglu_bwd_colsum: too many columns");
-    launch_k(geglu_bwd_colsum_kernel, dim3(colblocks, geglu_colsum_chunks(M, half)), dim3(256), (size_t)(0), (cudaStream_t)stream,
-             (const __nv_bfloat16*)dy, (const __nv_bfloat16*)aux, M, half, (__nv_bfloat16*)daux, (float*)workspace, (__nv_bfloat16*)db, accumulate);
-    AOZ_CHECK_LAUNCH("geglu_bwd_colsum_kernel");
     return AOZ_OK;
 }
 
@@ -720,43 +597,6 @@ int aoz_colsum(const void* x, int groups, long long M, int N, long long ld, long
     launch_k(colsum_kernel, dim3(colblocks, chunks, groups), dim3(256), (size_t)(0), s, (const __nv_bfloat16*)x, M, N, ld, group_stride, (float*)workspace,
                                                                  (__nv_bfloat16*)out, accumulate);
     AOZ_CHECK_LAUNCH("colsum_kernel");
-    return AOZ_OK;
-}
-
-// Batched form of aoz_colsum: out_i[c] (+)= sum_r x_i[r, c] for i in [0, n), n <= 8, ONE launch.  x_ptrs / out_ptrs: HOST arrays
-// of n device pointers (uint64); Ms / lds: HOST int64[n]; Ns: HOST int32[n]; workspace >= 64 * sum(N_i) floats.
-int aoz_colsum_batch(int n, const void* x_ptrs, const void* Ms, const void* Ns, const void* lds, const void* out_ptrs, int accumulate,
-                     void* workspace, void* stream) {
-    AOZ_CHECK_ARG(n >= 1 && n <= COLSUM_BATCH, "aoz_colsum_batch: 1..%d tensors per launch (got %d)", COLSUM_BATCH, n);
-    AOZ_CHECK_ARG(x_ptrs && Ms && Ns && lds && out_ptrs && workspace, "aoz_colsum_batch: bad arguments");
-    const uint64_t* xp = (const uint64_t*)x_ptrs; const uint64_t* op = (const uint64_t*)out_ptrs;
-    const long long* M = (const long long*)Ms; const long long* ld = (const long long*)lds; const int* N = (const int*)Ns;
-    ColsumBatch B;
-    memset(&B, 0, sizeof(B));
-    B.accumulate = accumulate;
-    int max_colblocks = 0, total_colblocks = 0;
-    long long max_m = 0;
-    for (int i = 0; i < n; ++i) {
-        AOZ_CHECK_ARG(xp[i] && op[i] && M[i] > 0 && N[i] > 0, "aoz_colsum_batch: tensor %d is empty", i);
-        AOZ_CHECK_ARG(N[i] % 8 == 0 && ld[i] % 8 == 0 && (xp[i] & 15) == 0, "aoz_colsum_batch: tensor %d: N, ld multiples of 8, 16-byte aligned", i);
-        const int cb = (N[i] + 255) / 256;
-        B.col_block_base[i] = total_colblocks;
-        total_colblocks += cb;
-        if (cb > max_colblocks) max_colblocks = cb;
-        if (M[i] > max_m) max_m = M[i];
-    }
-    AOZ_CHECK_ARG(total_colblocks <= 4096, "aoz_colsum_batch: too many column blocks (%d)", total_colblocks);
-    int chunks = (sm_count() * 4 + total_colblocks - 1) / total_colblocks;
-    if (chunks > 64) chunks = 64;
-    if ((long long)chunks > (max_m + 7) / 8) chunks = (int)((max_m + 7) / 8);
-    if (chunks < 1) chunks = 1;
-    float* ws = (float*)workspace;
-    for (int i = 0; i < n; ++i) {
-        B.p[i] = ColsumProb{(const __nv_bfloat16*)xp[i], M[i], ld[i], ws, (__nv_bfloat16*)op[i], N[i], (N[i] + 255) / 256};
-        ws += (long long)64 * N[i];
-    }
-    launch_k(colsum_batch_kernel, dim3(max_colblocks, chunks, n), dim3(256), (size_t)(0), (cudaStream_t)stream, B);
-    AOZ_CHECK_LAUNCH("colsum_batch_kernel");
     return AOZ_OK;
 }
 

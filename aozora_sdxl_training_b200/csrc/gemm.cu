@@ -19,9 +19,6 @@
 // exactly the conv's zero padding.
 #include "common.cuh"
 #include <cstring>
-#include <string>
-#include <unordered_map>
-#include <vector>
 
 namespace aoz {
 
@@ -51,7 +48,6 @@ struct GemmParams {
     int mode, epi;
     int dbg;                        // experiment flags: 1 = epilogue does not load/store, 2 = MMA ignores full barriers, 4 = producer ignores empty barriers
     int bn, stages;                 // N extent of the accumulator tile (multiple of 32, <= 256; 320 = the wide one-wave plan); smem pipeline depth
-    int wide_n2;                    // bn == 320 (CTA pairs only): N of the second MMA of a K step (64; 128 = whole third B chunk, MN-major fallback)
     int a_mn, b_mn;                 // 1 = MN-major operand
     int M, N, K;                    // logical extents (CONV_FWD: M = NB*H*W output pixels, K = taps*cin_chunks*64)
     int m_tiles, n_tiles, k_iters;  // tile counts; k_iters = total K iterations (before split)
@@ -61,7 +57,6 @@ struct GemmParams {
     // `tail_ws` ([slice][128 rows][bn]) and finished (sum + fused epilogue) by tail_fixup_kernel.
     int full_work, tail_tiles, tail_splits;
     float* tail_ws;
-    int tail_inkernel;              // 1: the slices' own CTAs sum the partials and run the fused epilogue (no tail_fixup_kernel launch)
     int vec_ok;                     // EPI_STORE: every output / bias / residual row segment is 16-byte aligned
     // conv geometry (NHWC).  H, W = OUTPUT spatial size (CONV_FWD) / dy spatial size (CONV_WGRAD)
     int NB, H, W, TH, TW, tiles_h, tiles_w;
@@ -158,19 +153,6 @@ __device__ __forceinline__ void unstage8(uint32_t stg, int lane, int step, float
     ld_shared_v4f(stg + rr * 128 + ((j0 ^ (rr & 7)) << 4), f);
     ld_shared_v4f(stg + rr * 128 + (((j0 + 1) ^ (rr & 7)) << 4), f + 4);
 }
-
-// In-kernel tail fix-up: per (tail tile, CTA rank) an arrival counter and a done counter.  Every K slice of a tail tile runs on its
-// own CTA (pair) in the last round (the planner keeps tail_tiles * tail_splits <= work units), so its epilogue warps may wait for
-// the sibling slices: after writing its fp32 partial a CTA arrives, waits until all tail_splits slices have arrived, and then sums
-// and stores ITS share of the tile's 32-column chunks (chunk c belongs to slice c % tail_splits).  The last CTA to finish
-// resets both counters for the next launch (launches that use the scratch are stream-ordered).
-__device__ unsigned int g_tail_arrive[1024], g_tail_done[1024];
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-    unsigned int v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 3, 256;" ::: "memory"); }      // the 8 epilogue warps
 
 struct WorkItem { int tile, split, k_begin, k_end, tail_slot; };      // tail_slot < 0: not a tail slice
 
@@ -473,7 +455,7 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
         // Descriptors are advanced by integer adds on their low word.
         if (leader) {
             const uint32_t idesc = make_idesc_bf16(CTA2 ? 256 : BM, WIDE ? 256 : BN, P.a_mn, P.b_mn);
-            const uint32_t idesc2 = make_idesc_bf16(256, P.wide_n2, P.a_mn, P.b_mn);          // wide plan: accumulator columns [256, 256 + wide_n2)
+            const uint32_t idesc2 = make_idesc_bf16(256, 64, P.a_mn, P.b_mn);          // wide plan: accumulator columns [256, 320)
             const uint64_t hi = ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) | ((uint64_t)2 << 61);   // SBO, version, SW128
             const uint32_t smem_lo = (smem_u32(smem) & 0x3ffffu) >> 4;
             const uint32_t a_lo0 = smem_lo | ((P.a_mn ? (8192u >> 4) : 1u) << 16);
@@ -567,11 +549,10 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                 rmap[st] = map_row(P, pr.M, m_blk, q * 32 + st * 8 + (lane >> 2));
                 rnext[st] = make_uint4(0u, 0u, 0u, 0u);
             }
-            // wide plan: accumulator chunk -> (TMEM column, output column).  CTA r holds B rows [160 r, 160 r + 160) of the tile, the
-            // first MMA covers rows [0, 128) of both CTAs and the second rows [128, 160): accumulator columns [0, 128) = n [0, 128),
-            // [128, 256) = n [160, 288), [256, 288) = n [128, 160), [256 + wide_n2 / 2, +32) = n [288, 320)
+            // wide plan: accumulator column -> output column.  CTA r holds B rows [160 r, 160 r + 160) of the tile, the first MMA
+            // covers rows [0, 128) of both CTAs and the second rows [128, 160): accumulator columns [0, 128) = n [0, 128),
+            // [128, 256) = n [160, 288), [256, 288) = n [128, 160), [288, 320) = n [288, 320)
             auto out_c = [&](int c) { return !WIDE ? c : c < 128 ? c : c < 256 ? c + 32 : c == 256 ? 128 : 288; };
-            auto tmem_c = [&](int c) { return (WIDE && c == 288) ? 256 + P.wide_n2 / 2 : c; };
             auto fetch_res = [&](int c) {
                 const int col = col0 + out_c(c) + lcol;
 #pragma unroll
@@ -656,52 +637,6 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
 #pragma unroll
                     for (int j = 0; j < 32; j += 4) *reinterpret_cast<uint4*>(dstp + c + j) = make_uint4(r[j], r[j + 1], r[j + 2], r[j + 3]);
                 }
-                if (P.tail_inkernel) {
-                    const int t = wi.tail_slot / P.tail_splits;
-                    const int cidx = t * m_sub + (int)rank;
-                    __threadfence();
-                    epi_bar_sync();
-                    if (warp == 2 && lane == 0) atomicAdd(&g_tail_arrive[cidx], 1u);
-                    if (lane == 0) {
-                        unsigned int spins = 0;
-                        while (ld_acquire_u32(&g_tail_arrive[cidx]) < (unsigned int)P.tail_splits) {
-                            __nanosleep(64);
-                            if (++spins > (1u << 24)) __trap();
-                        }
-                    }
-                    __syncwarp();
-                    // this slice's share of the chunks; its two warps per lane quarter alternate over them
-                    const int n_chunks = BN / 32;
-                    const long long slice_stride = (long long)m_sub * BM * BN;
-                    const float* base = P.tail_ws + ((long long)(t * P.tail_splits * m_sub + (int)rank) * BM) * BN;
-                    int pos = 0;
-                    for (int ci = split; ci < n_chunks; ci += P.tail_splits, ++pos) {
-                        if ((pos & 1) != half) continue;
-                        const int colg = col0 + ci * 32 + lcol;
-#pragma unroll
-                        for (int st = 0; st < 4; ++st) {
-                            if (!rmap[st].ok || colg >= col_limit) continue;
-                            const int rit = q * 32 + st * 8 + (lane >> 2);
-                            const float* src = base + (long long)rit * BN + ci * 32 + lcol;
-                            float f[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-#pragma unroll 4
-                            for (int sp = 0; sp < P.tail_splits; ++sp) {
-                                const float4 v0 = __ldcg(reinterpret_cast<const float4*>(src + sp * slice_stride));
-                                const float4 v1 = __ldcg(reinterpret_cast<const float4*>(src + sp * slice_stride + 4));
-                                f[0] += v0.x; f[1] += v0.y; f[2] += v0.z; f[3] += v0.w;
-                                f[4] += v1.x; f[5] += v1.y; f[6] += v1.z; f[7] += v1.w;
-                            }
-                            epi_store8(P, pr.C, pr.ldc, rmap[st].row, rmap[st].group, colg, col_limit, f);
-                        }
-                    }
-                    epi_bar_sync();
-                    if (warp == 2 && lane == 0) {
-                        if (atomicAdd(&g_tail_done[cidx], 1u) == (unsigned int)P.tail_splits - 1u) {
-                            g_tail_arrive[cidx] = 0u; g_tail_done[cidx] = 0u;
-                            __threadfence();
-                        }
-                    }
-                }
             } else if (P.epi == EPI_PARTIAL) {
 #pragma unroll 1
                 for (int c = half * 32; c < OUT_COLS; c += 64) {
@@ -709,7 +644,7 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                     if (cbase >= col_limit) { if (WIDE) continue; break; }          // warp-uniform
                     uint32_t r[32];
                     if (!empty_split) {
-                        tmem_ld32(taddr + tmem_c(c), r);
+                        tmem_ld32(taddr + c, r);
                         tc_wait_ld();
                     } else {
 #pragma unroll
@@ -750,7 +685,7 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                 // the accumulator chunk of the NEXT iteration is requested as soon as this one's registers are staged, so the
                 // TMEM read (~300 cycles) runs under the four store steps
                 uint32_t r[32];
-                tmem_ld32(taddr + tmem_c(half * 32), r);
+                tmem_ld32(taddr + half * 32, r);
 #pragma unroll 1
                 for (int c = half * 32; c < BN; c += 64) {
                     uint4 rcur[4];
@@ -769,7 +704,7 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                     tc_wait_ld();
                     stage_chunk(stg, lane, r);
                     __syncwarp();
-                    if (c + 64 < BN) tmem_ld32(taddr + tmem_c(c + 64), r);
+                    if (c + 64 < BN) tmem_ld32(taddr + c + 64, r);
                     const int oc = out_c(c);
                     const uint32_t bw[4] = {bcur.x, bcur.y, bcur.z, bcur.w};
 #pragma unroll
@@ -811,7 +746,7 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                     if (pre_res && c + 64 < OUT_COLS && col0 + c + 64 < col_limit) fetch_res(c + 64);
                     uint32_t r[32];
                     if (!empty_split && !(P.dbg & 16)) {          // dbg 16 (experiments): epilogue without the TMEM read
-                        tmem_ld32(taddr + tmem_c(c), r);
+                        tmem_ld32(taddr + c, r);
                         tc_wait_ld();
                     } else {
 #pragma unroll
@@ -861,7 +796,8 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
 // ---- tail fix-up: sum the K slices of the tail tiles and apply the fused EPI_STORE epilogue -----------------------
 // grid = tail_tiles x m_sub x 4 row blocks x (bn / 32) column blocks; a 128-thread block owns 32 rows x 32 columns:
 // 4 lanes cover the 32 columns (128 B) of one row, so a warp reads 8 whole rows of a slice per step (coalesced) and
-// writes 8 x 64-byte output segments.
+// writes 8 x 64-byte output segments.  Summing in the slices' own CTAs instead measured ~2.5 ms per step slower (DESIGN.md 4.2):
+// the slices of a tile wait for the slowest sibling, and then few CTAs do the reduction this kernel spreads over thousands of threads.
 __global__ void __launch_bounds__(128)
 tail_fixup_kernel(const __grid_constant__ GemmParams P, int m_sub) {
     pdl_enter();
@@ -980,14 +916,9 @@ static inline int gemm_sms() {
     const int n = sm_count();
     return (g_gemm_sm_budget > 0 && g_gemm_sm_budget < n) ? g_gemm_sm_budget : n;
 }
-// Measured inside the step (B200, two runs each, same box): in-kernel 136.9 / 136.4 ms, separate launch 134.1 / 133.9 ms -- the slices
-// of a tile wait for the slowest sibling (which may still be finishing a full tile) and then few CTAs do the reduction that
-// tail_fixup_kernel spreads over thousands of threads.  Off by default.
-static int g_tail_inkernel = 0;   // 1 = tail slices are summed and stored by their own CTAs, 0 = separate tail_fixup_kernel launch (default)
 // Wide one-wave plan for outputs that are a little more than one wave of 256 x 256 pair tiles (4096 x 1280: 80 tiles on 74 pairs):
-// 0 = off, 1 = the cost model may pick it (default), 2 = whenever the shape allows it.  g_wide_mn_n2: N of the second MMA for MN-major B.
+// 0 = off, 1 = the cost model may pick it (default), 2 = whenever the shape allows it.
 static int g_wide_mode = 1;
-static int g_wide_mn_n2 = 64;
 static int g_wide_max_rounds = 2;       // rounds of 320-wide tiles the planner may consider (aoz_gemm_set_wide_max_rounds)
 static int g_tail_mode = 1;       // 0 = never cut the last wave along K, 1 = the cost model may (default), 2 = whenever possible
 static float* g_tail_ws = nullptr;        // caller-owned scratch for the tail slices (aoz_gemm_set_scratch)
@@ -1007,7 +938,6 @@ static int launch_gemm_t(GemmParams& P, cudaStream_t stream) {
     if (P.tail_tiles > 0) {
         P.full_work = tiles - P.tail_tiles;
         P.tail_ws = g_tail_ws;
-        P.tail_inkernel = (g_tail_inkernel && P.tail_tiles * (CTA2 ? 2 : 1) <= 1024) ? 1 : 0;
     } else {
         P.full_work = tiles * P.splits;
         P.tail_tiles = 0; P.tail_splits = 1;
@@ -1121,76 +1051,6 @@ static TilePlan plan_tiles(int m_tiles128, int n_extent, int k_iters_per_unit, i
     return plan_tiles_core(units_of, m_tiles128 >= 2, k_iters_per_unit, splits, b_mn, geglu, allow_tail);
 }
 
-// ---- measured plan selection ------------------------------------------------------------------------------------
-// The cycle model above is off by up to ~60 % on mid-size shapes (the L2 -> SM feed rate depends on how many SMs pull at
-// once), so the first EAGER call of every distinct problem times the candidate plans on the caller's own operands and
-// remembers the fastest (cuBLASLt-style).  Nothing is timed during CUDA-graph capture (the model decides for shapes never
-// seen eagerly), with accumulate epilogues (re-running would change the result) or while a tile / pair / tail mode is forced.
-static int g_autotune = 0;      // off by default: plans timed on L2-warm operands mis-rank the in-step (cold weight) behaviour
-static std::unordered_map<std::string, TilePlan> g_tuned;
-
-template <class UnitsFn>
-static std::vector<TilePlan> enumerate_plans(UnitsFn units_of, bool can_pair, int k_iters_per_unit, bool b_mn, bool geglu, bool allow_tail) {
-    std::vector<TilePlan> out;
-    const int sms = gemm_sms();
-    const int step = b_mn ? 64 : 32;
-    for (int pair = 0; pair <= 1; ++pair) {
-        if (pair && !can_pair) continue;
-        for (int bn = 64; bn <= 256; bn += step) {
-            if (geglu && bn != 256 && bn != 128) continue;
-            if (pair && (bn % (2 * step))) continue;
-            int n_tiles = 0;
-            const long long units = units_of(pair != 0, bn, &n_tiles);
-            const int slots = pair ? sms / 2 : sms;
-            if (units > 24LL * slots && bn < 128) continue;          // many waves of narrow tiles never win
-            out.push_back(TilePlan{bn, pair != 0, n_tiles, 0.0, 0, 1});
-            const int r = (int)(units % slots);
-            if (!allow_tail || geglu || r == 0 || !g_tail_ws) continue;
-            int ts_max = slots / r;
-            if (ts_max > k_iters_per_unit / 2) ts_max = k_iters_per_unit / 2;
-            if (ts_max > 16) ts_max = 16;
-            int last = 0;
-            const int tries[4] = {2, 4, 8, ts_max};
-            for (int t = 0; t < 4; ++t) {
-                const int ts = tries[t] < ts_max ? tries[t] : ts_max;
-                if (ts < 2 || ts == last) continue;
-                last = ts;
-                if ((long long)r * ts * (pair ? 2 : 1) * BM * bn * 4 > g_tail_bytes) continue;
-                out.push_back(TilePlan{bn, pair != 0, n_tiles, 0.0, r, ts});
-            }
-        }
-    }
-    return out;
-}
-
-static bool tuning_allowed(cudaStream_t stream) {
-    if (!g_autotune || g_force_bn > 0 || g_pair_mode != 1 || g_tail_mode != 1 || g_dbg) return false;
-    cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(stream, &st) != cudaSuccess || st != cudaStreamCaptureStatusNone) return false;
-    return true;
-}
-
-// run(plan) launches the problem with that plan; returns the fastest candidate (or `fallback` if anything fails)
-template <class RunFn>
-static TilePlan tune_plan(const std::string& key, const std::vector<TilePlan>& cands, const TilePlan& fallback, RunFn run, cudaStream_t stream) {
-    static cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (!e0) { cudaEventCreate(&e0); cudaEventCreate(&e1); }
-    TilePlan best = fallback;
-    float best_ms = 1e30f;
-    for (const TilePlan& c : cands) {
-        if (run(c) != AOZ_OK) return fallback;                       // warm (tensor maps, instruction cache)
-        cudaEventRecord(e0, stream);
-        if (run(c) != AOZ_OK || run(c) != AOZ_OK) return fallback;
-        cudaEventRecord(e1, stream);
-        if (cudaEventSynchronize(e1) != cudaSuccess) return fallback;
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, e0, e1);
-        if (ms < best_ms) { best_ms = ms; best = c; }
-    }
-    g_tuned[key] = best;
-    return best;
-}
-
 // Wide one-wave plan (see the kernel's WIDE note): cycles by the model above, or 1e300 where the shape does not allow it.  One round:
 // main loop (MMA-bound: 640 cycles per K iteration at full clock, calibrated like plan_tiles_core) + the exposed epilogue of a
 // 320-wide tile + fill / drain.
@@ -1243,17 +1103,10 @@ int aoz_gemm_set_sm_budget(int sms) { g_gemm_sm_budget = sms > 0 ? (sms & ~1) : 
 
 // 0 = never split the last wave along K, 1 = cost model decides (default), 2 = split whenever the shape allows it
 int aoz_gemm_set_tail_mode(int mode) { g_tail_mode = mode; return AOZ_OK; }
-// 0 = never use the 320-wide one-wave plan, 1 = cost model decides (default), 2 = whenever the shape allows it;
-// mn_n2 (64 | 128, <= 0 keeps the current value): N of the second MMA of a K step when B is MN-major
-int aoz_gemm_set_wide_mode(int mode, int mn_n2) {
-    g_wide_mode = mode;
-    if (mn_n2 == 64 || mn_n2 == 128) g_wide_mn_n2 = mn_n2;
-    return AOZ_OK;
-}
+// 0 = never use the 320-wide one-wave plan, 1 = cost model decides (default), 2 = whenever the shape allows it
+int aoz_gemm_set_wide_mode(int mode) { g_wide_mode = mode; return AOZ_OK; }
 // rounds of 320-wide tiles the planner may consider (default 2; 1 = only one-wave launches)
 int aoz_gemm_set_wide_max_rounds(int rounds) { g_wide_max_rounds = rounds < 1 ? 1 : rounds; return AOZ_OK; }
-// experiment switch: 1 = in-kernel tail fix-up, 0 = tail_fixup_kernel launch (default: measured 2.5 ms per step faster)
-int aoz_gemm_set_tail_inkernel(int on) { g_tail_inkernel = on ? 1 : 0; return AOZ_OK; }
 
 // Caller-owned fp32 scratch for the K slices of tail tiles (stream-ordered: every GEMM that uses it must run on the
 // same stream).  Without it the tail split is off.  20 MB covers every shape (148 slices x 128 x 256 floats).
@@ -1262,10 +1115,6 @@ int aoz_gemm_set_scratch(void* ptr, long long bytes) {
     g_tail_bytes = ptr ? bytes : 0;
     return AOZ_OK;
 }
-
-// 1: time candidate plans on the first eager call of every distinct problem; 0 (default): cost model only
-int aoz_gemm_set_autotune(int on) { g_autotune = on; return AOZ_OK; }
-int aoz_gemm_tuned_plans(void) { return (int)g_tuned.size(); }
 
 int aoz_gemm_force_bn(int bn) { g_force_bn = bn; return AOZ_OK; }
 int aoz_gemm_debug_flags(int flags) { g_dbg = flags; return AOZ_OK; }
@@ -1321,86 +1170,59 @@ int aoz_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long lo
         AOZ_CHECK_ARG((N % 2) == 0 && !b_mn && splits == 1, "aoz_gemm_bf16: GEGLU needs even N, K-major B, no split");
         P.geglu_half = N / 2;
     }
-    const int m_tiles128 = P.m_tiles;
-    const bool allow_tail = splits == 1 && !geglu;
-    const int kit = ceil_div(P.k_iters, splits);
     if (splits > 1) {
         AOZ_CHECK_ARG(workspace != nullptr, "aoz_gemm_bf16: split-K needs a workspace");
         AOZ_CHECK_ARG(!bias && !residual && !rowgroup_bias, "aoz_gemm_bf16: split-K does not fuse bias/residual");
     }
-    const GemmParams base = P;
-    auto run = [&](const TilePlan& tp) -> int {
-        GemmParams Q = base;
-        const int bn = tp.bn;
-        const bool pair = tp.pair;
-        Q.bn = bn;
-        Q.wide_n2 = (bn == 320 && b_mn) ? g_wide_mn_n2 : 64;
-        Q.n_tiles = tp.n_tiles;
-        Q.splits = splits;
-        Q.tail_tiles = tp.tail_tiles; Q.tail_splits = tp.tail_splits;
-        Q.vec_ok = ((((uintptr_t)C | (uintptr_t)bias | (uintptr_t)rowgroup_bias | (uintptr_t)residual) & 15) == 0) && (ldc % 8) == 0 &&
-                   (ld_rgb % 8) == 0 && (ldr % 8) == 0;
-        if (splits > 1) {
-            Q.epi = EPI_PARTIAL;
-            Q.partial = (float*)workspace;
-        }
-        Q.C = (__nv_bfloat16*)C; Q.ldc = ldc;
-        Q.bias = (const __nv_bfloat16*)bias;
-        Q.rowgroup_bias = (const __nv_bfloat16*)rowgroup_bias; Q.rows_per_group = rows_per_group; Q.ld_rgb = ld_rgb;
-        Q.residual = (const __nv_bfloat16*)residual; Q.ldr = ldr;
-        Q.aux = (__nv_bfloat16*)aux; Q.ld_aux = ld_aux;
-        Q.accumulate = accumulate;
-        int rc;
-        {   // A map
-            uint64_t dims[2], strides[1]; uint32_t box[2];
-            if (!a_mn) { dims[0] = K; dims[1] = M; box[0] = 64; box[1] = BM; }
-            else       { dims[0] = M; dims[1] = K; box[0] = 64; box[1] = BK; }
-            strides[0] = (uint64_t)lda * 2;
-            if ((rc = make_tmap_bf16(&Q.tmA, A, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
-        }
-        {   // B map
-            uint64_t dims[2], strides[1]; uint32_t box[2];
-            const int b_rows = pair ? bn / 2 : bn;
-            if (!b_mn) { dims[0] = K; dims[1] = N; box[0] = 64; box[1] = (uint32_t)((geglu && !pair) ? bn / 2 : b_rows); }
-            else       { dims[0] = N; dims[1] = K; box[0] = 64; box[1] = BK; }
-            strides[0] = (uint64_t)ldb * 2;
-            if ((rc = make_tmap_bf16(&Q.tmB, B, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
-        }
-        if ((rc = launch_gemm(Q, pair, (cudaStream_t)stream)) != AOZ_OK) return rc;
-        if (splits > 1) {
-            const long long total = ((long long)M * N + 3) / 4;
-            int grid = (int)((total + 255) / 256); if (grid > sm_count() * 16) grid = sm_count() * 16;
-            launch_k(splitk_reduce_kernel, dim3(grid), dim3(256), (size_t)(0), (cudaStream_t)stream, (const float*)workspace, splits, M, N, (__nv_bfloat16*)C,
-                                                                        ldc, 0, 0, 0, accumulate);
-            AOZ_CHECK_LAUNCH("splitk_reduce_kernel");
-        }
-        return AOZ_OK;
-    };
-    auto units_of = [&](bool pair, int bn, int* n_tiles) -> long long {
-        const int n_out = geglu ? bn / 2 : bn;
-        *n_tiles = ceil_div(geglu ? N / 2 : N, n_out);
-        return (long long)(pair ? ceil_div(m_tiles128, 2) : m_tiles128) * (*n_tiles) * splits;
-    };
-    TilePlan tp = plan_tiles(m_tiles128, geglu ? N / 2 : N, kit, splits, b_mn != 0, geglu, 1, allow_tail);
+    const int kit = ceil_div(P.k_iters, splits);
+    TilePlan tp = plan_tiles(P.m_tiles, geglu ? N / 2 : N, kit, splits, b_mn != 0, geglu, 1, /*allow_tail=*/splits == 1 && !geglu);
     if (!geglu && splits == 1) {
-        const double cyc = wide_plan_cycles(m_tiles128, N, kit);
+        const double cyc = wide_plan_cycles(P.m_tiles, N, kit);
         if (cyc < 1e299 && (g_wide_mode == 2 || cyc < tp.cycles)) tp = TilePlan{320, true, N / 320, cyc, 0, 1};
     }
-    if (!accumulate && tuning_allowed((cudaStream_t)stream)) {
-        char key[160];
-        snprintf(key, sizeof(key), "L %d %d %d %d %d e%d s%d f%d%d%d a%d", M, N, K, a_mn, b_mn, epi, splits, bias != nullptr, residual != nullptr,
-                 rowgroup_bias != nullptr, aux != nullptr);
-        auto it = g_tuned.find(key);
-        if (it != g_tuned.end()) tp = it->second;
-        else tp = tune_plan(key, enumerate_plans(units_of, m_tiles128 >= 2, kit, b_mn != 0, geglu, allow_tail), tp, run, (cudaStream_t)stream);
-    } else if (g_autotune && !accumulate && g_force_bn == 0 && g_pair_mode == 1 && g_tail_mode == 1) {
-        char key[160];                                              // capturing: reuse a plan measured earlier, never time
-        snprintf(key, sizeof(key), "L %d %d %d %d %d e%d s%d f%d%d%d a%d", M, N, K, a_mn, b_mn, epi, splits, bias != nullptr, residual != nullptr,
-                 rowgroup_bias != nullptr, aux != nullptr);
-        auto it = g_tuned.find(key);
-        if (it != g_tuned.end()) tp = it->second;
+    const int bn = tp.bn;
+    const bool pair = tp.pair;
+    P.bn = bn;
+    P.n_tiles = tp.n_tiles;
+    P.splits = splits;
+    P.tail_tiles = tp.tail_tiles; P.tail_splits = tp.tail_splits;
+    P.vec_ok = ((((uintptr_t)C | (uintptr_t)bias | (uintptr_t)rowgroup_bias | (uintptr_t)residual) & 15) == 0) && (ldc % 8) == 0 &&
+               (ld_rgb % 8) == 0 && (ldr % 8) == 0;
+    if (splits > 1) {
+        P.epi = EPI_PARTIAL;
+        P.partial = (float*)workspace;
     }
-    return run(tp);
+    P.C = (__nv_bfloat16*)C; P.ldc = ldc;
+    P.bias = (const __nv_bfloat16*)bias;
+    P.rowgroup_bias = (const __nv_bfloat16*)rowgroup_bias; P.rows_per_group = rows_per_group; P.ld_rgb = ld_rgb;
+    P.residual = (const __nv_bfloat16*)residual; P.ldr = ldr;
+    P.aux = (__nv_bfloat16*)aux; P.ld_aux = ld_aux;
+    P.accumulate = accumulate;
+    int rc;
+    {   // A map
+        uint64_t dims[2], strides[1]; uint32_t box[2];
+        if (!a_mn) { dims[0] = K; dims[1] = M; box[0] = 64; box[1] = BM; }
+        else       { dims[0] = M; dims[1] = K; box[0] = 64; box[1] = BK; }
+        strides[0] = (uint64_t)lda * 2;
+        if ((rc = make_tmap_bf16(&P.tmA, A, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
+    }
+    {   // B map
+        uint64_t dims[2], strides[1]; uint32_t box[2];
+        const int b_rows = pair ? bn / 2 : bn;
+        if (!b_mn) { dims[0] = K; dims[1] = N; box[0] = 64; box[1] = (uint32_t)((geglu && !pair) ? bn / 2 : b_rows); }
+        else       { dims[0] = N; dims[1] = K; box[0] = 64; box[1] = BK; }
+        strides[0] = (uint64_t)ldb * 2;
+        if ((rc = make_tmap_bf16(&P.tmB, B, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
+    }
+    if ((rc = launch_gemm(P, pair, (cudaStream_t)stream)) != AOZ_OK) return rc;
+    if (splits > 1) {
+        const long long total = ((long long)M * N + 3) / 4;
+        int grid = (int)((total + 255) / 256); if (grid > sm_count() * 16) grid = sm_count() * 16;
+        launch_k(splitk_reduce_kernel, dim3(grid), dim3(256), (size_t)(0), (cudaStream_t)stream, (const float*)workspace, splits, M, N, (__nv_bfloat16*)C,
+                                                                    ldc, 0, 0, 0, accumulate);
+        AOZ_CHECK_LAUNCH("splitk_reduce_kernel");
+    }
+    return AOZ_OK;
 }
 
 // Grouped GEMM: C_g[M_g, N_g] = op(A_g) op(B_g) for g in [0, n), n <= 10, ONE persistent launch.  All problems share K, the
@@ -1491,58 +1313,38 @@ int aoz_conv_fwd_bf16(const void* x, int NB, int Hin, int Win, int Cin, const vo
     P.k_iters = ks * ks * P.cin_chunks;
     P.M = NB * H * W; P.N = Cout; P.K = P.k_iters * 64;
     P.m_tiles = NB * P.tiles_h * P.tiles_w;
-    const int m_tiles128 = P.m_tiles;
-    const GemmParams base = P;
-    auto run = [&](const TilePlan& tp) -> int {
-        GemmParams Q = base;
-        const int bn = tp.bn;
-        const bool pair = tp.pair;
-        Q.bn = bn;
-        Q.wide_n2 = 64;
-        Q.n_tiles = tp.n_tiles;
-        Q.splits = 1;
-        Q.tail_tiles = tp.tail_tiles; Q.tail_splits = tp.tail_splits;
-        Q.vec_ok = ((((uintptr_t)y | (uintptr_t)bias | (uintptr_t)rowgroup_bias | (uintptr_t)residual) & 15) == 0) && (Cout % 8) == 0;
-        Q.C = (__nv_bfloat16*)y; Q.ldc = Cout;
-        Q.bias = (const __nv_bfloat16*)bias;
-        Q.rowgroup_bias = (const __nv_bfloat16*)rowgroup_bias; Q.ld_rgb = Cout;
-        Q.residual = (const __nv_bfloat16*)residual; Q.ldr = Cout;
-        Q.accumulate = accumulate;
-        int rc;
-        {
-            uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)Win, (uint64_t)Hin, (uint64_t)NB};
-            uint64_t strides[3] = {(uint64_t)Cin * 2, (uint64_t)Win * Cin * 2, (uint64_t)Hin * Win * Cin * 2};
-            uint32_t box[4] = {64, (uint32_t)(Q.TW * stride), (uint32_t)(Q.TH * stride), 1};
-            uint32_t es[4] = {1, (uint32_t)stride, (uint32_t)stride, 1};
-            if ((rc = make_tmap_bf16(&Q.tmA, x, 4, dims, strides, box, es)) != AOZ_OK) return rc;
-        }
-        {
-            uint64_t dims[2] = {(uint64_t)Q.K, (uint64_t)Cout};
-            uint64_t strides[1] = {(uint64_t)Q.K * 2};
-            uint32_t box[2] = {64, (uint32_t)(pair ? bn / 2 : bn)};
-            if ((rc = make_tmap_bf16(&Q.tmB, wpack, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
-        }
-        return launch_gemm(Q, pair, (cudaStream_t)stream);
-    };
-    auto units_of = [&](bool pair, int bn, int* n_tiles) -> long long {
-        *n_tiles = ceil_div(Cout, bn);
-        return (long long)(pair ? ceil_div(m_tiles128, 2) : m_tiles128) * (*n_tiles);
-    };
-    TilePlan tp = plan_tiles(m_tiles128, Cout, P.k_iters, 1, false, false, 1, /*allow_tail=*/true);
+    TilePlan tp = plan_tiles(P.m_tiles, Cout, P.k_iters, 1, false, false, 1, /*allow_tail=*/true);
     {   // the 320-wide plan (one or two rounds of 256 x 320 tiles): 1280- and 640-channel convolutions at 32 x 32 / 64 x 64
-        const double cyc = wide_plan_cycles(m_tiles128, Cout, P.k_iters);
+        const double cyc = wide_plan_cycles(P.m_tiles, Cout, P.k_iters);
         if (cyc < 1e299 && (g_wide_mode == 2 || cyc < tp.cycles)) tp = TilePlan{320, true, Cout / 320, cyc, 0, 1};
     }
-    if (!accumulate && g_autotune && g_force_bn == 0 && g_pair_mode == 1 && g_tail_mode == 1) {
-        char key[160];
-        snprintf(key, sizeof(key), "C %d %d %d %d %d k%d s%d p%d f%d%d%d%d", NB, Hin, Win, Cin, Cout, ks, stride, pad, flip, bias != nullptr,
-                 rowgroup_bias != nullptr, residual != nullptr);
-        auto it = g_tuned.find(key);
-        if (it != g_tuned.end()) tp = it->second;
-        else if (tuning_allowed((cudaStream_t)stream))
-            tp = tune_plan(key, enumerate_plans(units_of, m_tiles128 >= 2, P.k_iters, false, false, true), tp, run, (cudaStream_t)stream);
+    const int bn = tp.bn;
+    const bool pair = tp.pair;
+    P.bn = bn;
+    P.n_tiles = tp.n_tiles;
+    P.splits = 1;
+    P.tail_tiles = tp.tail_tiles; P.tail_splits = tp.tail_splits;
+    P.vec_ok = ((((uintptr_t)y | (uintptr_t)bias | (uintptr_t)rowgroup_bias | (uintptr_t)residual) & 15) == 0) && (Cout % 8) == 0;
+    P.C = (__nv_bfloat16*)y; P.ldc = Cout;
+    P.bias = (const __nv_bfloat16*)bias;
+    P.rowgroup_bias = (const __nv_bfloat16*)rowgroup_bias; P.ld_rgb = Cout;
+    P.residual = (const __nv_bfloat16*)residual; P.ldr = Cout;
+    P.accumulate = accumulate;
+    int rc;
+    {
+        uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)Win, (uint64_t)Hin, (uint64_t)NB};
+        uint64_t strides[3] = {(uint64_t)Cin * 2, (uint64_t)Win * Cin * 2, (uint64_t)Hin * Win * Cin * 2};
+        uint32_t box[4] = {64, (uint32_t)(P.TW * stride), (uint32_t)(P.TH * stride), 1};
+        uint32_t es[4] = {1, (uint32_t)stride, (uint32_t)stride, 1};
+        if ((rc = make_tmap_bf16(&P.tmA, x, 4, dims, strides, box, es)) != AOZ_OK) return rc;
     }
-    return run(tp);
+    {
+        uint64_t dims[2] = {(uint64_t)P.K, (uint64_t)Cout};
+        uint64_t strides[1] = {(uint64_t)P.K * 2};
+        uint32_t box[2] = {64, (uint32_t)(pair ? bn / 2 : bn)};
+        if ((rc = make_tmap_bf16(&P.tmB, wpack, 2, dims, strides, box, nullptr)) != AOZ_OK) return rc;
+    }
+    return launch_gemm(P, pair, (cudaStream_t)stream);
 }
 
 // Convolution weight gradient: dW[cout][tap][cin] = sum_pixels dy[pix][cout] * x[pix*stride + tap - pad][cin].
@@ -1577,7 +1379,6 @@ int aoz_conv_wgrad_bf16(const void* dy, const void* x, int NB, int H, int W, int
     }
     const int bn = tp.bn;
     P.bn = bn;
-    P.wide_n2 = g_wide_mn_n2;
     P.n_tiles_per_tap = ceil_div(Cin, bn);
     P.n_tiles = taps * P.n_tiles_per_tap;
     P.splits = splits;

@@ -7,8 +7,8 @@
 // read p, g, m, v once, write p, m, v once (14 B/param with bf16 state, 28 B/param all-fp32).
 //
 // Work is cut into fixed chunks of CHUNK elements; chunk c belongs to tensor chunk_tensor[c] and the chunks
-// of one tensor are consecutive (chunk_start[t] .. chunk_start[t+1]).  Pure HBM streaming: 128-bit
-// L1-bypassing loads/stores, 4 independent 16-byte requests per stream in flight per thread.
+// of one tensor are consecutive (chunk_start[t] .. chunk_start[t+1]).  Pure HBM streaming: the update moves its
+// operands by bulk copies through shared memory, the gradient norm by 128-bit L1-bypassing loads.
 #include "common.cuh"
 #include <cuda_fp16.h>
 
@@ -41,9 +41,8 @@ template <> struct Elem<DT_F16> {
     static __device__ __forceinline__ void st(T* p, float v) { *p = __float2half_rn(v); }
 };
 
-// load / store 8 consecutive elements as fp32
+// load 8 consecutive elements as fp32
 template <int DT> __device__ __forceinline__ void ld8(const void* base, size_t i, float* f);
-template <int DT> __device__ __forceinline__ void st8(void* base, size_t i, const float* f);
 
 template <> __device__ __forceinline__ void ld8<DT_F32>(const void* base, size_t i, float* f) {
     const float* p = (const float*)base + i;
@@ -51,19 +50,10 @@ template <> __device__ __forceinline__ void ld8<DT_F32>(const void* base, size_t
     f[0] = __uint_as_float(a.x); f[1] = __uint_as_float(a.y); f[2] = __uint_as_float(a.z); f[3] = __uint_as_float(a.w);
     f[4] = __uint_as_float(b.x); f[5] = __uint_as_float(b.y); f[6] = __uint_as_float(b.z); f[7] = __uint_as_float(b.w);
 }
-template <> __device__ __forceinline__ void st8<DT_F32>(void* base, size_t i, const float* f) {
-    float* p = (float*)base + i;
-    st_stream(p, make_uint4(__float_as_uint(f[0]), __float_as_uint(f[1]), __float_as_uint(f[2]), __float_as_uint(f[3])));
-    st_stream(p + 4, make_uint4(__float_as_uint(f[4]), __float_as_uint(f[5]), __float_as_uint(f[6]), __float_as_uint(f[7])));
-}
 template <> __device__ __forceinline__ void ld8<DT_BF16>(const void* base, size_t i, float* f) {
     uint4 a = ld_stream((const __nv_bfloat16*)base + i);
     f[0] = bf16lo(a.x); f[1] = bf16hi(a.x); f[2] = bf16lo(a.y); f[3] = bf16hi(a.y);
     f[4] = bf16lo(a.z); f[5] = bf16hi(a.z); f[6] = bf16lo(a.w); f[7] = bf16hi(a.w);
-}
-template <> __device__ __forceinline__ void st8<DT_BF16>(void* base, size_t i, const float* f) {
-    st_stream((__nv_bfloat16*)base + i,
-              make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7])));
 }
 __device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
     __half2 v = __floats2half2_rn(lo, hi);
@@ -74,10 +64,6 @@ template <> __device__ __forceinline__ void ld8<DT_F16>(const void* base, size_t
     const __half2* h = reinterpret_cast<const __half2*>(&a);
 #pragma unroll
     for (int k = 0; k < 4; ++k) { float2 t = __half22float2(h[k]); f[2 * k] = t.x; f[2 * k + 1] = t.y; }
-}
-template <> __device__ __forceinline__ void st8<DT_F16>(void* base, size_t i, const float* f) {
-    st_stream((__half*)base + i,
-              make_uint4(pack_f16(f[0], f[1]), pack_f16(f[2], f[3]), pack_f16(f[4], f[5]), pack_f16(f[6], f[7])));
 }
 
 // 8 consecutive elements <-> fp32 in SHARED memory (the bulk-copy ring of raven_step_bulk_kernel)
@@ -127,62 +113,13 @@ __device__ __forceinline__ void raven_elem(float& p, float g, float& m, float& v
     p = __fmaf_rn(-h.step_size, __fdiv_rn(m, denom), p);                            // addcdiv_(m, denom, -step_size)
 }
 
-template <int PDT, int GDT, int MDT>
-__global__ void __launch_bounds__(MT_THREADS)
-raven_step_mt_kernel(int n_chunks, const uint64_t* __restrict__ p_ptrs, const uint64_t* __restrict__ g_ptrs,
-                     const uint64_t* __restrict__ m_ptrs, const uint64_t* __restrict__ v_ptrs,
-                     const int64_t* __restrict__ numel, const int32_t* __restrict__ chunk_start,
-                     const int32_t* __restrict__ chunk_tensor, const RavenHyper* __restrict__ hyper,
-                     const float* __restrict__ clip_coef) {
-    using PE = Elem<PDT>;
-    using GE = Elem<GDT>;
-    using ME = Elem<MDT>;
-    const bool use_clip = clip_coef != nullptr;
-    const float clip = use_clip ? __ldg(clip_coef) : 1.0f;
-    for (int c = blockIdx.x; c < n_chunks; c += gridDim.x) {
-        const int t = chunk_tensor[c];
-        const RavenHyper h = hyper[t];
-        typename PE::T* p = (typename PE::T*)p_ptrs[t];
-        const typename GE::T* g = (const typename GE::T*)g_ptrs[t];
-        typename ME::T* m = (typename ME::T*)m_ptrs[t];
-        typename ME::T* v = (typename ME::T*)v_ptrs[t];
-        const int64_t n = numel[t];
-        const int64_t begin = (int64_t)(c - chunk_start[t]) * MT_CHUNK;
-        const int64_t end = min(begin + (int64_t)MT_CHUNK, n);
-        const bool aligned = ((((uintptr_t)p) & (PDT == DT_F32 ? 31 : 15)) == 0) && ((((uintptr_t)g) & (GDT == DT_F32 ? 31 : 15)) == 0) &&
-                             ((((uintptr_t)m | (uintptr_t)v) & (MDT == DT_F32 ? 31 : 15)) == 0);
-        int64_t vec_end = aligned ? begin + ((end - begin) & ~(int64_t)7) : begin;
-        // vector body: 2 independent groups of 8 elements per thread per iteration
-        for (int64_t i = begin + (int64_t)threadIdx.x * 8; i < vec_end; i += (int64_t)MT_THREADS * 16) {
-            const int64_t i2 = i + (int64_t)MT_THREADS * 8;
-            const bool two = i2 < vec_end;
-            float pf[2][8], gf[2][8], mf[2][8], vf[2][8];
-            ld8<PDT>(p, i, pf[0]); ld8<GDT>(g, i, gf[0]); ld8<MDT>(m, i, mf[0]); ld8<MDT>(v, i, vf[0]);
-            if (two) { ld8<PDT>(p, i2, pf[1]); ld8<GDT>(g, i2, gf[1]); ld8<MDT>(m, i2, mf[1]); ld8<MDT>(v, i2, vf[1]); }
-#pragma unroll
-            for (int k = 0; k < 8; ++k) raven_elem<GDT>(pf[0][k], gf[0][k], mf[0][k], vf[0][k], h, clip, use_clip);
-            st8<PDT>(p, i, pf[0]); st8<MDT>(m, i, mf[0]); st8<MDT>(v, i, vf[0]);
-            if (two) {
-#pragma unroll
-                for (int k = 0; k < 8; ++k) raven_elem<GDT>(pf[1][k], gf[1][k], mf[1][k], vf[1][k], h, clip, use_clip);
-                st8<PDT>(p, i2, pf[1]); st8<MDT>(m, i2, mf[1]); st8<MDT>(v, i2, vf[1]);
-            }
-        }
-        // scalar tail (or whole chunk when a pointer is not 16/32-byte aligned)
-        for (int64_t i = vec_end + threadIdx.x; i < end; i += MT_THREADS) {
-            float pf = PE::ld(p + i), gf = GE::ld(g + i), mf = ME::ld(m + i), vf = ME::ld(v + i);
-            raven_elem<GDT>(pf, gf, mf, vf, h, clip, use_clip);
-            PE::st(p + i, pf); ME::st(m + i, mf); ME::st(v + i, vf);
-        }
-    }
-}
-
-// ---- the same update, streamed through shared memory by the TMA engine --------------------------------------
-// The register-streaming kernel above keeps 2 x 4 16-byte requests per thread in flight, alternates load and compute / store phases
-// and stalls ~1 us at every chunk start on the dependent metadata loads: 0.73-0.79 of the measured HBM bandwidth over the real
-// 1680-tensor table.  Here one thread per CTA runs BULK_STAGES - 1 items ahead of the math: an item is BULK_SUB elements of one
-// chunk, fetched as four cp.async.bulk copies (p, g, m, v) into a ring in shared memory; 256 threads update 8 elements each in
-// place (one 16-byte shared-memory access per stream); three bulk copies write p, m, v back.  No register ever waits on HBM.
+// ---- the update, streamed through shared memory by the TMA engine ---------------------------------------------
+// One thread per CTA runs BULK_STAGES - 1 items ahead of the math: an item is BULK_SUB elements of one chunk, fetched as four
+// cp.async.bulk copies (p, g, m, v) into a ring in shared memory; 256 threads update 8 elements each in place (one 16-byte
+// shared-memory access per stream); three bulk copies write p, m, v back.  No register ever waits on HBM, and the dependent loads
+// of a chunk's metadata are hidden behind the items in flight.  (Streaming through registers -- 2 x 4 16-byte requests per thread,
+// load and compute / store phases alternating, ~1 us stalls at every chunk start -- reached 0.73-0.79 of the measured HBM
+// bandwidth over the real 1680-tensor table; this kernel took the step's update from 7.4 to 6.9 ms.)
 // Pieces that cannot be moved in 16-byte granules (pointers off alignment, the last < 8 elements of a tensor) take the direct path.
 constexpr int BULK_SUB = 2048;                  // elements per item = 8 per thread
 constexpr int BULK_STAGES = 4;
@@ -424,10 +361,6 @@ extern "C" {
 
 int aoz_mt_chunk_elems(void) { return MT_CHUNK; }
 
-// experiment switch: 1 = the update streams through shared memory with bulk copies (default), 0 = register-streaming kernel
-static int g_raven_bulk = 1;
-int aoz_raven_set_bulk(int on) { g_raven_bulk = on ? 1 : 0; return AOZ_OK; }
-
 int aoz_raven_step_mt(int n_tensors, int n_chunks, const void* p_ptrs, const void* g_ptrs, const void* m_ptrs,
                       const void* v_ptrs, const void* numel, const void* chunk_start, const void* chunk_tensor,
                       const void* hyper, const void* clip_coef, int p_dtype, int g_dtype, int m_dtype, void* stream) {
@@ -435,25 +368,20 @@ int aoz_raven_step_mt(int n_tensors, int n_chunks, const void* p_ptrs, const voi
     if (n_tensors == 0 || n_chunks == 0) return AOZ_OK;
     AOZ_CHECK_ARG(p_ptrs && g_ptrs && m_ptrs && v_ptrs && numel && chunk_start && chunk_tensor && hyper,
                   "aoz_raven_step_mt: null table pointer");
-    int grid = n_chunks < sm_count() * 8 ? n_chunks : sm_count() * 8;
     cudaStream_t s = (cudaStream_t)stream;
 #define AOZ_RAVEN_LAUNCH(P, G, M)                                                                                  \
-    if (g_raven_bulk) {                                                                                            \
+    do {                                                                                                           \
         constexpr int esz = (P == DT_F32 ? 4 : 2) + (G == DT_F32 ? 4 : 2) + 2 * (M == DT_F32 ? 4 : 2);             \
         constexpr int smem = BULK_STAGES * BULK_SUB * esz;                                                         \
         static bool attr = false;                                                                                  \
         if (!attr) { cudaFuncSetAttribute(raven_step_bulk_kernel<P, G, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); attr = true; } \
         const int per_sm = (200 * 1024) / (smem + 1024) > 0 ? (200 * 1024) / (smem + 1024) : 1;                    \
-        const int bgrid = n_chunks < sm_count() * per_sm ? n_chunks : sm_count() * per_sm;                         \
-        raven_step_bulk_kernel<P, G, M><<<bgrid, MT_THREADS, smem, s>>>(                                           \
+        const int grid = n_chunks < sm_count() * per_sm ? n_chunks : sm_count() * per_sm;                          \
+        raven_step_bulk_kernel<P, G, M><<<grid, MT_THREADS, smem, s>>>(                                            \
             n_chunks, (const uint64_t*)p_ptrs, (const uint64_t*)g_ptrs, (const uint64_t*)m_ptrs, (const uint64_t*)v_ptrs, \
             (const int64_t*)numel, (const int32_t*)chunk_start, (const int32_t*)chunk_tensor, (const RavenHyper*)hyper,  \
             (const float*)clip_coef);                                                                              \
-    } else                                                                                                         \
-    raven_step_mt_kernel<P, G, M><<<grid, MT_THREADS, 0, s>>>(                                                     \
-        n_chunks, (const uint64_t*)p_ptrs, (const uint64_t*)g_ptrs, (const uint64_t*)m_ptrs, (const uint64_t*)v_ptrs, \
-        (const int64_t*)numel, (const int32_t*)chunk_start, (const int32_t*)chunk_tensor, (const RavenHyper*)hyper,  \
-        (const float*)clip_coef)
+    } while (0)
 #define AOZ_RAVEN_M(P, G)                                                          \
     if (m_dtype == DT_BF16) AOZ_RAVEN_LAUNCH(P, G, DT_BF16);                        \
     else if (m_dtype == DT_F32) AOZ_RAVEN_LAUNCH(P, G, DT_F32);                     \
@@ -465,7 +393,7 @@ int aoz_raven_step_mt(int n_tensors, int n_chunks, const void* p_ptrs, const voi
     else { set_error("aoz_raven_step_mt: unsupported dtypes p=%d g=%d m=%d", p_dtype, g_dtype, m_dtype); return AOZ_ERR_UNSUPPORTED; }
 #undef AOZ_RAVEN_M
 #undef AOZ_RAVEN_LAUNCH
-    AOZ_CHECK_LAUNCH("raven_step_mt_kernel");
+    AOZ_CHECK_LAUNCH("raven_step_bulk_kernel");
     return AOZ_OK;
 }
 

@@ -390,21 +390,14 @@ def mse_loss(pred, target_nchw, tickets, table, denom, grad_scale=1.0, *, pred_n
     return loss, per, dpred
 
 
-def geglu_bwd(dy, aux, bias_grad=None):
-    """-> daux.  ``bias_grad``: a bf16 [2 * half] destination: the column sums of daux (the projection's bias gradient) are formed
-    in the same pass (saves the column-sum launch's re-read of daux)."""
+def geglu_bwd(dy, aux):
+    """GEGLU backward: dy [.., half] and the saved pre-activation aux [.., 2 * half] -> daux [.., 2 * half]."""
     _chk(dy, "geglu_bwd dy")
     _chk(aux, "geglu_bwd aux")
     half = dy.shape[-1]
     M = dy.numel() // half
     daux = torch.empty_like(aux)
-    if bias_grad is not None:
-        _chk(bias_grad, "geglu_bwd bias_grad")
-        ws = workspace(_lib.query("aoz_geglu_bwd_colsum_workspace_floats", M, half), dy.device)
-        _lib.call("aoz_geglu_bwd_colsum", dy.data_ptr(), aux.data_ptr(), M, half, daux.data_ptr(), bias_grad.data_ptr(), 0,
-                  ws.data_ptr(), _stream())
-    else:
-        _lib.call("aoz_geglu_bwd", dy.data_ptr(), aux.data_ptr(), M, half, daux.data_ptr(), _stream())
+    _lib.call("aoz_geglu_bwd", dy.data_ptr(), aux.data_ptr(), M, half, daux.data_ptr(), _stream())
     _count()
     return daux
 
@@ -491,39 +484,6 @@ def colsum(x2d, out=None, accumulate=False):
     _lib.call("aoz_colsum", x2d.data_ptr(), 1, M, N, x2d.stride(0), 0, out.data_ptr(), int(accumulate), ws.data_ptr(), _stream())
     _count(2)
     return out
-
-
-COLSUM_BATCH = 8
-
-
-def colsum_batch(items):
-    """Column sums of several independent 2-D tensors in ONE launch: ``items`` = [(x2d, out_or_None), ...] -> [out, ...]
-    (a transformer block's Linear bias gradients)."""
-    import ctypes
-    items = list(items)
-    if not items:
-        return []
-    if len(items) == 1:
-        return [colsum(items[0][0], out=items[0][1])]
-    if len(items) > COLSUM_BATCH:
-        return colsum_batch(items[:COLSUM_BATCH]) + colsum_batch(items[COLSUM_BATCH:])
-    n = len(items)
-    outs = []
-    for x, out in items:
-        _chk(x, "colsum_batch x", contiguous=False)
-        if x.dim() != 2 or x.stride(1) != 1:
-            raise _lib.AozoraError("colsum_batch: tensors must be 2-D with unit inner stride")
-        if out is None:
-            out = torch.empty((x.shape[1],), dtype=BF16, device=x.device)
-        outs.append(_chk(out, "colsum_batch out"))
-    u64, i64, i32 = ctypes.c_uint64 * n, ctypes.c_longlong * n, ctypes.c_int * n
-    xp, op = u64(*[x.data_ptr() for x, _ in items]), u64(*[o.data_ptr() for o in outs])
-    ms, lds, ns = i64(*[x.shape[0] for x, _ in items]), i64(*[x.stride(0) for x, _ in items]), i32(*[x.shape[1] for x, _ in items])
-    ws = workspace(64 * sum(x.shape[1] for x, _ in items), items[0][0].device)
-    _lib.call("aoz_colsum_batch", n, ctypes.addressof(xp), ctypes.addressof(ms), ctypes.addressof(ns), ctypes.addressof(lds),
-              ctypes.addressof(op), 0, ws.data_ptr(), _stream())
-    _count()
-    return outs
 
 
 def colsum_grouped(x3d):

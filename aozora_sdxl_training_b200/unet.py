@@ -16,8 +16,6 @@ always-on gradient checkpointing, train.py:2660, is unnecessary).  The ``nn.Conv
 """
 from __future__ import annotations
 
-import os
-
 from types import SimpleNamespace
 
 import torch
@@ -31,13 +29,6 @@ BF16 = torch.bfloat16
 # ------------------------------------------------------------------------------------------------------------
 # parameter containers (names and registration order follow diffusers; see SURVEY.md 8a appendix / 8b)
 # ------------------------------------------------------------------------------------------------------------
-# A/B switch (AOZ_LN_COLSUM=0): bias gradients of to_out / ff.net.2 / proj_in as separate column-sum launches instead of riding the
-# LayerNorm backward that produces their dy
-LN_COLSUM = os.environ.get("AOZ_LN_COLSUM", "1") != "0"
-# A/B switch (AOZ_GEGLU_COLSUM=1): ff.net.0.proj's bias gradient formed inside the GEGLU backward kernel.  Off: the column-owner
-# thread mapping that the fused sums need streams worse than the elementwise kernel (tools/geglu_bwd_bench.py, 4096 x 10240:
-# 61-66 us fused against 50.8 us for geglu_bwd + colsum)
-GEGLU_COLSUM = os.environ.get("AOZ_GEGLU_COLSUM", "0") == "1"
 
 
 class TimestepEmbedding(nn.Module):
@@ -178,7 +169,6 @@ class GradSink:
         self.on_grad = None        # optional callback(param, grad): data-parallel bucket scheduling during the sweep
         self.pending = []          # deferred Linear weight gradients: (params stacked by rows, dy, x)
         self.pending_late = []     # the same, flushed once per Transformer2DModel (cross-attention k/v: K = text tokens)
-        self.pending_bias = []     # deferred Linear bias gradients: (bias, dy) -> one batched column-sum launch per flush
         self.dest = None           # optional callback(param) -> tensor the gradient must be written to (data-parallel flat buffer)
 
     def out_for(self, params):
@@ -215,12 +205,9 @@ class GradSink:
         else:
             self._hand_out(params, ops.gemm(dy, x, a_mn=True, b_mn=True, out=self.out_for(params)))
 
-    def bias_grad(self, b, dy, defer=False):
-        """db = column sums of dy.  ``defer``: queue it; ``flush`` sums every queued tensor in ONE launch."""
-        if defer:
-            self.pending_bias.append((b, dy))
-        else:
-            self.add(b, ops.colsum(dy, out=self.out_for(b)))
+    def bias_grad(self, b, dy):
+        """db = column sums of dy."""
+        self.add(b, ops.colsum(dy, out=self.out_for(b)))
 
     def _hand_out(self, params, dw):
         r = 0
@@ -233,11 +220,6 @@ class GradSink:
             jobs, self.pending_late = self.pending_late, []
         else:
             jobs, self.pending = self.pending, []
-            if self.pending_bias:
-                bjobs, self.pending_bias = self.pending_bias, []
-                outs = ops.colsum_batch([(dy, self.out_for(b)) for b, dy in bjobs])
-                for (b, _), db in zip(bjobs, outs):
-                    self.add(b, db)
         by_k = {}
         for job in jobs:
             by_k.setdefault(job[2].shape[0], []).append(job)
@@ -295,7 +277,7 @@ def _linear(x, w, b, G, *, residual=None, need_dx=True, w_param=None, defer=Fals
                 G.wgrad((wp,), dy, x, defer=defer)
             else:
                 G.add(wp, ops.gemm(dy, x, a_mn=True, b_mn=True))
-        if b is not None and b.requires_grad and not (bias_done and LN_COLSUM):
+        if b is not None and b.requires_grad and not bias_done:
             G.bias_grad(b, dy)          # right away: dy is still L2-resident (deferring it to the block's flush measured slower)
         if not need_dx:
             return None
@@ -309,16 +291,9 @@ def _geglu(x, w, b, G, defer=False):
     y = ops.gemm(x, w, bias=b, epi=ops.EPI_GEGLU, aux=aux)
 
     def bwd(dy):
-        if b.requires_grad and GEGLU_COLSUM:        # the bias gradient (column sums of daux) in the same pass -- measured slower
-            db = G.out_for(b)
-            if db is None:
-                db = torch.empty_like(b)
-            daux = ops.geglu_bwd(dy, aux, bias_grad=db)
-            G.add(b, db)
-        else:
-            daux = ops.geglu_bwd(dy, aux)
-            if b.requires_grad:
-                G.bias_grad(b, daux)
+        daux = ops.geglu_bwd(dy, aux)
+        if b.requires_grad:
+            G.bias_grad(b, daux)
         if w.requires_grad:
             G.wgrad((w,), daux, x, defer=defer)
         return ops.gemm(daux, w, b_mn=True)
@@ -379,7 +354,7 @@ def _layernorm(x, mod, G):
         called with ``bias_done=True``)."""
         both = mod.weight.requires_grad and mod.bias.requires_grad
         dcol = None
-        if LN_COLSUM and bias_of_dx is not None and bias_of_dx.requires_grad:
+        if bias_of_dx is not None and bias_of_dx.requires_grad:
             dcol = G.out_for(bias_of_dx)
             if dcol is None:
                 dcol = torch.empty_like(bias_of_dx)

@@ -39,8 +39,6 @@ int aoz_mt_chunk_elems(void);
 int aoz_raven_step_mt(int n_tensors, int n_chunks, const void* p_ptrs, const void* g_ptrs, const void* m_ptrs,
                       const void* v_ptrs, const void* numel, const void* chunk_start, const void* chunk_tensor,
                       const void* hyper, const void* clip_coef, int p_dtype, int g_dtype, int m_dtype, void* stream);
-/* experiment switch: 1 = the update streams through shared memory with cp.async.bulk copies (default), 0 = register-streaming kernel */
-int aoz_raven_set_bulk(int on);
 /* out3 = {total_norm, clip_coef = min(1, max_norm/(norm+1e-6)), sum_of_squares}; partial: n_chunks floats */
 int aoz_gradnorm_mt(int n_tensors, int n_chunks, const void* g_ptrs, const void* numel, const void* chunk_start,
                     const void* chunk_tensor, void* partial, float max_norm, int emulate_bf16, void* out3,
@@ -59,22 +57,13 @@ int aoz_gemm_force_bn(int bn);
  * scratch, finished by a fix-up kernel).  mode 0 = off, 1 = cost model decides (default), 2 = whenever possible.
  * The scratch (>= 20 MB covers every shape) is used stream-ordered: all GEMM / conv calls must share one stream. */
 int aoz_gemm_set_tail_mode(int mode);
-/* experiment switch: 1 = the K slices of tail tiles are summed and stored by their own CTAs, 0 = tail_fixup_kernel launch (default:
- * the in-kernel form measured 2.5 ms per step slower) */
-int aoz_gemm_set_tail_inkernel(int on);
 /* wide one-wave plan: outputs that are slightly more than one wave of 256 x 256 pair tiles (4096 x 1280 = 80 tiles on 74 SM pairs)
  * run as ONE round of 256 x 320 tiles (a single 320-column accumulator, two MMAs per K step).  mode 0 = off, 1 = cost model
- * decides (default), 2 = whenever the shape allows it (N % 320 == 0, tiles <= SM pairs, store epilogue, no split-K);
- * mn_n2 = 64 | 128 selects the second MMA's N for MN-major B (<= 0: keep): 64 (default, the tested path) reads half a 64-wide
- * swizzle atom per CTA, 128 reads the whole third chunk into 64 spare accumulator columns (fallback, not exercised by the tests). */
-int aoz_gemm_set_wide_mode(int mode, int mn_n2);
+ * decides (default), 2 = whenever the shape allows it (N % 320 == 0, tiles <= SM pairs, store epilogue, no split-K).
+ * The second MMA has N = 64: for MN-major B it reads half a 64-wide swizzle atom per CTA. */
+int aoz_gemm_set_wide_mode(int mode);
 /* rounds of 320-wide tiles per SM pair the planner may consider (default 2; the single accumulator serialises a pair's tiles) */
 int aoz_gemm_set_wide_max_rounds(int rounds);
-/* measured plan selection: the first EAGER call of every distinct GEMM / conv problem times the candidate tile plans on the
- * caller's operands and caches the fastest (never during CUDA-graph capture, never for accumulate epilogues).  Off by
- * default: on B200 the L2-warm timings mis-ranked the plans for the in-step (cold-weight) launches (profiles/r01 notes). */
-int aoz_gemm_set_autotune(int on);
-int aoz_gemm_tuned_plans(void);
 int aoz_gemm_set_scratch(void* ptr, long long bytes);
 int aoz_gemm_debug_flags(int flags);
 int aoz_gemm_auto_splits(int M, int N, int K, int b_mn);
@@ -145,13 +134,6 @@ int aoz_mse_loss(const void* pred, long long p_sn, long long p_sc, long long p_s
                  void* per_sample, void* weights, void* loss_out, void* dpred, long long d_sn, long long d_sc, long long d_shw,
                  void* stream);
 int aoz_geglu_bwd(const void* dy, const void* aux, long long M, int half, void* daux, void* stream);
-/* The same pass also forming db = column sums of daux (the bias gradient of ff.net.0.proj, from the rounded values: equal to
- * aoz_colsum over daux); workspace: aoz_geglu_bwd_colsum_workspace_floats(M, half) floats */
-int aoz_geglu_bwd_colsum(const void* dy, const void* aux, long long M, int half, void* daux, void* db, int accumulate, void* workspace,
-                         void* stream);
-long long aoz_geglu_bwd_colsum_workspace_floats(long long M, int half);
-/* experiment knob: row chunks of the fused kernel ~ this many blocks per SM (capped at 64 chunks) */
-int aoz_geglu_colsum_set_blocks_per_sm(int n);
 int aoz_silu_fwd(const void* x, long long n, void* y, void* stream);
 int aoz_silu_bwd(const void* dy, const void* x, long long n, void* dx, void* stream);
 int aoz_add(const void* a, const void* b, long long n, void* y, void* stream);
@@ -163,11 +145,6 @@ int aoz_copy_channels(const void* src, long long src_ld, int src_off, void* dst,
 long long aoz_colsum_workspace_floats(int groups, int N);
 int aoz_colsum(const void* x, int groups, long long M, int N, long long ld, long long group_stride, void* out, int accumulate,
                void* workspace, void* stream);
-/* Batched column sums (train.py:2765 autograd: the bias gradients of one BasicTransformerBlock's Linear layers): n <= 8
- * tensors x_i [M_i, N_i] bf16 (row stride ld_i) -> out_i [N_i] bf16 in ONE launch.  x_ptrs / out_ptrs: HOST uint64[n] device
- * pointers; Ms / lds: HOST int64[n]; Ns: HOST int32[n]; workspace >= 64 * sum(N_i) floats. */
-int aoz_colsum_batch(int n, const void* x_ptrs, const void* Ms, const void* Ns, const void* lds, const void* out_ptrs, int accumulate,
-                     void* workspace, void* stream);
 int aoz_timestep_embedding(const void* t, int n, int dim, void* out, void* stream);
 
 #ifdef __cplusplus

@@ -27,7 +27,7 @@ def _defaults():
         _lib.call("aoz_gemm_set_scratch", buf.data_ptr(), buf.numel())
     else:
         _lib.call("aoz_gemm_set_scratch", 0, 0)
-    _lib.call("aoz_gemm_set_wide_mode", 1, 64)
+    _lib.call("aoz_gemm_set_wide_mode", 1)
     _lib.call("aoz_gemm_set_wide_max_rounds", 2)
     _lib.call("aoz_gemm_set_tail_mode", 1)
     _lib.call("aoz_gemm_set_pair_mode", 1)
@@ -51,10 +51,10 @@ def test_wide_plan_needs_whole_320_column_tiles_and_few_rounds():
 
 
 def test_wide_plan_switches():
-    _lib.call("aoz_gemm_set_wide_mode", 0, 0)
+    _lib.call("aoz_gemm_set_wide_mode", 0)
     p = plan(4096, 1280, 1280)
     assert p["bn"] != 320 and p["bn"] <= 256
-    _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+    _lib.call("aoz_gemm_set_wide_mode", 1)
     _lib.call("aoz_gemm_set_pair_mode", 0)                      # single-CTA tiles only: no pairs, no wide plan
     assert plan(4096, 1280, 1280)["pair"] == 0
     _lib.call("aoz_gemm_set_pair_mode", 1)
@@ -65,7 +65,7 @@ def test_wide_plan_switches():
 
 def test_tail_split_covers_the_ragged_last_wave():
     """80 pair tiles on 74 SM pairs: the 6 tiles of the last wave are cut along K over the idle pairs (wide plan off)."""
-    _lib.call("aoz_gemm_set_wide_mode", 0, 0)
+    _lib.call("aoz_gemm_set_wide_mode", 0)
     p = plan(4096, 1280, 10240, 1)
     assert p["pair"] == 1 and p["bn"] == 256 and p["tail_tiles"] == 6 and 2 <= p["tail_splits"] <= 12
     assert p["tail_tiles"] * p["tail_splits"] <= 74

@@ -176,13 +176,13 @@ def test_conv_wide_plan_equals_ordinary_tiles():
         runs = {}
         for mode in (0, 2):
             try:
-                _lib.call("aoz_gemm_set_wide_mode", mode, 0)
+                _lib.call("aoz_gemm_set_wide_mode", mode)
                 _lib.call("aoz_gemm_set_wide_max_rounds", 3)
                 _lib.call("aoz_gemm_set_tail_mode", 0)
                 runs[mode] = (ops.conv_fwd(x, wf, Cout, 3, bias=b, rowgroup_bias=temb), ops.conv_fwd(x, wf, Cout, 3, bias=b, residual=res),
                               ops.conv_fwd(dy, wd, Cin, 3, stride=1, pad=1, flip=True))
             finally:
-                _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+                _lib.call("aoz_gemm_set_wide_mode", 1)
                 _lib.call("aoz_gemm_set_wide_max_rounds", 2)
                 _lib.call("aoz_gemm_set_tail_mode", 1)
         conv = torch.nn.functional.conv2d(x.float().permute(0, 3, 1, 2), w.float(), b.float(), padding=1).permute(0, 2, 3, 1)
@@ -208,10 +208,10 @@ def test_conv_wgrad_wide_plan_equals_ordinary_tiles():
         runs = {}
         for mode in (0, 2):
             try:
-                _lib.call("aoz_gemm_set_wide_mode", mode, 0)
+                _lib.call("aoz_gemm_set_wide_mode", mode)
                 runs[mode] = [ops.conv_wgrad(dy, x, 3, stride=stride, pad=1, splits=sp) for sp in (1, 2, None)]
             finally:
-                _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+                _lib.call("aoz_gemm_set_wide_mode", 1)
         xr = x.float().permute(0, 3, 1, 2)
         wr = torch.zeros(Cout, Cin, 3, 3, device="cuda", requires_grad=True)
         torch.nn.functional.conv2d(xr, wr, None, stride=stride, padding=1).backward(dy.float().permute(0, 3, 1, 2))
@@ -240,27 +240,6 @@ def test_geglu_fused_epilogue_and_backward(M, C):
     check(ops.geglu_bwd(dy, aux), pr.grad, rel=8e-3)
 
 
-def test_gemm_tail_fixup_in_kernel_equals_separate_launch():
-    """Switchable path (off by default): the K slices of the tail tiles summed and stored by their own CTAs instead of by
-    tail_fixup_kernel -- same partials, same summation order, same fused epilogue: identical bits."""
-    from aozora_sdxl_training_b200 import _lib
-    ops = _ops()
-    g = gen(58)
-    for M, N, K in ((4096, 1280, 1280), (4096, 1280, 5120), (16384, 640, 640)):
-        x = torch.randn(M, K, device="cuda", generator=g).to(BF16)
-        w = (torch.randn(N, K, device="cuda", generator=g) * 0.05).to(BF16)
-        b = torch.randn(N, device="cuda", generator=g).to(BF16)
-        res = torch.randn(M, N, device="cuda", generator=g).to(BF16)
-        ref = ops.gemm(x, w, bias=b, residual=res)
-        try:
-            _lib.call("aoz_gemm_set_tail_inkernel", 1)
-            for _ in range(3):                                  # the counters must come back to zero after every launch
-                got = ops.gemm(x, w, bias=b, residual=res)
-        finally:
-            _lib.call("aoz_gemm_set_tail_inkernel", 0)
-        assert torch.equal(got, ref)
-
-
 def test_gemm_wide_one_wave_plan_equals_two_round_plan():
     """The 320-wide one-wave plan (one 256 x 320 tile per CTA pair, two MMAs per K step into a single accumulator, permuted column
     chunks in the epilogue) against the ordinary plans: every output element is the same K-ordered fp32 sum, so the bits agree; both
@@ -279,7 +258,7 @@ def test_gemm_wide_one_wave_plan_equals_two_round_plan():
         runs = {}
         for mode in (0, 2):
             try:
-                _lib.call("aoz_gemm_set_wide_mode", mode, 0)
+                _lib.call("aoz_gemm_set_wide_mode", mode)
                 _lib.call("aoz_gemm_set_wide_max_rounds", 3)
                 _lib.call("aoz_gemm_set_tail_mode", 0)              # a tail split sums K slices in another order: not the reference here
                 plain = ops.gemm(x, w, b_mn=b_mn, splits=1)
@@ -287,7 +266,7 @@ def test_gemm_wide_one_wave_plan_equals_two_round_plan():
                 acc = acc0.clone()
                 ops.gemm(x, w, b_mn=b_mn, out=acc, accumulate=True, splits=1)
             finally:
-                _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+                _lib.call("aoz_gemm_set_wide_mode", 1)
                 _lib.call("aoz_gemm_set_wide_max_rounds", 2)
                 _lib.call("aoz_gemm_set_tail_mode", 1)
             runs[mode] = (plain, fused, acc)
@@ -317,26 +296,6 @@ def test_layernorm_backward_with_column_sums_of_dx():
         want = dx1.float().sum(0)
         err = (col.float() - want).abs()
         assert bool((err <= 2 ** -7 * want.abs() + 2e-2).all()), float(err.max())
-
-
-def test_geglu_backward_with_fused_bias_gradient():
-    """geglu_bwd_colsum_kernel: daux identical to geglu_bwd_kernel's, and the bias gradient equal to the column sums of that daux
-    (formed from the rounded values; same partial / ticket scheme as colsum, other chunking -> fp32 summation order differs)."""
-    ops = _ops()
-    g = gen(56)
-    for M, C in ((4096, 1280), (1000, 640), (16, 320)):
-        half = 4 * C
-        dy = torch.randn(M, half, device="cuda", generator=g).to(BF16)
-        aux = torch.randn(M, 2 * half, device="cuda", generator=g).to(BF16)
-        ref = ops.geglu_bwd(dy, aux)
-        db = torch.empty(2 * half, device="cuda", dtype=BF16)
-        got = ops.geglu_bwd(dy, aux, bias_grad=db)
-        assert torch.equal(got, ref)
-        want = ref.float().sum(0)
-        err = (db.float() - want).abs()
-        assert bool((err <= 2 ** -7 * want.abs() + 2e-2).all()), float(err.max())
-        check(db, ops.colsum(ref), rel=3e-3)
-
 
 
 @pytest.mark.parametrize("NB,H,W,Cin,Cout,ks,stride", [
@@ -519,26 +478,22 @@ def test_layernorm_fwd_bwd(rows, C):
     assert torch.equal(dg2, dg) and torch.equal(db2, db)                  # fixed summation order: bit-reproducible
 
 
-def test_batched_column_sums_match_single_launches():
-    """One launch for several bias gradients (different heights and widths, strided rows) == the per-tensor kernel, bit for bit."""
+def test_column_sums_of_strided_wide_and_tiny_tensors():
+    """Bias gradients by colsum (different heights and widths, strided rows, a caller's destination) against fp32 sums, and
+    bit-equal from run to run (fixed summation order, no atomics on data; the finalize tickets reset after every launch)."""
     ops = _ops()
     g = gen(21)
     big = torch.randn(4096, 3840, device="cuda", generator=g).to(BF16)
     xs = [torch.randn(4096, 1280, device="cuda", generator=g).to(BF16), big[:, 1280:2560], torch.randn(4096, 10240, device="cuda", generator=g).to(BF16),
           torch.randn(308, 640, device="cuda", generator=g).to(BF16), torch.randn(1, 8, device="cuda", generator=g).to(BF16)]
     dest = torch.zeros(1280, device="cuda", dtype=BF16)
-    outs = ops.colsum_batch([(xs[0], dest)] + [(x, None) for x in xs[1:]])
+    outs = [ops.colsum(xs[0], out=dest)] + [ops.colsum(x) for x in xs[1:]]
     assert outs[0].data_ptr() == dest.data_ptr()
     for x, o in zip(xs, outs):
         check(o, x.float().sum(0))
-    # same chunking rule only when the launch geometry matches, so compare against fp32 sums within bf16 rounding (above) and
-    # check run-to-run reproducibility (fixed summation order, no atomics on data)
-    outs2 = ops.colsum_batch([(x, None) for x in xs])
+    outs2 = [ops.colsum(x) for x in xs]
     for a, b in zip(outs, outs2):
         assert torch.equal(a, b)
-    nine = ops.colsum_batch([(x, None) for x in (xs * 2)[:9]])           # more than 8 tensors: split into two launches
-    assert len(nine) == 9
-    check(nine[8], xs[3].float().sum(0))
 
 
 def test_glue_kernels():

@@ -26,7 +26,7 @@ def main():
         res = torch.randn(M, N, device="cuda").to(BF)
         out = torch.empty(M, N, device="cuda", dtype=BF)
         fn = (lambda: ops.gemm(x, w, b_mn=b_mn, bias=bias, residual=res, out=out)) if fused else (lambda: ops.gemm(x, w, b_mn=b_mn, out=out, splits=1))
-        _lib.call("aoz_gemm_set_wide_mode", wide, 0)
+        _lib.call("aoz_gemm_set_wide_mode", wide)
         _lib.call("aoz_gemm_set_tail_mode", 0)
         us = call_us(fn)
         scratch = ops._gemm_scratch[torch.cuda.current_device()]
@@ -44,7 +44,7 @@ def main():
                 f" epilogue_warps_done={min(epi)}..{max(epi)} teardown={t[7] - t0}")
         print(line, flush=True)
         lines.append(line)
-    _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+    _lib.call("aoz_gemm_set_wide_mode", 1)
     _lib.call("aoz_gemm_set_tail_mode", 1)
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     open(os.path.join(ROOT, "gpurun_out", "gemm_timeline.txt"), "w").write("\n".join(lines) + "\n")

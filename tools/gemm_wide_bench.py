@@ -1,6 +1,6 @@
 """The 320-wide one-wave plan against the ordinary plans on the 4096 x 1280 x K projection shapes of the step: device time of every
 kernel a call launches (GEMM + tail fix-up), median over calls, L2-warm and with a 256 MB flush between calls (weights cold, as in
-the step).      python tools/gemm_wide_bench.py [mn_n2]"""
+the step).      python tools/gemm_wide_bench.py"""
 import collections
 import json
 import os
@@ -34,7 +34,6 @@ def call_us(fn, n=8, interleave=None):
 
 
 def main():
-    n2 = int(sys.argv[1]) if len(sys.argv) > 1 else 0
     big = torch.empty(64 << 20, device="cuda", dtype=torch.float32)
     flush = lambda: big.zero_()
     rows = []
@@ -53,10 +52,10 @@ def main():
         fn = (lambda: ops.gemm(x, w, b_mn=b_mn, bias=bias, residual=res, out=out)) if fused else (lambda: ops.gemm(x, w, b_mn=b_mn, out=out))
         row = {"M": M, "N": N, "K": K, "b_mn": int(b_mn), "fused": int(fused)}
         for mode in (0, 2):
-            _lib.call("aoz_gemm_set_wide_mode", mode, n2)
+            _lib.call("aoz_gemm_set_wide_mode", mode)
             row[f"wide{mode}_warm_us"] = call_us(fn)
             row[f"wide{mode}_cold_us"] = call_us(fn, interleave=flush)
-        _lib.call("aoz_gemm_set_wide_mode", 1, 0)
+        _lib.call("aoz_gemm_set_wide_mode", 1)
         row["tflops_cold"] = [round(2.0 * M * N * K / row[f"wide{m}_cold_us"] * 1e-6, 1) for m in (0, 2)]
         rows.append(row)
         print(row, flush=True)

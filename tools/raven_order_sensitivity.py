@@ -1,7 +1,7 @@
 """How far two fp32 evaluation orders of the SAME Raven update (raven.py:126-143) drift apart on a 29.5 M-element tensor, CPU only.
 
 Order A = CPU ATen as the oracle runs it (``oracle/host_ref.raven_update_``); order B = CUDA ATen's (FMA contraction, multiply by
-1/sqrt_bc2) as ``raven_step_mt_kernel`` implements it, emulated here through float64 FMAs.  Output: how many elements exceed
+1/sqrt_bc2) as ``raven_step_bulk_kernel`` implements it, emulated here through float64 FMAs.  Output: how many elements exceed
 1e-6 x (|p| + |update|) -- the cancelled result -- and 1e-6 x (|p| + update TERMS), the scale tests/test_gpu_fullsize.py uses.
 """
 import os
