@@ -586,9 +586,9 @@ gemm_bf16_kernel(const __grid_constant__ GemmParams P) {
                     stage_chunk(stg, lane, rg);
                     __syncwarp();
                     const int col = col0 + c + lcol;
-                    if (col < col_limit) {                   // N/2 is a multiple of 8 for every SDXL layer
+                    if (col < col_limit) {                   // aoz_gemm_bf16 requires N/2 % 8 == 0: col + 7 < col_limit too
                         uint32_t bh[4] = {0u, 0u, 0u, 0u}, bg[4] = {0u, 0u, 0u, 0u};
-                        if (P.bias) {       // N/2 and the tile origin are multiples of 8: 16-byte aligned vectors
+                        if (P.bias) {       // N/2 and the tile origin are multiples of 8, pointers checked: 16-byte aligned vectors
                             const uint4 t0 = __ldg(reinterpret_cast<const uint4*>(P.bias + col));
                             const uint4 t1 = __ldg(reinterpret_cast<const uint4*>(P.bias + P.geglu_half + col));
                             bh[0] = t0.x; bh[1] = t0.y; bh[2] = t0.z; bh[3] = t0.w;
@@ -1168,6 +1168,10 @@ int aoz_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long lo
     const bool geglu = epi == EPI_GEGLU;
     if (geglu) {
         AOZ_CHECK_ARG((N % 2) == 0 && !b_mn && splits == 1, "aoz_gemm_bf16: GEGLU needs even N, K-major B, no split");
+        // the GEGLU epilogue loads bias and stores C / aux as 16-byte vectors of 8 columns with no scalar tail
+        AOZ_CHECK_ARG(((N / 2) % 8) == 0, "aoz_gemm_bf16: GEGLU needs N/2 to be a multiple of 8 (got N=%d)", N);
+        AOZ_CHECK_ARG(((((uintptr_t)C | (uintptr_t)aux | (uintptr_t)bias) & 15) == 0) && (ldc % 8) == 0 && (!aux || (ld_aux % 8) == 0),
+                      "aoz_gemm_bf16: GEGLU needs 16-byte aligned C / aux / bias and ldc / ld_aux multiples of 8 elements");
         P.geglu_half = N / 2;
     }
     if (splits > 1) {

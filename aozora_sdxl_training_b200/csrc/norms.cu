@@ -34,7 +34,10 @@ __device__ __forceinline__ void unpack8v(const uint4& a, float2* f) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// GroupNorm statistics: x [NB, HW, C] -> partial [NB][chunks][GROUPS][2] (sum, sumsq) -> mean / rstd [NB][GROUPS]
+// GroupNorm statistics: x [NB, HW, C] -> partial [NB][chunks][GROUPS][2] (sum, sumsq of x - pivot) -> mean / rstd [NB][GROUPS]
+// The sums are taken of x - pivot with pivot = x[n, 0, g * cpg] (the group's first element), so var = E[d^2] - E[d]^2 subtracts two
+// numbers of the size of the variance: E[x^2] - mean^2 cancels catastrophically once |mean| >> std (offset activations), and
+// Welford's update would cost a division per element.  Still one pass, same order, deterministic.
 // grid (chunks, NB) ~ one block per SM; block = `cols` vector columns x `row_lanes` row lanes (<= 1024 threads, rounded up to
 // whole warps).  A thread owns one 8-channel vector column and walks its row lane of the chunk with four rows in flight.
 // No float atomics anywhere (they would make the low bits of every statistic and gradient differ run to run): the row-lane
@@ -62,11 +65,12 @@ gn_stats_kernel(const __nv_bfloat16* __restrict__ x, int HW, int C, float eps, i
     const int r0 = chunk * rows_per_chunk, r1 = min(HW, r0 + rows_per_chunk);
     const __nv_bfloat16* xb = x + (size_t)n * HW * C;
     const int tc = threadIdx.x % cols, tr = threadIdx.x / cols;
+    const int cpg = C / GN_GROUPS;
     if (tr < row_lanes) {
         for (int v = tc; v < vec_per_row; v += cols) {             // one trip unless C/8 exceeds the block (then row_lanes == 1)
-            float s[8], q[8];
+            float s[8], q[8], pv[8];
 #pragma unroll
-            for (int e = 0; e < 8; ++e) { s[e] = 0.f; q[e] = 0.f; }
+            for (int e = 0; e < 8; ++e) { s[e] = 0.f; q[e] = 0.f; pv[e] = __bfloat162float(xb[((v * 8 + e) / cpg) * cpg]); }
             int r = r0 + tr;
             for (; r + 3 * row_lanes < r1; r += 4 * row_lanes) {           // four rows in flight
                 uint4 px[4];
@@ -77,14 +81,14 @@ gn_stats_kernel(const __nv_bfloat16* __restrict__ x, int HW, int C, float eps, i
                     float f[8];
                     unpack8(px[u], f);
 #pragma unroll
-                    for (int e = 0; e < 8; ++e) { s[e] += f[e]; q[e] = fmaf(f[e], f[e], q[e]); }
+                    for (int e = 0; e < 8; ++e) { const float d = f[e] - pv[e]; s[e] += d; q[e] = fmaf(d, d, q[e]); }
                 }
             }
             for (; r < r1; r += row_lanes) {
                 float f[8];
                 unpack8(ld_stream(xb + (size_t)r * C + v * 8), f);
 #pragma unroll
-                for (int e = 0; e < 8; ++e) { s[e] += f[e]; q[e] = fmaf(f[e], f[e], q[e]); }
+                for (int e = 0; e < 8; ++e) { const float d = f[e] - pv[e]; s[e] += d; q[e] = fmaf(d, d, q[e]); }
             }
             float* d = sm + (size_t)tr * 2 * C + v * 8;
 #pragma unroll
@@ -93,7 +97,6 @@ gn_stats_kernel(const __nv_bfloat16* __restrict__ x, int HW, int C, float eps, i
     }
     __syncthreads();
     // (group, which) pairs: 16 threads each, fixed summation order
-    const int cpg = C / GN_GROUPS;
     const int sub = threadIdx.x & 15;
     const int count = row_lanes * cpg;
     for (int p = threadIdx.x >> 4; p < 2 * GN_GROUPS; p += blockDim.x >> 4) {
@@ -127,8 +130,9 @@ gn_stats_kernel(const __nv_bfloat16* __restrict__ x, int HW, int C, float eps, i
     if (threadIdx.x < GN_GROUPS) {
         const int g = threadIdx.x;
         const float cnt = (float)HW * (float)cpg;
-        const float mean = s_fin[0][g] / cnt;
-        const float var = fmaxf(s_fin[1][g] / cnt - mean * mean, 0.f);
+        const float dm = s_fin[0][g] / cnt;                      // mean of x - pivot
+        const float var = fmaxf(s_fin[1][g] / cnt - dm * dm, 0.f);
+        const float mean = __bfloat162float(xb[g * cpg]) + dm;
         mean_out[n * GN_GROUPS + g] = mean;
         rstd_out[n * GN_GROUPS + g] = rsqrtf(var + eps);
     }
@@ -454,18 +458,20 @@ gn_slab_fwd_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __r
     float gm[8], bt[8];
     unpack8(*reinterpret_cast<const uint4*>(gamma + g * cpg + tc * 8), gm);
     unpack8(*reinterpret_cast<const uint4*>(beta + g * cpg + tc * 8), bt);
+    const float pivot = __bfloat162float(x[(size_t)n * HW * C + g * cpg]);     // sums of x - pivot: see gn_stats_kernel
     cp_async_wait_all();
     float s = 0.f, q = 0.f;
     for (int idx = threadIdx.x; idx < nvec; idx += T) {
         float f[8];
         unpack8(*reinterpret_cast<const uint4*>(gn_slab + (size_t)idx * 16), f);
 #pragma unroll
-        for (int e = 0; e < 8; ++e) { s += f[e]; q = fmaf(f[e], f[e], q); }
+        for (int e = 0; e < 8; ++e) { const float d = f[e] - pivot; s += d; q = fmaf(d, d, q); }
     }
     block_sum2(s, q, s_red);
     const float cnt = (float)HW * (float)cpg;
-    const float mean = s / cnt;
-    const float rstd = rsqrtf(fmaxf(q / cnt - mean * mean, 0.f) + eps);
+    const float dm = s / cnt;
+    const float mean = pivot + dm;
+    const float rstd = rsqrtf(fmaxf(q / cnt - dm * dm, 0.f) + eps);
     if (threadIdx.x == 0) { mean_out[n * GN_GROUPS + g] = mean; rstd_out[n * GN_GROUPS + g] = rstd; }
     float sc[8], sh[8];
 #pragma unroll

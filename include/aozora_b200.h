@@ -49,8 +49,9 @@ int aoz_clip_coef_from_sumsq(const void* sumsq, float max_norm, int emulate_bf16
  *      time/add embedding MLPs) forward, dgrad, wgrad; nn.Conv2d 3x3/1x1 as implicit GEMM -------------------- */
 int aoz_gemm_set_pair_mode(int mode);
 /* SMs the persistent GEMM / conv launches may occupy (0 = all, rounded down to even): data-parallel runs leave NCCL's CTAs their own
- * SMs (set NCCL_MAX_CTAS to the difference) so that no persistent CTA waits behind a collective kernel.  Set before the first GEMM:
- * tile plans are cached per shape. */
+ * SMs (set NCCL_MAX_CTAS to the difference) so that no persistent CTA waits behind a collective kernel.  Nothing is cached: every
+ * GEMM / conv call plans its tiles (CTA pairs, tail split, wide plan) for the budget in force at that call, while launches already
+ * captured into a CUDA graph keep the plan they were captured with. */
 int aoz_gemm_set_sm_budget(int sms);
 int aoz_gemm_force_bn(int bn);
 /* tail split: tiles of the last, partly filled wave are cut along K across the idle SMs (fp32 slices in the caller-owned
