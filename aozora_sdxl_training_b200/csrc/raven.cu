@@ -353,6 +353,78 @@ __global__ void clip_coef_from_sumsq_kernel(const float* __restrict__ sumsq, flo
     out[1] = fminf(coef, 1.0f);
 }
 
+// ---- gradient accumulation: y[t] = copy ? b[t] : a[t] + b[t], bf16, every tensor in one launch -----------------------
+// The arithmetic is add_kernel's (elementwise.cu): fp32 add, one round-to-nearest-even to bf16, so each tensor is bit-identical to
+// aoz_add on it.  y may alias a or b: every element is read and then written by the same thread and never read again, which is why
+// the loads are the coherent ones and no pointer is __restrict__.  Each CTA owns a contiguous run of chunks, so consecutive chunks
+// mostly share a tensor and its table entries stay in registers.  A chunk whose pointers are not all 16-byte aligned, and the last
+// (< 8) elements of a tensor, go element by element.
+constexpr int ACC_UNROLL = 4;                   // 16-byte vectors per operand in flight per thread
+
+__device__ __forceinline__ uint4 ld_once(const void* p) {
+    uint4 r;
+    asm volatile("ld.global.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p) : "memory");
+    return r;
+}
+
+template <bool COPY>
+__global__ void __launch_bounds__(MT_THREADS)
+grad_accum_mt_kernel(int n_chunks, int chunks_per_cta, const uint64_t* __restrict__ a_ptrs, const uint64_t* __restrict__ b_ptrs,
+                     const uint64_t* __restrict__ y_ptrs, const int64_t* __restrict__ numel,
+                     const int32_t* __restrict__ chunk_start, const int32_t* __restrict__ chunk_tensor) {
+    const int c0 = blockIdx.x * chunks_per_cta;
+    const int c1 = min(c0 + chunks_per_cta, n_chunks);
+    if (c0 >= c1) return;
+    int t = chunk_tensor[c0];
+    int t_first = chunk_start[t], t_next = chunk_start[t + 1];
+    const __nv_bfloat16* a = COPY ? nullptr : (const __nv_bfloat16*)a_ptrs[t];
+    const __nv_bfloat16* b = (const __nv_bfloat16*)b_ptrs[t];
+    __nv_bfloat16* y = (__nv_bfloat16*)y_ptrs[t];
+    int64_t n = numel[t];
+    for (int c = c0; c < c1; ++c) {
+        if (c >= t_next) {                      // tensors without elements own no chunk: skip past them
+            do { ++t; t_first = t_next; t_next = chunk_start[t + 1]; } while (c >= t_next);
+            if (!COPY) a = (const __nv_bfloat16*)a_ptrs[t];
+            b = (const __nv_bfloat16*)b_ptrs[t];
+            y = (__nv_bfloat16*)y_ptrs[t];
+            n = numel[t];
+        }
+        const int64_t begin = (int64_t)(c - t_first) * MT_CHUNK;
+        const int64_t end = min(begin + (int64_t)MT_CHUNK, n);
+        const bool aligned = ((((uintptr_t)a | (uintptr_t)b | (uintptr_t)y) & 15) == 0);
+        const int64_t vec_end = aligned ? begin + ((end - begin) & ~(int64_t)7) : begin;
+        for (int64_t i = begin + (int64_t)threadIdx.x * 8; i < vec_end; i += (int64_t)MT_THREADS * 8 * ACC_UNROLL) {
+            uint4 va[ACC_UNROLL], vb[ACC_UNROLL];
+#pragma unroll
+            for (int u = 0; u < ACC_UNROLL; ++u) {
+                const int64_t j = i + (int64_t)u * MT_THREADS * 8;
+                if (j < vec_end) {
+                    vb[u] = ld_once(b + j);
+                    if (!COPY) va[u] = ld_once(a + j);
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < ACC_UNROLL; ++u) {
+                const int64_t j = i + (int64_t)u * MT_THREADS * 8;
+                if (j < vec_end) {
+                    if (COPY) {
+                        st_stream(y + j, vb[u]);
+                    } else {
+                        const uint4 ra = va[u], rb = vb[u];
+                        st_stream(y + j, make_uint4(pack_bf16(bf16lo(ra.x) + bf16lo(rb.x), bf16hi(ra.x) + bf16hi(rb.x)),
+                                                    pack_bf16(bf16lo(ra.y) + bf16lo(rb.y), bf16hi(ra.y) + bf16hi(rb.y)),
+                                                    pack_bf16(bf16lo(ra.z) + bf16lo(rb.z), bf16hi(ra.z) + bf16hi(rb.z)),
+                                                    pack_bf16(bf16lo(ra.w) + bf16lo(rb.w), bf16hi(ra.w) + bf16hi(rb.w))));
+                    }
+                }
+            }
+        }
+        for (int64_t i = vec_end + threadIdx.x; i < end; i += MT_THREADS)
+            y[i] = COPY ? b[i] : __float2bfloat16_rn(__bfloat162float(a[i]) + __bfloat162float(b[i]));
+    }
+}
+
 }  // namespace aoz
 
 using namespace aoz;
@@ -428,6 +500,37 @@ int aoz_clip_coef_from_sumsq(const void* sumsq, float max_norm, int emulate_bf16
     AOZ_CHECK_ARG(sumsq && out2, "aoz_clip_coef_from_sumsq: null pointer");
     clip_coef_from_sumsq_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((const float*)sumsq, max_norm, emulate_bf16, (float*)out2);
     AOZ_CHECK_LAUNCH("clip_coef_from_sumsq_kernel");
+    return AOZ_OK;
+}
+
+int aoz_grad_accum_mt(int n_tensors, int n_chunks, const void* a_ptrs, const void* b_ptrs, const void* y_ptrs,
+                      const void* numel, const void* chunk_start, const void* chunk_tensor, int copy, void* stream) {
+    AOZ_CHECK_ARG(n_tensors > 0 && n_chunks >= 0, "aoz_grad_accum_mt: n_tensors must be positive, n_chunks non-negative");
+    AOZ_CHECK_ARG(b_ptrs && y_ptrs && numel && chunk_start && chunk_tensor && (copy || a_ptrs),
+                  "aoz_grad_accum_mt: null table pointer");
+    AOZ_CHECK_ARG(((((uintptr_t)a_ptrs | (uintptr_t)b_ptrs | (uintptr_t)y_ptrs | (uintptr_t)numel) & 7) == 0) &&
+                  ((((uintptr_t)chunk_start | (uintptr_t)chunk_tensor) & 3) == 0),
+                  "aoz_grad_accum_mt: misaligned table pointer");
+    if (n_chunks == 0) return AOZ_OK;
+    static int per_sm = 0;
+    if (per_sm == 0) {
+        int k = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k, grad_accum_mt_kernel<false>, MT_THREADS, 0);
+        per_sm = k > 0 ? k : 1;
+    }
+    const int ctas = n_chunks < sm_count() * per_sm ? n_chunks : sm_count() * per_sm;
+    const int per_cta = (n_chunks + ctas - 1) / ctas;
+    const int grid = (n_chunks + per_cta - 1) / per_cta;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (copy)
+        grad_accum_mt_kernel<true><<<grid, MT_THREADS, 0, s>>>(n_chunks, per_cta, (const uint64_t*)a_ptrs, (const uint64_t*)b_ptrs,
+                                                               (const uint64_t*)y_ptrs, (const int64_t*)numel,
+                                                               (const int32_t*)chunk_start, (const int32_t*)chunk_tensor);
+    else
+        grad_accum_mt_kernel<false><<<grid, MT_THREADS, 0, s>>>(n_chunks, per_cta, (const uint64_t*)a_ptrs, (const uint64_t*)b_ptrs,
+                                                                (const uint64_t*)y_ptrs, (const int64_t*)numel,
+                                                                (const int32_t*)chunk_start, (const int32_t*)chunk_tensor);
+    AOZ_CHECK_LAUNCH("grad_accum_mt_kernel");
     return AOZ_OK;
 }
 

@@ -6,6 +6,7 @@ PyTorch is plumbing here (device memory, streams).  Every function launches hand
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -426,6 +427,31 @@ def add(a, b, out=None):
     _lib.call("aoz_add", a.data_ptr(), b.data_ptr(), a.numel(), out.data_ptr(), _stream())
     _count()
     return out
+
+
+def grad_accum_mt(ys, as_, bs, plan, stage, copy=False):
+    """``ys[t] = bs[t]`` (``copy``) or ``as_[t] + bs[t]`` for every t, bf16, in ONE launch; each tensor is bit-identical to
+    ``add``.  ``ys`` may alias ``as_`` or ``bs``.  ``plan`` is the caller's ``MultiTensorPlan`` and ``stage`` its ``_Staging``
+    (optimizers/raven.py): the pointer tables go through ``stage``, so a call under CUDA-graph capture bakes its own tables in."""
+    n = len(ys)
+    if n == 0 or len(bs) != n or (not copy and len(as_) != n):
+        raise _lib.AozoraError("grad_accum_mt: need the same, non-zero number of tensors in every list")
+    for i in range(n):
+        for t, name in ((ys[i], "grad_accum_mt y"), (bs[i], "grad_accum_mt b")) + (() if copy else ((as_[i], "grad_accum_mt a"),)):
+            _chk(t, name)
+            if t.numel() != ys[i].numel():
+                raise _lib.AozoraError(f"{name}: tensor {i} has {t.numel()} elements, y has {ys[i].numel()}")
+    dev = ys[0].device
+    plan.ensure([y.numel() for y in ys], dev)
+
+    def table(name, ts):
+        return stage.put(name, np.fromiter((t.data_ptr() for t in ts), dtype=np.uint64, count=n).view(np.int64), dev).data_ptr()
+
+    yp, bp = table("acc_y", ys), table("acc_b", bs)
+    ap = 0 if copy else table("acc_a", as_)
+    _lib.call("aoz_grad_accum_mt", plan.n_tensors, plan.n_chunks, ap, bp, yp, plan.numel.data_ptr(), plan.chunk_start.data_ptr(),
+              plan.chunk_tensor.data_ptr(), int(bool(copy)), _stream())
+    _count()
 
 
 def upsample2x_fwd(x):

@@ -28,7 +28,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from . import _lib
+from . import _lib, ops
 from .optimizers.raven import RavenAdamW, raven_host_scalars, _DT
 
 ALIGN = 8                    # elements: keeps every parameter slot 16-byte aligned for the vector kernels
@@ -55,6 +55,10 @@ class _KernelBackend:
                   tables["m"].data_ptr(), tables["v"].data_ptr(), plan.numel.data_ptr(), plan.chunk_start.data_ptr(),
                   plan.chunk_tensor.data_ptr(), hyper.data_ptr(), 0 if clip_coef is None else clip_coef.data_ptr(), _DT[pdt],
                   _DT[gdt], _DT[mdt], torch.cuda.current_stream().cuda_stream)
+
+    @staticmethod
+    def add(a, b, out):
+        ops.add(a, b, out=out)
 
 
 def _ptr_table(tensors, device):
@@ -212,6 +216,7 @@ class DataParallel:
         self.flat_p = torch.zeros(L.total, dtype=self.dtype, device=self.device)
         self.flat_g = torch.zeros(L.total, dtype=self.dtype, device=self.device)
         self.g_shard = torch.zeros(L.shard_elems(), dtype=self.dtype, device=self.device)
+        self.acc_shard = None                # gradient accumulation across micro-steps (reduce_accumulate)
         self.index = {}
         with torch.no_grad():
             for i, p in enumerate(self.params):
@@ -238,6 +243,8 @@ class DataParallel:
         self._seg_cache = None
         self._pending = None
         self._works = []
+        self._issued = []                    # buckets reduced so far in this micro-step, in issue order
+        self._reduce_order = list(range(len(L.buckets)))     # the last complete micro-step's issue order
         self._norm = torch.zeros(4, dtype=torch.float32, device=self.device)
         self._coef = torch.zeros(2, dtype=torch.float32, device=self.device)
         self.optimizer = None
@@ -339,6 +346,9 @@ class DataParallel:
 
     # ---- gradient path -----------------------------------------------------------------------------------
     def _reset_pending(self):
+        if len(self._issued) == len(self.layout.buckets):
+            self._reduce_order = self._issued
+        self._issued = []
         self._pending = list(self.bucket_need)
         self._arrived = bytearray(len(self.params))
         self._works = []
@@ -348,11 +358,12 @@ class DataParallel:
         self._reset_pending()
         self.flat_g.zero_()
         self._arrived = bytearray(b"\x01" * len(self.params))
-        for k in range(len(self.layout.buckets)):
+        for k in self._reduce_order:              # collectives pair up by issue order: the order the other ranks' sweeps use
             self._pending[k] = 0
             self._reduce_bucket(k)
 
     def _reduce_bucket(self, k):
+        self._issued.append(k)
         s, e = self.layout.buckets[k]
         n = (e - s) // self.world
         out = self.g_shard[self._slice_base[k]:self._slice_base[k] + n]
@@ -417,10 +428,9 @@ class DataParallel:
             return opt._stage.put("dp_hyper", hy, self.device)
         return torch.from_numpy(hy)
 
-    def reduce_clip_step(self, optimizer, max_norm):
-        """Finish the reduce-scatter, clip by the GLOBAL norm, update this rank's slices, all-gather the parameters.
-        CUDA-graph capturable: under capture the step counter / hyper table are left to ``advance_host_state``."""
-        capturing = self.device.type == "cuda" and torch.cuda.is_current_stream_capturing()
+    def _finish_reduce(self):
+        """Reduce every bucket the sweep left incomplete and wait for all reduce-scatters of this micro-step: ``g_shard`` then
+        holds this rank's slices of the summed gradient."""
         if any(c != 0 for c in self._pending):
             # parameters that produced no gradient in this sweep: their slots still hold an earlier step's values -- this
             # rank's contribution is zero, so clear them before the buckets they sit in are reduced
@@ -434,6 +444,28 @@ class DataParallel:
         for w in self._works:
             w.wait()
         self._reset_pending()
+
+    def reduce_accumulate(self, first):
+        """GRADIENT_ACCUMULATION_STEPS > 1, every micro-step of a window but the last: finish this micro-step's reduce-scatter
+        and accumulate the reduced shard (``first``: start the window with it), in bf16 with one rounding per add as torch's
+        ``p.grad`` accumulation does.  The accumulator is 1/N of the flat gradient, allocated on the first call."""
+        self._finish_reduce()
+        if self.acc_shard is None:
+            self.acc_shard = torch.empty_like(self.g_shard)
+        if first:
+            self.acc_shard.copy_(self.g_shard)
+        else:
+            self.backend.add(self.acc_shard, self.g_shard, self.acc_shard)
+
+    def reduce_clip_step(self, optimizer, max_norm, accumulated=False):
+        """Finish the reduce-scatter, clip by the GLOBAL norm, update this rank's slices, all-gather the parameters.
+        ``accumulated``: last micro-step of an accumulation window -- the shard accumulated by ``reduce_accumulate`` is added to
+        this micro-step's before the norm.  CUDA-graph capturable: under capture the step counter / hyper table are left to
+        ``advance_host_state``."""
+        capturing = self.device.type == "cuda" and torch.cuda.is_current_stream_capturing()
+        self._finish_reduce()
+        if accumulated:
+            self.backend.add(self.acc_shard, self.g_shard, self.g_shard)
         opt = optimizer
         seg_p, seg_g, seg_m, seg_v, seg_params, tables = self._segment_views(opt)
         if capturing:

@@ -18,6 +18,7 @@ from dataclasses import dataclass
 import torch
 
 from . import _lib, host, ops
+from .optimizers.raven import MultiTensorPlan, _Staging
 from .scheduler import DDPMScheduler
 
 BF16 = torch.bfloat16
@@ -60,9 +61,6 @@ class SDXLTrainStep:
         if self.global_batch % self.world:
             raise ValueError("BATCH_SIZE (global) must be divisible by the number of ranks")
         self.local_batch = self.global_batch // self.world
-        if dp is not None and self.grad_accum != 1:
-            raise ValueError("data-parallel training reduces every micro-step: GRADIENT_ACCUMULATION_STEPS must be 1 "
-                             "(raise the per-GPU batch instead; 180 GB of HBM holds b=16 at 1024x1024)")
         if not hasattr(config, "is_rectified_flow"):
             config.is_rectified_flow = self.is_rf
         self.sampler = host.TimestepSampler(config, self.device)
@@ -76,10 +74,15 @@ class SDXLTrainStep:
         self.micro_step = 0
         self.optimizer_steps = 0
         self._accum = None              # {param: grad} carried across micro-steps when GRADIENT_ACCUMULATION_STEPS > 1
+        self._acc = None                # the captured step's accumulator: one flat bf16 buffer, one 16-byte-aligned view per parameter
+        self._acc_views = None
+        self._acc_plan = MultiTensorPlan()
+        self._acc_stage = _Staging()
         self.trainable = [p for p in unet.parameters() if p.requires_grad]
         self.use_cuda_graph = use_cuda_graph          # capture the device side of the step once, replay it afterwards
         self.graph_warmup = graph_warmup
         self._graphs = {}
+        self._pools = {}                # GRADIENT_ACCUMULATION_STEPS > 1: one graph memory pool per input shape, shared by its phases
 
     # ---- pieces ------------------------------------------------------------------------------------------
     def _to_device(self, t, dtype=None):
@@ -181,10 +184,21 @@ class SDXLTrainStep:
         if self.lr_scheduler is not None:
             self.lr_scheduler.step(self.micro_step)
         self.dp.no_gradients_this_step()
-        norm = self._optimizer_phase(None)
-        self.optimizer_steps += 1
+        phase = self._phase()
+        norm = None
+        if phase == "last":
+            norm = self._optimizer_phase(None)
+            self.optimizer_steps += 1
+        else:
+            self.dp.reduce_accumulate(first=phase == "first")
         return StepResult(loss=torch.zeros(1, dtype=torch.float32, device=self.device), grad_norm=norm, timesteps=tickets,
-                          did_optimizer_step=True, lr=self.optimizer.param_groups[0]["lr"])
+                          did_optimizer_step=phase == "last", lr=self.optimizer.param_groups[0]["lr"])
+
+    def _phase(self):
+        """Where the micro-step just counted sits in its accumulation window: "first", "middle" or "last" (optimizer step).
+        With GRADIENT_ACCUMULATION_STEPS = 1 every micro-step is "last"."""
+        r = self.micro_step % self.grad_accum
+        return "last" if r == 0 else "first" if r == 1 else "middle"
 
     @torch.no_grad()
     def step(self, batch, *, noise=None, jitter=None, taps=None) -> StepResult:
@@ -193,33 +207,67 @@ class SDXLTrainStep:
         if self.dp is not None and batch.get("latents") is None:
             return self._rank_without_rows(batch)
         inputs = self._host_inputs(batch, noise, jitter)
-        if self.use_cuda_graph and self.grad_accum == 1 and taps is None:
+        if self.use_cuda_graph and taps is None:
             return self._graph_step(inputs)
         latents, embeds, pooled, time_ids, tickets, noise, jitter, global_len = inputs
         loss, grads = self._device_step(latents, embeds, pooled, time_ids, tickets, noise, jitter, global_len, taps=taps)
         self.micro_step += 1
-        if self.grad_accum > 1:
+        if self.grad_accum > 1 and self.dp is None:
             if self._accum is None:
                 self._accum = grads
             else:
-                for p, g in grads.items():
-                    ops.add(self._accum[p], g, out=self._accum[p])
+                ps = list(grads)
+                acc = [self._accum[p] for p in ps]
+                ops.grad_accum_mt(acc, acc, [grads[p] for p in ps], self._acc_plan, self._acc_stage)
             grads = self._accum
         if self.lr_scheduler is not None:
             self.lr_scheduler.step(self.micro_step)
-        did = self.micro_step % self.grad_accum == 0
+        phase = self._phase()
+        did = phase == "last"
         norm = None
         if did:
             norm = self._optimizer_phase(grads)
             self._accum = None
             self.optimizer_steps += 1
+        elif self.dp is not None:
+            self.dp.reduce_accumulate(first=phase == "first")
         return StepResult(loss=loss, grad_norm=norm, timesteps=tickets, did_optimizer_step=did,
                           lr=self.optimizer.param_groups[0]["lr"])
 
     def _optimizer_phase(self, grads):
         if self.dp is not None:
-            return self.dp.reduce_clip_step(self.optimizer, self.clip)
+            return self.dp.reduce_clip_step(self.optimizer, self.clip, accumulated=self.grad_accum > 1)
         return self.optimizer.clip_and_step(self.clip, grads=grads)
+
+    def _after_sweep(self, grads, phase):
+        """The device work that follows the reverse sweep in the captured form of the step (also run eagerly by its warm-up).
+        One GPU with GRADIENT_ACCUMULATION_STEPS > 1 accumulates into the persistent ``_acc``: the first micro-step of a window
+        copies its gradient there, the middle ones add to it, and the last adds it into its own gradient tensors in place -- so
+        the norm and Raven launches of the last phase are exactly the ones a window of one captures.  Data parallel accumulates
+        the reduced shard instead (``DataParallel.reduce_accumulate``).  Returns the norm on the last phase, else None."""
+        if phase != "last":
+            if self.dp is not None:
+                self.dp.reduce_accumulate(first=phase == "first")
+                return None
+            ps = [p for p in self.trainable if p in grads]
+            acc, g = self._accumulator(ps), [grads[p] for p in ps]
+            ops.grad_accum_mt(acc, acc, g, self._acc_plan, self._acc_stage, copy=phase == "first")
+            return None
+        if self.dp is None and self.grad_accum > 1:
+            ps = [p for p in self.trainable if p in grads]
+            g = [grads[p] for p in ps]
+            ops.grad_accum_mt(g, self._accumulator(ps), g, self._acc_plan, self._acc_stage)
+        return self._optimizer_phase(grads)
+
+    def _accumulator(self, params):
+        if self._acc is None:
+            offs, off = [], 0
+            for p in self.trainable:
+                offs.append(off)
+                off += (p.numel() + 7) // 8 * 8
+            self._acc = torch.empty(off, dtype=BF16, device=self.device)
+            self._acc_views = {p: self._acc[o:o + p.numel()].view(p.shape) for p, o in zip(self.trainable, offs)}
+        return [self._acc_views[p] for p in params]
 
     # ---- CUDA-graph path: the whole device side of the step is captured once and replayed ---------------------
     def _graph_step(self, inputs):
@@ -228,6 +276,18 @@ class SDXLTrainStep:
         self.micro_step += 1
         if self.lr_scheduler is not None:
             self.lr_scheduler.step(self.micro_step)
+        phase = self._phase()
+        pool = None
+        if self.grad_accum > 1:
+            # every phase of one shape shares one memory pool: a replay's intermediates are dead when it ends, and what outlives
+            # it (static inputs, st["out"], the accumulators) is allocated outside the pool or never freed
+            pool = self._pools.get(key)
+            if pool is None:
+                pool = self._pools[key] = torch.cuda.graph_pool_handle()
+            key = key + (phase,)
+        last = phase == "last"
+        if self.grad_accum > 1 and self.dp is None:
+            self._accumulator(())          # before the first warm-up's activations, whose cached segments it would otherwise split
         st = self._graphs.get(key)
         if st is None:
             st = self._graphs[key] = dict(calls=0, graph=None)
@@ -235,19 +295,19 @@ class SDXLTrainStep:
         if st["graph"] is None and st["calls"] <= self.graph_warmup:
             # eager warm-up: sizes the workspaces, allocates optimizer state, loads every kernel
             loss, grads = self._device_step(latents, embeds, pooled, time_ids, tickets, noise, jitter, global_len)
-            norm = self._optimizer_phase(grads)
-            self.optimizer_steps += 1
-            return StepResult(loss=loss, grad_norm=norm, timesteps=tickets, did_optimizer_step=True,
+            norm = self._after_sweep(grads, phase)
+            self.optimizer_steps += int(last)
+            return StepResult(loss=loss, grad_norm=norm, timesteps=tickets, did_optimizer_step=last,
                               lr=self.optimizer.param_groups[0]["lr"])
         if st["graph"] is None:
             st["static"] = [t.clone() if t is not None else None for t in (latents, embeds, pooled, time_ids, tickets, noise, jitter)]
             self.unet._packs.d.clear()             # packed conv weights must be (re)built inside the graph on every replay
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
+            with torch.cuda.graph(g, pool=pool):
                 sl, se, sp, sti, stk, sn, sj = st["static"]
                 loss, grads = self._device_step(sl, se, sp, sti, stk, sn, sj, global_len)
-                norm = self._optimizer_phase(grads)
+                norm = self._after_sweep(grads, phase)
                 st["out"] = (loss, norm)
                 del grads
             st["graph"] = g
@@ -255,9 +315,10 @@ class SDXLTrainStep:
         for dst, src in zip(st["static"], (latents, embeds, pooled, time_ids, tickets, noise, jitter)):
             if dst is not None:
                 dst.copy_(src, non_blocking=True)
-        self.optimizer.advance_host_state()
+        if last:
+            self.optimizer.advance_host_state()
         st["graph"].replay()
-        self.optimizer_steps += 1
+        self.optimizer_steps += int(last)
         loss, norm = st["out"]
-        return StepResult(loss=loss.clone(), grad_norm=norm.clone(), timesteps=tickets, did_optimizer_step=True,
+        return StepResult(loss=loss.clone(), grad_norm=norm.clone() if last else None, timesteps=tickets, did_optimizer_step=last,
                           lr=self.optimizer.param_groups[0]["lr"])

@@ -44,6 +44,13 @@ int aoz_gradnorm_mt(int n_tensors, int n_chunks, const void* g_ptrs, const void*
                     const void* chunk_tensor, void* partial, float max_norm, int emulate_bf16, void* out3,
                     int g_dtype, void* stream);
 int aoz_clip_coef_from_sumsq(const void* sumsq, float max_norm, int emulate_bf16, void* out2, void* stream);
+/* Gradient accumulation (train.py:2765 with GRADIENT_ACCUMULATION_STEPS > 1: torch adds each micro-step's bf16 gradient into
+ * p.grad): y[t] = copy ? b[t] : a[t] + b[t] for every tensor t, bf16, one launch over the multi-tensor tables above.  Each
+ * element is bit-identical to aoz_add on the same pair (fp32 add, one round to nearest even).  y may alias a or b.  a_ptrs may
+ * be null when copy != 0.  Tensors need only bf16 alignment: chunks whose pointers are all 16-byte aligned are vectorised.
+ * The tables must be aligned to their element size; n_tensors must be positive. */
+int aoz_grad_accum_mt(int n_tensors, int n_chunks, const void* a_ptrs, const void* b_ptrs, const void* y_ptrs,
+                      const void* numel, const void* chunk_start, const void* chunk_tensor, int copy, void* stream);
 
 /* ---- dense contractions [3P]: nn.Linear (to_q/k/v, to_out.0, proj_in/out, ff.net.0.proj + GEGLU, ff.net.2,
  *      time/add embedding MLPs) forward, dgrad, wgrad; nn.Conv2d 3x3/1x1 as implicit GEMM -------------------- */
